@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the hot path (VocoderProject DSP core, batched over streams).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic streams: per stream it is
@@ -15,6 +15,9 @@ on the engine's stream, max over ranks). `e2e`: the same batch through the C-ABI
 vp_engine_process_host with pinned HOST buffers (H2D + compute + D2H inside the timed region).
 `--impl reference`: the reference's own C++ (oracle/_ref, compiled in place; else the C oracle
 port) on the host cores, on a bounded sample of the same workload.
+`--dump-outputs DIR`: after the timed steps, a fixed, seeded sample (at most 64 MB) of the audio the last timed step
+returned, as DIR/outL_rows.npy and DIR/outL_cols.npy (float32). The inputs are seeded too, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -115,8 +118,51 @@ def mix_roofline(workload, samples_per_step, ms_per_step, peaks_fp, sm_mhz, n_sm
                                            "of a step; DADD / DMUL / FADD / FMUL count like an FMA of their pipe" % w["samples_per_pass_capture"]}
 
 
+DUMP_BYTES = 64 << 20   # --dump-outputs writes at most this much in all
+
+
+def dump_sample(read_row, S, n, budget=DUMP_BYTES, seed=0):
+    """A fixed, seeded sample of a float32 [S][n] output that read_row(s) returns one row at a time, in two arrays of at most
+    budget / 2 bytes each: "rows", a few whole streams (a seeded window of each when a stream alone is larger), and
+    "cols", every stream at a few seeded sample positions. The sample depends on (S, n, budget, seed) only, so that runs
+    of two builds with the same arguments can be compared value for value. Returns ({name: array}, {what was sampled})."""
+    rng = np.random.default_rng(seed)
+    half = budget // 2 // 4
+    L = min(n, half)
+    streams = np.sort(rng.choice(S, size=max(1, min(S, half // L)), replace=False))
+    off = int(rng.integers(0, n - L + 1))
+    cols = np.sort(rng.choice(n, size=max(1, min(n, half // S)), replace=False))
+    rows = np.empty((len(streams), L), np.float32)
+    at = np.empty((S, len(cols)), np.float32)
+    for s in range(S):
+        row = read_row(s)
+        at[s] = row[cols]
+        k = np.searchsorted(streams, s)
+        if k < len(streams) and streams[k] == s:
+            rows[k] = row[off:off + L]
+    return {"rows": rows, "cols": at}, {"streams": streams.tolist(), "row_offset": off, "row_length": L, "cols": len(cols),
+                                        "seed": seed}
+
+
+def dump_outputs(eng, do, S, n, group, out_dir):
+    """--dump-outputs: writes a sample of what the last timed step left in the output buffer `do` (outL, float32 [S][n] on
+    the device) as out_dir/outL_rows.npy and out_dir/outL_cols.npy (see dump_sample); with several ranks each writes its
+    own shard's sample as rank<r>_outL_*.npy, and the ranks share the size budget."""
+    def read_row(s):
+        row = np.empty(n, np.float32)
+        eng._check(eng.lib.vp_memcpy_d2h(eng.h, row.ctypes.data, C.c_void_p(do + s * n * 4), n * 4))
+        return row
+    arrays, what = dump_sample(read_row, S, n, budget=DUMP_BYTES // group.world)
+    os.makedirs(out_dir, exist_ok=True)
+    prefix = "rank%d_" % group.rank if group.world > 1 else ""
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, "%soutL_%s.npy" % (prefix, k)), a)
+    return dict(what, dir=out_dir, arrays={prefix + "outL_" + k: list(a.shape) for k, a in arrays.items()})
+
+
 def run_sub(vp, args, name, group, peaks_fp, sm_mhz):
-    """Short device-resident run of another BASELINE configuration (5 timed steps) for the driver-observed line."""
+    """Short device-resident run of another BASELINE configuration (--warmup and --steps as given), for the result line's
+    other_workloads."""
     wl = WORKLOADS[name]
     fs, B = wl["fs"], wl["B"]
     n = int(fs * wl["seconds"]) // B * B
@@ -127,11 +173,11 @@ def run_sub(vp, args, name, group, peaks_fp, sm_mhz):
         nb = S * n * 4
         dv, dl, do = eng.device_alloc(nb), eng.device_alloc(nb), eng.device_alloc(nb)
         eng.synth_device(0, group.rank * S, S, n, n, dv, dl, None)
-        for _ in range(3):
+        for _ in range(args.warmup):
             eng.reset()
             eng.process_device(n // B, dv, dl, None, do, None, n, sync=False)
         eng.sync()
-        steps = 5
+        steps = args.steps
         eng.timer_record(0)
         for _ in range(steps):
             eng.reset()
@@ -142,7 +188,7 @@ def run_sub(vp, args, name, group, peaks_fp, sm_mhz):
         sm = slot_model(eng.sizes, prm)
         slots = (sm["voc_per_sample"] if prm.vocBool else 0.0) + (sm["pitch_per_sample"] if prm.pitchBool else 0.0)
         ms = 1e3 * sec / steps
-        res = {"workload": wl["desc"], "value": S * n / fs * steps / sec, "unit": "audio-s/s", "ms_per_step": ms, "steps": steps, "warmup": 3,
+        res = {"workload": wl["desc"], "value": S * n / fs * steps / sec, "unit": "audio-s/s", "ms_per_step": ms, "steps": steps, "warmup": args.warmup,
                "streams": S, "seconds_per_stream": n / fs,
                "chain_frac": slots * S * n * steps / sec / peaks_fp["fp32_fma_per_s"], "slots_per_sample": slots}
         mx = mix_roofline(name, float(S) * n, ms, peaks_fp, sm_mhz)
@@ -485,6 +531,7 @@ def run_engine(args, wl, group):
     clocks = sampler.window(t0, t1)
     audio_rank = S * n / fs * args.steps
     value, t_max, audio_total = vp.shard.aggregate_throughput(group, audio_rank, dev_s)
+    dump = dump_outputs(eng, do, S, n, group, args.dump_outputs) if args.dump_outputs else None
 
     # ---- parity at the benchmarked size: a spread of streams of the LAST timed step, full length, against the reference
     # on the host cores (oracle/_ref, else the C port). Test infrastructure used as the checker only.
@@ -561,7 +608,7 @@ def run_engine(args, wl, group):
             ths = [threading.Thread(target=quantise, args=(pr,)) for pr in ((qv, hv.array), (ql, hl.array))]
             [t.start() for t in ths]
             [t.join() for t in ths]
-            ksteps = max(1, min(args.steps, 5))
+            ksteps = args.steps
             eng.reset()
             eng.process_host_pcm16_ptrs(nBlocks, hv.ptr, hl.ptr, None, ho.ptr, None, n)
             group.barrier()
@@ -686,6 +733,8 @@ def run_engine(args, wl, group):
             line["parity"] = parity
         if cpu is not None:
             line["cpu_baseline"] = cpu
+        if dump is not None:
+            line["dump_outputs"] = dump
     eng.close()
     if group.world == 1 and not args.no_sub and not args.streams and args.workload == "chain48":
         # the other BASELINE configurations, driver-observed: chain @ 44.1 kHz is the north_star target line
@@ -817,7 +866,13 @@ def main():
     ap.add_argument("--stream-blocks", type=int, default=1500, help="blocks timed by the streaming latency test")
     ap.add_argument("--no-stream", action="store_true", help="skip the streaming (p99 block latency) sub-test")
     ap.add_argument("--stream-only", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed, seeded sample (at most 64 MB) of the output of the last timed step as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "engine" or args.stream_only):
+        ap.error("--dump-outputs writes the outputs of the engine's batch run: not with --impl reference or --stream-only")
     if args.warmup < 3 and args.impl == "engine":
         print("note: --warmup < 3 breaks the timing rules; use it for smoke runs only", file=sys.stderr)
     wl = dict(WORKLOADS[args.workload])

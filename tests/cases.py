@@ -85,6 +85,21 @@ KAT_MARKS = {
 }
 KAT_PERIOD, KAT_NOTE, KAT_BETA, KAT_PERIODNEW = 221, 6, 0.9822107863034768, 225
 
+# (fs, B, keyPitch, flavour) of tests/test_oracle.py::test_oracle_bit_exact_vs_reference_build: block sizes and rates the
+# golden fixtures above do not cover. Their pins are in tests/golden/reference_build_pins.json.
+REF_BUILD_CASES = [(44100.0, 64, 3, 0), (48000.0, 1000, 12, 1), (44100.0, 128, 0, 0)]
+
+
+def ref_build_inputs(vp, fs, B, flavour):
+    """(voice, synthL, synthR) float32 [n] of a REF_BUILD_CASES entry: 1.5 s of whole blocks."""
+    n = int(fs * 1.5) // B * B
+    v, l, r = vp.synth_host(fs, 1, n, flavour=flavour, first_stream=40 + B)
+    return v[0], l[0], r[0]
+
+
+def ref_build_key(fs, B, key, flavour):
+    return "fs=%g,B=%d,key=%d,flavour=%d" % (fs, B, key, flavour)
+
 
 def case_schedule(case):
     """[(block, cumulative parameter dict), ...] of a case ('schedule' entries override what is in force so far)."""

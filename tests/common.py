@@ -1,5 +1,6 @@
 """Shared helpers of the parity tests: the SURVEY App. E known-answer inputs,
 error metrics, decision comparison, golden-fixture access."""
+import hashlib
 import json
 import os
 import zlib
@@ -157,6 +158,22 @@ def golden_index():
 
 def golden_load(name):
     return np.load(os.path.join(GOLDEN, name + ".npz"))
+
+
+def sha256(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def reference_pin(r):
+    """A run of the reference (or of the oracle) in the form tests/golden/reference_build_pins.json stores it: both output
+    channels by SHA-256 of their float bytes, the sizes, and every pitch decision in full."""
+    return {"outL_sha256": sha256(r["outL"]), "outR_sha256": sha256(r["outR"]), "n": int(len(r["outL"])),
+            "sizes": r["sizes"], "decisions": oracle_decisions(r["pitch"])}
+
+
+def reference_pins():
+    with open(os.path.join(GOLDEN, "reference_build_pins.json")) as f:
+        return json.load(f)
 
 
 def reference_runs(jobs, threads=None):

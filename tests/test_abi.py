@@ -5,6 +5,8 @@ import ctypes as C
 import glob
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -63,15 +65,29 @@ def test_bad_arguments_are_codes_not_crashes(vp):
     assert lib.vp_stage_name(0) == b"gate" and lib.vp_stage_name(99) == b""
 
 
+NO_DEVICE_CHECK = """
+import ctypes as C
+import sys
+sys.path.insert(0, %r)
+import vocoderproject_b200 as vp
+lib = vp.load_library()
+assert lib.vp_device_count() == 0, lib.vp_device_count()
+h = C.c_void_p()
+assert lib.vp_engine_create(C.byref(h), 0) == vp.VP_E_CUDA and not h.value
+try:
+    vp.Engine(44100.0, 1024, 1, 4)
+except vp.EngineError as ex:
+    assert ex.code == vp.VP_E_CUDA, ex.code
+else:
+    raise AssertionError("an engine was created without a device")
+"""
+
+
 def test_no_cpu_fallback_without_a_device(vp):
-    lib = vp.load_library()
-    if lib.vp_device_count() > 0:
-        pytest.skip("a CUDA device is present")
-    h = C.c_void_p()
-    assert lib.vp_engine_create(C.byref(h), 0) == vp.VP_E_CUDA and not h.value
-    with pytest.raises(vp.EngineError) as ei:
-        vp.Engine(44100.0, 1024, 1, 4)
-    assert ei.value.code == vp.VP_E_CUDA
+    """In a child process that sees no CUDA device (CUDA_VISIBLE_DEVICES empty), so that it holds on a GPU machine too."""
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    res = subprocess.run([sys.executable, "-c", NO_DEVICE_CHECK % ROOT], env=env, capture_output=True, text=True, timeout=120)
+    assert res.returncode == 0, res.stdout + res.stderr
 
 
 def test_missing_library_fails_loudly(vp, tmp_path):
