@@ -9,7 +9,10 @@
  * ABI; INTEGRATION.md shows the PluginProcessor-side binding.
  *
  * Semantics. One "stream" is one plug-in instance (1 mono voice + stereo
- * side-chain in, stereo out). vp_engine_prepare is prepareToPlay(sampleRate,
+ * side-chain in, stereo out). Each stream has its own key and gains
+ * (vp_stream_params, vp_engine_set_stream_params); the remaining parameters
+ * (LPC orders, vocBool / pitchBool, window, mode) are one set per engine.
+ * vp_engine_prepare is prepareToPlay(sampleRate,
  * samplesPerBlock) for every stream; each vp_engine_process* call is, per
  * stream, nBlocks further consecutive processBlock calls. Results do
  * depend (sparsely) on samplesPerBlock exactly as in the reference (whole-ring
@@ -53,6 +56,15 @@ typedef struct vp_params {
     int vocBool;     /* default 1 */
 } vp_params;
 
+/* The per-instance part of vp_params: what one stream's plug-in instance holds in its parameter tree and the engine reads
+ * per stream. Only these five are per stream: the others (lpcVoice, lpcSynth, lpcPitch, vocBool, pitchBool, the window and
+ * the mode) stay per engine, because the frame grids are host state every stream shares (a bypassed block freezes them) and
+ * the orders select the tuned kernels and size the coefficient rows. 20 bytes. */
+typedef struct vp_stream_params {
+    float gainPitch, gainVoice, gainSynth, gainVoc; /* dB, [-60, 6]; the dry paths are on above -59 dB */
+    int keyPitch;                                   /* 0..12 */
+} vp_stream_params;
+
 /* Sizes prepareToPlay derives from the sample rate
  * (PluginProcessor.cpp:160-176, PitchProcess.cpp:100-107, MyBuffer.cpp:46-48). */
 typedef struct vp_sizes {
@@ -62,7 +74,7 @@ typedef struct vp_sizes {
     int latency, keep;         /* plug-in latency, samplesToKeep */
     int inSize, outSize;       /* MyBuffer ring lengths for this block size */
     int anCap;                 /* capacity of the pitch-mark vectors */
-    int nFreq;                 /* entries in the note table for keyPitch */
+    int nFreq;                 /* entries in the note table for the engine's keyPitch (vp_params) */
 } vp_sizes;
 
 /* Per pitch frame decisions (one record per processChunkStart call,
@@ -81,7 +93,7 @@ typedef struct vp_pitch_frame {
     int32_t period;           /* detected period in samples (0 = unvoiced) */
     int32_t periodPsola;      /* period else prevVoicedPeriod (PitchProcess.cpp:669-672) */
     int32_t periodNew;        /* synthesis mark spacing */
-    int32_t note;             /* snapped note index in the key's table, -1 if none */
+    int32_t note;             /* snapped note index in the table of the stream's key, -1 if none */
     int32_t nAn, nSt;
     int32_t anStale;          /* storage slot anMarks[nAn] (PitchProcess.cpp:818) */
     int32_t nAnOv;
@@ -125,8 +137,20 @@ int vp_engine_prepare(vp_engine* e, double sampleRate, int samplesPerBlock, int 
  * orders at prepare), vocBool / pitchBool per block: a block with vocBool off skips VocoderProcess::process (its frame grid
  * freezes relative to the block, frames in flight still come out), a block with pitchBool off is PitchProcess::silence()
  * (PluginProcessor.cpp:214-221, PitchProcess.cpp:146-158). lpcPitch is read in PitchProcess::prepare only (:70): a change on
- * a running stream is ignored until the next vp_engine_prepare, as in the reference. */
+ * a running stream is ignored until the next vp_engine_prepare, as in the reference.
+ * The five per-instance fields (gainPitch, gainVoice, gainSynth, gainVoc, keyPitch) are written to EVERY stream, replacing
+ * what vp_engine_set_stream_params set: a caller that never sets streams one by one has one parameter set for the batch. */
 int vp_engine_set_params(vp_engine* e, const vp_params* p);
+/* Per-stream key and gains: streams firstStream .. firstStream + count - 1 take p[0 .. count). Valid after vp_engine_prepare,
+ * which sets every stream from the engine's vp_params (VP_E_STATE before). A range outside [0, nStreams) is VP_E_ARG; a
+ * value outside the plug-in's range is VP_E_RANGE, and then no stream changes. A new value takes effect at the next process
+ * call of those streams, where the reference reads it (vp_engine_set_params): gainVoc per vocoder frame, gainPitch per
+ * emitted chunk, gainVoice / gainSynth per block, keyPitch per pitch frame. vp_engine_reset keeps the values (a plug-in's
+ * parameter tree survives prepareToPlay). Setting the values a stream already has costs nothing. The table goes to the
+ * device with the next process call: a call already issued (vp_engine_process_device is asynchronous) keeps the values it
+ * was issued with. */
+int vp_engine_set_stream_params(vp_engine* e, int firstStream, int count, const vp_stream_params* p);
+int vp_engine_get_stream_params(const vp_engine* e, int firstStream, int count, vp_stream_params* out);
 /* Behaviour at the places where the reference's C++ has undefined behaviour (SURVEY.md App. B U1-U6):
  *   VP_MODE_PARITY  (default) what the reference build actually does: the stale vector slot of PitchProcess.cpp:818 and the
  *                   popped table slot of Notes.cpp:99 are modelled, the other sites keep going and the frame is flagged VP_PF_UB;
@@ -186,7 +210,7 @@ int vp_grid_plan(double sampleRate, int samplesPerBlock, int nCalls, const int* 
  * heard through the dry side-chain mix, gainSynth > -59 dB). When it is given its
  * ring is carried on every call whatever gainSynth is, as in the reference
  * (MyBuffer.cpp:69-92), so gainSynth can be automated on mid-stream. outR may be
- * NULL (then only L is written; L == R whenever gainSynth <= -59 dB).
+ * NULL (then only L is written; L == R for every stream whose gainSynth <= -59 dB).
  * The outputs must NOT overlap the inputs (no in-place use: the mix reads the
  * delayed inputs while the outputs are being written) -- VP_E_ARG otherwise.
  * Asynchronous on the engine's stream; vp_engine_sync waits.
@@ -215,9 +239,11 @@ int vp_engine_sync(vp_engine* e);
 
 /* Low-latency streaming, one host block per call (BASELINE config 5). The engine owns pinned host buffers
  * voice / synthL / outL, each float[nStreams][samplesPerBlock]: fill the inputs, call vp_engine_stream_block, read
- * outL when it returns (L == R; gainSynth must be off; synthR is not carried). Equivalent to
+ * outL when it returns (L == R; gainSynth must be off on every stream, else VP_E_ARG; synthR is not carried). Equivalent to
  * vp_engine_process_host(e, 1, ...). The block's H2D copies, kernels and D2H copy are replayed from a CUDA graph
- * captured the first time each block phase (position of the block on the frame grids) occurs. */
+ * captured the first time each block phase (position of the block on the frame grids) occurs. Per-stream key and gain
+ * changes between blocks need no new capture (the table is uploaded before the graph is launched); whether some stream has
+ * the dry voice on is part of the graph's identity (it selects the mix kernel). */
 int vp_engine_stream_buffers(vp_engine* e, float** voice, float** synthL, float** outL);
 int vp_engine_stream_block(vp_engine* e);
 int vp_engine_stream_stats(const vp_engine* e, uint64_t* graphLaunches, uint64_t* graphCaptures);

@@ -31,6 +31,7 @@ ABI_SYMBOLS = [
     "vp_synth_host", "vp_synth_device", "vp_measure_peaks", "vp_engine_timing_reset", "vp_engine_timer_record",
     "vp_engine_timer_elapsed_ms", "vp_engine_last_timing_counts", "vp_measure_peaks2", "vp_engine_reset", "vp_engine_stream_buffers", "vp_engine_stream_block",
     "vp_engine_stream_stats", "vp_engine_get_info", "vp_engine_reserve_orders", "vp_grid_plan", "vp_engine_set_mode", "vp_engine_process_host_pcm16", "vp_engine_set_window",
+    "vp_engine_set_stream_params", "vp_engine_get_stream_params",
 ]
 
 
@@ -38,6 +39,28 @@ class Params(C.Structure):
     _fields_ = [("gainPitch", C.c_float), ("gainVoice", C.c_float), ("gainSynth", C.c_float),
                 ("gainVoc", C.c_float), ("lpcVoice", C.c_int), ("lpcPitch", C.c_int), ("lpcSynth", C.c_int),
                 ("keyPitch", C.c_int), ("pitchBool", C.c_int), ("vocBool", C.c_int)]
+
+
+class StreamParams(C.Structure):
+    """vp_stream_params: the per-instance part of Params (key and gains of one stream)."""
+    _fields_ = [("gainPitch", C.c_float), ("gainVoice", C.c_float), ("gainSynth", C.c_float), ("gainVoc", C.c_float),
+                ("keyPitch", C.c_int)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+STREAM_PARAM_FIELDS = tuple(k for k, _ in StreamParams._fields_)
+
+
+def stream_params(**kw):
+    """StreamParams with the plug-in's defaults (gains 0 / -60 / -60 / 0 dB, chromatic key), overridden by kw."""
+    p = StreamParams(0.0, -60.0, -60.0, 0.0, 12)
+    for k, v in kw.items():
+        if k not in STREAM_PARAM_FIELDS:
+            raise KeyError(k)
+        setattr(p, k, v)
+    return p
 
 
 class Sizes(C.Structure):
@@ -91,6 +114,8 @@ def load_library(path=None):
         "vp_last_error": (C.c_char_p, [vp]),
         "vp_engine_prepare": (i, [vp, dbl, i, i, i, sz]),
         "vp_engine_set_params": (i, [vp, C.POINTER(Params)]),
+        "vp_engine_set_stream_params": (i, [vp, i, i, C.POINTER(StreamParams)]),
+        "vp_engine_get_stream_params": (i, [vp, i, i, C.POINTER(StreamParams)]),
         "vp_engine_get_sizes": (i, [vp, C.POINTER(Sizes)]),
         "vp_engine_get_info": (i, [vp, C.POINTER(i), C.POINTER(i), C.POINTER(sz)]),
         "vp_engine_reserve_orders": (i, [vp, i, i]),
@@ -292,8 +317,34 @@ class Engine:
         self._check(self.lib.vp_engine_set_mode(self.h, int(mode)))
 
     def set_params(self, params):
+        """Engine-wide parameters; the key and gains go to every stream (replacing per-stream values)."""
         self._check(self.lib.vp_engine_set_params(self.h, C.byref(params)))
         self.params = params
+
+    def set_stream_params(self, first, items):
+        """Key and gains of streams first .. first + len(items) - 1; items are StreamParams or dicts (missing fields of a
+        dict keep the stream's current value). Takes effect with the next process call."""
+        items = list(items)
+        cur = self.stream_params(first, len(items)) if any(isinstance(it, dict) for it in items) else None
+        arr = (StreamParams * max(len(items), 1))()
+        for k, it in enumerate(items):
+            if isinstance(it, StreamParams):
+                C.memmove(C.byref(arr[k]), C.byref(it), C.sizeof(StreamParams))
+            else:
+                for f in STREAM_PARAM_FIELDS:
+                    setattr(arr[k], f, it[f] if f in it else cur[k][f])
+                for f in it:
+                    if f not in STREAM_PARAM_FIELDS:
+                        raise KeyError(f)
+        self._check(self.lib.vp_engine_set_stream_params(self.h, int(first), len(items), arr))
+
+    def stream_params(self, first=0, count=None):
+        """[dict] of the key and gains of streams first .. first + count - 1 (default: to the last stream)."""
+        if count is None:
+            count = self.n_streams - int(first)
+        arr = (StreamParams * max(int(count), 1))()
+        self._check(self.lib.vp_engine_get_stream_params(self.h, int(first), int(count), arr))
+        return [arr[k].as_dict() for k in range(int(count))]
 
     # ---- host-buffer API (what a plug-in host calls) ----
     def process(self, voice, synthL, synthR=None, want_right=True):

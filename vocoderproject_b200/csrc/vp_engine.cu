@@ -24,8 +24,9 @@ static const char* kStageNames[VP_NSTAGES] = {"gate", "voc_autocorr", "voc_levin
 thread_local cudaError_t g_vpLaunchError = cudaSuccess;  // per host thread: engines driven from different threads do not see each other's launch failures
 
 // ---------------------------------------------------------------------------
-// Frame grids: absolute positions on the delayed timeline. Every stream of an engine shares them (one parameter set per
-// engine), so this is plain host state; it is what VocoderProcess::startSample, PitchProcess::startSample and
+// Frame grids: absolute positions on the delayed timeline. Every stream of an engine shares them (the parameters that move
+// the grids -- vocBool, pitchBool, the LPC orders -- are per engine; only the key and the gains are per stream), so this is
+// plain host state; it is what VocoderProcess::startSample, PitchProcess::startSample and
 // PitchProcess::nChunk are in the reference, plus the bookkeeping of the frames that outlive the call they started in.
 // Pure host logic (no CUDA): vp_grid_plan runs it stand-alone.
 // ---------------------------------------------------------------------------
@@ -78,8 +79,18 @@ struct vp_engine {
     double *dWS = nullptr;  // synthesis window when it differs from the analysis window ("hann")
     int window = VP_WINDOW_SINE;
     double *dWV = nullptr, *dStP = nullptr, *dHann = nullptr, *dLutBeta = nullptr;
-    int *dHannOff = nullptr, *dLutPeriodNew = nullptr, *dLutNote = nullptr;
-    int lutKey = -1;
+    int *dHannOff = nullptr, *dLutPeriodNew = nullptr, *dLutNote = nullptr;  // note LUTs: [13 keys][tauMax + 1]
+    // ---- per-stream parameters (vp_engine_set_stream_params): what each stream's plug-in instance holds, in dB, and the
+    // table the kernels read (spTab on the host, dSP on the device, [S]). A changed table goes up through the pinned staging
+    // buffer spPinned on the engine's stream before the next call's first kernel; evSpUp marks when that copy has read it.
+    std::vector<vp_stream_params> sprm;
+    std::vector<VPStreamParam> spTab;
+    VPStreamParam *spPinned = nullptr, *dSP = nullptr;
+    cudaEvent_t evSpUp = nullptr;
+    bool spDirty = false;
+    bool anyDry = false, anySynth = false;  // some stream has a dry path (voice or side-chain) / the dry side-chain on
+    bool pitchGainUniform = true;           // every stream has the same gainPitch (k_pitch_iir then takes it as an argument)
+    bool capturing = false;                 // a streaming graph is being captured: nothing table-derived may be baked in
     // workspace (device), sized for Sc streams x maxBlocks
     uint8_t* dGate = nullptr;
     double* dGatePart = nullptr;
@@ -223,30 +234,32 @@ static int build_note_lut(vp_engine* e) {
     // closestFreq / beta / periodNew / note are pure functions of (period, key):
     // pitch = fS / tau (PitchProcess.cpp:441), Notes::getClosestFreq (Notes.cpp:79-110),
     // beta = closestFreq / pitch, periodNew = round(period / beta) (PitchProcess.cpp:594-596).
-    double freq[128];
-    const int nf = notes_table(e->prm.keyPitch, 100.0, 800.0, freq);
-    const int tauMax = e->sz.tauMax;
-    std::vector<double> beta(tauMax + 1, 1.0);
-    std::vector<int> pnew(tauMax + 1, 0), note(tauMax + 1, -1);
-    for (int tau = 1; tau <= tauMax; ++tau) {
-        const double pitch = e->fs / tau;
-        const int idx = (int)(std::lower_bound(freq, freq + nf, pitch) - freq);
-        int pick;
-        if (idx > 0) pick = (fabs(freq[idx] - pitch) <= fabs(freq[idx - 1] - pitch)) ? idx : idx - 1;  // idx == nf reads the popped slot
-        else pick = idx;
-        if (e->mode == VP_MODE_DEFINED && idx == nf) pick = nf - 1;  // above the table the closest note is the last one
-        const double closest = freq[pick];
-        beta[tau] = closest / pitch;
-        pnew[tau] = (int)round(tau / beta[tau]);
-        note[tau] = pick;
+    // One row per key (every stream reads the row of its own key); the rows depend on the mode (Notes.cpp:99, U6).
+    const int tauMax = e->sz.tauMax, row = tauMax + 1;
+    std::vector<double> beta((size_t)13 * row, 1.0);
+    std::vector<int> pnew((size_t)13 * row, 0), note((size_t)13 * row, -1);
+    for (int key = 0; key <= 12; ++key) {
+        double freq[128];
+        const int nf = notes_table(key, 100.0, 800.0, freq);
+        for (int tau = 1; tau <= tauMax; ++tau) {
+            const double pitch = e->fs / tau;
+            const int idx = (int)(std::lower_bound(freq, freq + nf, pitch) - freq);
+            int pick;
+            if (idx > 0) pick = (fabs(freq[idx] - pitch) <= fabs(freq[idx - 1] - pitch)) ? idx : idx - 1;  // idx == nf reads the popped slot
+            else pick = idx;
+            if (e->mode == VP_MODE_DEFINED && idx == nf) pick = nf - 1;  // above the table the closest note is the last one
+            const double closest = freq[pick];
+            const size_t i = (size_t)key * row + tau;
+            beta[i] = closest / pitch;
+            pnew[i] = (int)round(tau / beta[i]);
+            note[i] = pick;
+        }
     }
     int rc;
     if ((rc = upload(e, &e->dLutBeta, beta))) return rc;
     if ((rc = upload(e, &e->dLutPeriodNew, pnew))) return rc;
     if ((rc = upload(e, &e->dLutNote, note))) return rc;
-    e->lutKey = e->prm.keyPitch;
     e->lutMode = e->mode;
-    e->sz.nFreq = nf;
     return VP_OK;
 }
 
@@ -301,7 +314,8 @@ static void free_workspace(vp_engine* e) {
                       (void**)&e->cFrames, (void**)&e->cMarks, (void**)&e->oAV, (void**)&e->oAS, (void**)&e->oEeS, (void**)&e->oG};
     for (void** p : cptrs) if (*p) { cudaFree(*p); *p = nullptr; }
     for (int i = 0; i < 2; ++i) for (int j = 0; j < 3; ++j) if (e->cHist[i][j]) { cudaFree(e->cHist[i][j]); e->cHist[i][j] = nullptr; }
-    void** ptrs[] = {(void**)&e->dGate, (void**)&e->dRV, (void**)&e->dRS, (void**)&e->dAV, (void**)&e->dAS, (void**)&e->dEeV,
+    if (e->spPinned) { cudaFreeHost(e->spPinned); e->spPinned = nullptr; }
+    void** ptrs[] = {(void**)&e->dSP, (void**)&e->dGate, (void**)&e->dRV, (void**)&e->dRS, (void**)&e->dAV, (void**)&e->dAS, (void**)&e->dEeV,
                      (void**)&e->dEeS, (void**)&e->dG, (void**)&e->dGs, (void**)&e->dPeriod, (void**)&e->dList, (void**)&e->dListCount,
                      (void**)&e->dYFlags, (void**)&e->dFrames, (void**)&e->dAP, (void**)&e->dOutE, (void**)&e->dOutV,
                      (void**)&e->dOutP, (void**)&e->dFramesAll, (void**)&e->dGateAll, (void**)&e->dEeVAll, (void**)&e->dEeSAll,
@@ -339,7 +353,8 @@ extern "C" int vp_engine_create(vp_engine** out, int device) {
         cudaStreamCreateWithFlags(&e->st2, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->evFork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->evJoin, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreate(&e->evT0) != cudaSuccess || cudaEventCreate(&e->evT1) != cudaSuccess) {
+        cudaEventCreate(&e->evT0) != cudaSuccess || cudaEventCreate(&e->evT1) != cudaSuccess ||
+        cudaEventCreateWithFlags(&e->evSpUp, cudaEventDisableTiming) != cudaSuccess) {
         cudaGetLastError();
         delete e;
         return VP_E_CUDA;
@@ -377,7 +392,7 @@ extern "C" void vp_engine_destroy(vp_engine* e) {
     cudaEventDestroy(e->evT0); cudaEventDestroy(e->evT1);
     for (int i = 0; i < 8; ++i) cudaEventDestroy(e->evTimer[i]);
     for (auto ev : e->evSide) cudaEventDestroy(ev);
-    cudaEventDestroy(e->evFork); cudaEventDestroy(e->evJoin);
+    cudaEventDestroy(e->evFork); cudaEventDestroy(e->evJoin); cudaEventDestroy(e->evSpUp);
     for (int i = 0; i < 2; ++i) { cudaEventDestroy(e->evYin[i]); cudaEventDestroy(e->evMarks[i]); cudaEventDestroy(e->evSideDone[i]); cudaEventDestroy(e->evMix[i]); }
     cudaStreamDestroy(e->st); cudaStreamDestroy(e->stIn); cudaStreamDestroy(e->stOut); cudaStreamDestroy(e->st2);
     delete e;
@@ -385,13 +400,15 @@ extern "C" void vp_engine_destroy(vp_engine* e) {
 
 extern "C" const char* vp_last_error(const vp_engine* e) { return e ? e->err.c_str() : "null engine"; }
 
+static bool gain_ok(float g) { return g >= -60.0f && g <= 6.0f; }  // (false for NaN)
+
 static int check_params(const vp_params* p) {
     if (!p) return VP_E_ARG;
     if (p->lpcVoice < 2 || p->lpcVoice > 100 || p->lpcPitch < 2 || p->lpcPitch > 100 || p->lpcSynth < 2 || p->lpcSynth > 30)
         return VP_E_RANGE;
     if (p->keyPitch < 0 || p->keyPitch > 12) return VP_E_RANGE;
     const float gs[4] = {p->gainPitch, p->gainVoice, p->gainSynth, p->gainVoc};
-    for (float g : gs) if (!(g >= -60.0f && g <= 6.0f)) return VP_E_RANGE;
+    for (float g : gs) if (!gain_ok(g)) return VP_E_RANGE;
     return VP_OK;
 }
 
@@ -433,11 +450,80 @@ extern "C" int vp_engine_reserve_orders(vp_engine* e, int maxLpcVoice, int maxLp
     return VP_OK;
 }
 
+static VPStreamParam stream_table_entry(const vp_stream_params& p) {
+    VPStreamParam q;
+    memset(&q, 0, sizeof q);
+    q.gainVocF = db_to_gain(p.gainVoc); q.gainPitchF = db_to_gain(p.gainPitch);
+    q.gainVoiceF = db_to_gain(p.gainVoice); q.gainSynthF = db_to_gain(p.gainSynth);
+    q.key = p.keyPitch;
+    q.dryOn = p.gainVoice > -59.0f; q.synthOn = p.gainSynth > -59.0f;
+    return q;
+}
+
+// streams [first, first + count) take the values p[0 .. count); only a changed table entry makes the next call upload
+static void put_stream_params(vp_engine* e, int first, int count, const vp_stream_params* p, size_t pStep) {
+    bool changed = false;
+    for (int i = 0; i < count; ++i) {
+        const vp_stream_params& v = p[(size_t)i * pStep];
+        const VPStreamParam t = stream_table_entry(v);
+        e->sprm[first + i] = v;
+        if (memcmp(&e->spTab[first + i], &t, sizeof t) != 0) { e->spTab[first + i] = t; changed = true; }
+    }
+    if (!changed) return;
+    e->spDirty = true;
+    e->anyDry = e->anySynth = false;
+    e->pitchGainUniform = true;
+    for (const VPStreamParam& t : e->spTab) {
+        e->anyDry = e->anyDry || t.dryOn || t.synthOn;
+        e->anySynth = e->anySynth || t.synthOn;
+        e->pitchGainUniform = e->pitchGainUniform && t.gainPitchF == e->spTab[0].gainPitchF;
+    }
+}
+
+static vp_stream_params stream_part(const vp_params& p) {
+    vp_stream_params q;
+    q.gainPitch = p.gainPitch; q.gainVoice = p.gainVoice; q.gainSynth = p.gainSynth; q.gainVoc = p.gainVoc; q.keyPitch = p.keyPitch;
+    return q;
+}
+
+// The table goes up before the first kernel of a call, on the engine's stream. The staging buffer is rewritten only after
+// the previous upload has read it: a call that is still queued (vp_engine_process_device returns before it runs) keeps the
+// values it was issued with.
+static int upload_stream_params(vp_engine* e) {
+    if (!e->spDirty) return VP_OK;
+    const size_t bytes = e->spTab.size() * sizeof(VPStreamParam);
+    VP_CUDA_OK(cudaEventSynchronize(e->evSpUp));
+    memcpy(e->spPinned, e->spTab.data(), bytes);
+    VP_CUDA_OK(cudaMemcpyAsync(e->dSP, e->spPinned, bytes, cudaMemcpyHostToDevice, e->st));
+    VP_CUDA_OK(cudaEventRecord(e->evSpUp, e->st));
+    e->spDirty = false;
+    return VP_OK;
+}
+
+extern "C" int vp_engine_set_stream_params(vp_engine* e, int firstStream, int count, const vp_stream_params* p) {
+    if (!e || !p) return VP_E_ARG;
+    if (!e->prepared) return vp_err(e, VP_E_STATE, "vp_engine_prepare has not been called");
+    if (firstStream < 0 || count < 0 || firstStream > e->S - count) return vp_err(e, VP_E_ARG, "stream range outside [0, nStreams)");
+    for (int i = 0; i < count; ++i)
+        if (p[i].keyPitch < 0 || p[i].keyPitch > 12 || !gain_ok(p[i].gainPitch) || !gain_ok(p[i].gainVoice) ||
+            !gain_ok(p[i].gainSynth) || !gain_ok(p[i].gainVoc))
+            return vp_err(e, VP_E_RANGE, "parameter outside the plug-in's range");
+    put_stream_params(e, firstStream, count, p, 1);
+    return VP_OK;
+}
+
+extern "C" int vp_engine_get_stream_params(const vp_engine* e, int firstStream, int count, vp_stream_params* out) {
+    if (!e || !out) return VP_E_ARG;
+    if (!e->prepared) return VP_E_STATE;
+    if (firstStream < 0 || count < 0 || firstStream > e->S - count) return VP_E_ARG;
+    for (int i = 0; i < count; ++i) out[i] = e->sprm[firstStream + i];
+    return VP_OK;
+}
+
 extern "C" int vp_engine_set_params(vp_engine* e, const vp_params* p) {
     if (!e) return VP_E_ARG;
     int rc = check_params(p);
     if (rc) return vp_err(e, rc, "parameter outside the plug-in's range");
-    const bool keyChanged = p->keyPitch != e->prm.keyPitch;
     vp_params q = *p;
     const bool running = e->prepared && e->gs.blocksDone > 0;
     // lpcPitch is read in PitchProcess::prepare only (PitchProcess.cpp:70): a change on a running stream has no effect until
@@ -454,17 +540,20 @@ extern "C" int vp_engine_set_params(vp_engine* e, const vp_params* p) {
     }
     // Every parameter is read where the reference reads it: gains per block / frame / chunk, keyPitch per pitch frame, the
     // LPC orders per vocoder frame, vocBool / pitchBool per block (PluginProcessor.cpp:214-221).
-    p = &q;
-    if (memcmp(&e->prm, p, sizeof *p) != 0) {  // kernel arguments are baked into the captured graphs
+    // The engine-wide fields are baked into the captured graphs' kernel arguments; the per-instance ones are table data.
+    if (q.lpcVoice != e->prm.lpcVoice || q.lpcPitch != e->prm.lpcPitch || q.lpcSynth != e->prm.lpcSynth ||
+        q.pitchBool != e->prm.pitchBool || q.vocBool != e->prm.vocBool) {
         for (auto& kv : e->graphs) cudaGraphExecDestroy(kv.second);
         e->graphs.clear();
     }
-    e->prm = *p;
-    if (e->prepared && (keyChanged || e->lutKey != p->keyPitch)) {
-        cudaSetDevice(e->device);
-        cudaStreamSynchronize(e->st);
-        return build_note_lut(e);
+    e->prm = q;
+    if (e->prepared) {
+        double freq[128];
+        e->sz.nFreq = notes_table(q.keyPitch, 100.0, 800.0, freq);
     }
+    // the per-instance part goes to every stream (a caller that never sets streams one by one gets one parameter set)
+    const vp_stream_params sp = stream_part(q);
+    put_stream_params(e, 0, (int)e->sprm.size(), &sp, 0);
     return VP_OK;
 }
 
@@ -617,6 +706,14 @@ extern "C" int vp_engine_prepare(vp_engine* e, double fs, int B, int S, int maxB
     if ((rc = wsalloc(e, &e->cGainHist, (size_t)S * 20))) return rc;
     if ((rc = wsalloc(e, &e->cFrames, (size_t)S * VP_PC))) return rc;
     if ((rc = wsalloc(e, &e->cMarks, (size_t)S))) return rc;
+    // every stream starts from the engine's parameters
+    if ((rc = wsalloc(e, &e->dSP, (size_t)S))) return rc;
+    VP_CUDA_OK(cudaHostAlloc((void**)&e->spPinned, (size_t)S * sizeof(VPStreamParam), cudaHostAllocDefault));
+    e->sprm.assign((size_t)S, stream_part(e->prm));
+    e->spTab.assign((size_t)S, stream_table_entry(e->sprm[0]));
+    e->spDirty = true;
+    e->anyDry = e->spTab[0].dryOn || e->spTab[0].synthOn; e->anySynth = e->spTab[0].synthOn != 0;
+    e->pitchGainUniform = true;
     e->capV = capV; e->capS = capS; e->capP = capP;
     if ((rc = reset_state(e))) return rc;
     e->launches = e->yinRechecked = e->yinFrames = 0;
@@ -671,9 +768,6 @@ static int make_geom(vp_engine* e, int nBlocks, size_t stride, VPGeom* g) {
     g->H = e->H;
     g->defined = e->mode == VP_MODE_DEFINED;
     grid_geom(e->gs, g);
-    g->gainVocF = db_to_gain(e->prm.gainVoc); g->gainPitchF = db_to_gain(e->prm.gainPitch);
-    g->gainVoiceF = db_to_gain(e->prm.gainVoice); g->gainSynthF = db_to_gain(e->prm.gainSynth);
-    g->dryOn = e->prm.gainVoice > -59.0f; g->synthOn = e->prm.gainSynth > -59.0f;
     g->yinEps = 1e-4;
     if (const char* ye = getenv("VP_YIN_EPS")) g->yinEps = atof(ye);
     return VP_OK;
@@ -709,7 +803,8 @@ struct PassCtx {
 static void pass_init(vp_engine* e, PassCtx& c, const VPGeom& gIO, int Sp, int streamBase, const float* voice, const float* synthL,
                       const float* synthR, float* outL, float* outR) {
     c.g = gIO;
-    c.tb = VPTables{e->dWV, e->dWS ? e->dWS : e->dWV, e->dStP, e->dHann, e->dHannOff, e->dLutBeta, e->dLutPeriodNew, e->dLutNote};
+    c.tb = VPTables{e->dWV, e->dWS ? e->dWS : e->dWV, e->dStP, e->dHann, e->dHannOff, e->dLutBeta, e->dLutPeriodNew, e->dLutNote,
+                    e->dSP + streamBase};
     c.Sp = Sp;
     c.sb = (size_t)streamBase;
     const int hc = e->histCur;
@@ -844,7 +939,9 @@ static int pass_P(vp_engine* e, PassCtx& c) {
         stage_mark(e, ST_PLPC);
         vp_launch_pitch_psola(st, g, c.tb, Sp, c.voice, e->dFrames, e->dAP, e->dOutE);
         stage_mark(e, ST_PFRAME);
-        vp_launch_pitch_iir(st, g, c.tb, Sp, e->dFrames, e->dAP, e->dOutE, e->dOutP);
+        // (a captured graph reads the table: a gain change between blocks must not need a new capture)
+        const bool uniform = e->pitchGainUniform && !e->capturing;
+        vp_launch_pitch_iir(st, g, c.tb, Sp, e->dFrames, e->dAP, e->dOutE, e->dOutP, uniform ? &e->spTab[0].gainPitchF : nullptr);
         stage_mark(e, ST_PIIR);
         e->launches += 4;
         e->yinFrames += (size_t)Sp * g.nFramesP;
@@ -882,7 +979,7 @@ static int pass_V(vp_engine* e, PassCtx& c, int part) {
     if (g.vocOn) {
         if (g.nFramesV > 0) {
             vp_launch_voc_levinson(st, g, c.tb, Sp, c.voice, c.synthL, e->dGate, e->dRV, e->dRS, e->dAV, e->dAS, e->dEeV, e->dEeS);
-            vp_launch_voc_gain(st, g, Sp, e->dEeV, e->dEeS, e->dG, e->dGs, e->cGainHist + sb * 20);
+            vp_launch_voc_gain(st, g, c.tb, Sp, e->dEeV, e->dEeS, e->dG, e->dGs, e->cGainHist + sb * 20);
             stage_mark(e, ST_VOC_LEV);
             e->launches += 2;
         }
@@ -927,7 +1024,7 @@ static int pass_M(vp_engine* e, PassCtx& c) {
     const size_t sb = c.sb;
     const int hc = e->histCur;
     const long long rowsP = g.nFramesP + VP_PC;
-    vp_launch_mix(st, g, Sp, c.voice, c.synthL, c.synthR, e->dOutV, e->dOutP, c.outL, c.outR);
+    vp_launch_mix(st, g, c.tb, e->anyDry, Sp, c.voice, c.synthL, c.synthR, e->dOutV, e->dOutP, c.outL, c.outR);
     e->launches++;
     stage_mark(e, ST_MIX);
     if (g.pitchMix) vp_launch_carry_out(st, e->cFrames + sb * VP_PC, e->dFrames, Sp, (int)sizeof(vp_pitch_frame), (int)sizeof(vp_pitch_frame), VP_PC, g.nFramesP, rowsP);
@@ -1178,6 +1275,7 @@ extern "C" int vp_engine_process_device(vp_engine* e, int nBlocks, const float* 
         if (ranges_overlap(outL, span, outR, span)) return vp_err(e, VP_E_ARG, "outL and outR must not overlap");
     }
     VP_CUDA_OK(cudaSetDevice(e->device));
+    if ((rc = upload_stream_params(e))) return rc;
     begin_call(e);
     VPGeom g;
     make_geom(e, nBlocks, stride, &g);
@@ -1234,7 +1332,7 @@ static int process_host_impl(vp_engine* e, int nBlocks, const void* voiceV, cons
     if (rc) return rc;
     VP_CUDA_OK(cudaSetDevice(e->device));
     const long long n = (long long)nBlocks * e->B;
-    const bool synthOn = e->prm.gainSynth > -59.0f;
+    const bool synthOn = e->anySynth;
     const size_t esz = pcm16 ? sizeof(int16_t) : sizeof(float);
     const char *voice = (const char*)voiceV, *synthL = (const char*)synthLV, *synthR = (const char*)synthRV;
     char *outL = (char*)outLV, *outR = (char*)outRV;
@@ -1254,7 +1352,7 @@ static int process_host_impl(vp_engine* e, int nBlocks, const void* voiceV, cons
         e->Sh = (int)Sh;
     }
     // the right side-chain travels whenever the caller has one (its ring is filled whatever gainSynth is); the right
-    // output only when the dry side-chain is mixed in (otherwise L == R)
+    // output only when some stream mixes the dry side-chain in (otherwise L == R; streams without it keep L == R)
     const bool haveR = synthR != nullptr;
     const size_t cnt = (size_t)e->Sh * (size_t)e->maxBlocks * e->B;
     if (haveR && !e->hIn[0][2])
@@ -1267,6 +1365,7 @@ static int process_host_impl(vp_engine* e, int nBlocks, const void* voiceV, cons
             for (int j = 0; j < ((synthOn && outR) ? 2 : 1); ++j) if (!e->pOut[i][j] && (rc = wsalloc(e, &e->pOut[i][j], cnt))) return rc;
         }
     }
+    if ((rc = upload_stream_params(e))) return rc;
     begin_call(e);
     e->sidePending = e->mixPending = false;
     VPGeom g;
@@ -1376,8 +1475,10 @@ extern "C" int vp_engine_stream_buffers(vp_engine* e, float** voice, float** syn
 extern "C" int vp_engine_stream_block(vp_engine* e) {
     if (!e) return VP_E_ARG;
     if (!e->prepared || !e->sHostV) return vp_err(e, VP_E_STATE, "call vp_engine_prepare and vp_engine_stream_buffers first");
-    if (e->prm.gainSynth > -59.0f) return vp_err(e, VP_E_ARG, "streaming mode carries side-chain channel 0 only: gainSynth must be off");
+    if (e->anySynth) return vp_err(e, VP_E_ARG, "streaming mode carries side-chain channel 0 only: gainSynth must be off on every stream");
     VP_CUDA_OK(cudaSetDevice(e->device));
+    // per-stream key and gains are table data: a change is uploaded here, outside the graph, and needs no new capture
+    { const int rc = upload_stream_params(e); if (rc) return rc; }
     begin_call(e);
     e->sidePending = e->mixPending = false;
     VPGeom g;
@@ -1386,13 +1487,14 @@ extern "C" int vp_engine_stream_block(vp_engine* e) {
     e->lastG = g;
     // everything that shapes the launch sequence or is baked into kernel arguments
     std::vector<long long> key = {e->gs.blocksDone > 0 ? 1 : 0, e->histCur, g.offV, g.offP, g.nFramesV, g.nFramesP, g.kV0, g.synV, g.synS,
-                                  g.vocOn, g.pitchOn, g.vocMix, g.pitchMix};
+                                  g.vocOn, g.pitchOn, g.vocMix, g.pitchMix, e->anyDry};
     for (int j = 0; j < VP_ORPH; ++j) { key.push_back(g.orphPos[j]); key.push_back(g.orphOrdV[j]); key.push_back(g.orphOrdS[j]); }
     for (int j = 0; j < VP_PC; ++j) { key.push_back(g.carryPosP[j]); key.push_back(g.carryLimP[j]); }
     auto it = e->graphs.find(key);
     if (it == e->graphs.end()) {
         const bool st = e->stageTiming;
         e->stageTiming = false;  // event queries make no sense inside a graph
+        e->capturing = true;
         const size_t bytes = (size_t)e->S * e->B * sizeof(float);
         cudaGraph_t graph = nullptr;
         VP_CUDA_OK(cudaStreamBeginCapture(e->st, cudaStreamCaptureModeGlobal));
@@ -1410,6 +1512,7 @@ extern "C" int vp_engine_stream_block(vp_engine* e) {
         }
         cudaError_t ce2 = cudaStreamEndCapture(e->st, &graph);
         e->stageTiming = st;
+        e->capturing = false;
         if (rc != VP_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
         if (ce != cudaSuccess) { if (graph) cudaGraphDestroy(graph); return vp_fail(e, ce, "stream capture", __FILE__, __LINE__); }
         if (ce2 != cudaSuccess) return vp_fail(e, ce2, "cudaStreamEndCapture", __FILE__, __LINE__);

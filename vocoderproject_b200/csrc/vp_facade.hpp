@@ -13,8 +13,8 @@
 // The DSP classes do not compute on the host. The call sequence of processBlock -- fillInputBuffers, VocoderProcess::
 // process, PitchProcess::process (or silence), addDryVoice, addSynth, fillOutputBuffer -- is recorded on the MyBuffer
 // and executed as ONE engine call (all CUDA kernels of the block for all streams) when fillOutputBuffer asks for the
-// block's output; the result is what the reference's sequence produces. Parameters are pushed (vp_params) instead of
-// pulled through audioProcPtr->treeState. Errors are exceptions (vpb200::Error) carrying the ABI's status code; there
+// block's output; the result is what the reference's sequence produces. Parameters are pushed (vp_params, and per stream
+// the key and gains of each instance's parameter tree, vp_stream_params) instead of pulled through audioProcPtr->treeState. Errors are exceptions (vpb200::Error) carrying the ABI's status code; there
 // is no CPU fallback.
 #pragma once
 #include <cmath>
@@ -110,7 +110,22 @@ public:
         engine.check(vp_engine_prepare(engine.h, sampleRate, B, S, maxBlocks, 0));
         beginBlock();
     }
-    void setParams(const vp_params& p) { params = p; engine.check(vp_engine_set_params(engine.h, &params)); }
+    // the engine-wide parameters; the key and gains go to every stream (and replace what setStreamParams set)
+    void setParams(const vp_params& p) {
+        params = p;
+        streamParams.clear();
+        engine.check(vp_engine_set_params(engine.h, &params));
+    }
+    // key and gains of streams first .. first + count - 1 (after prepare); kept until the next setParams
+    void setStreamParams(int first, int count, const vp_stream_params* p) {
+        engine.check(vp_engine_set_stream_params(engine.h, first, count, p));
+        if (streamParams.empty()) {
+            streamParams.resize((size_t)S);
+            engine.check(vp_engine_get_stream_params(engine.h, 0, S, streamParams.data()));
+        } else {
+            for (int i = 0; i < count; ++i) streamParams[(size_t)(first + i)] = p[i];
+        }
+    }
     // largest lpcVoice / lpcSynth that may be set while the streams run (before prepare; VocoderProcess.cpp:50-57 sizes its
     // vectors for the ends of the parameter ranges: 100 / 30)
     void setWindow(bool hann) { engine.check(vp_engine_set_window(engine.h, hann ? VP_WINDOW_HANN : VP_WINDOW_SINE)); }
@@ -133,6 +148,8 @@ public:
         p.gainVoice = dryVoiceDb;
         p.gainSynth = drySynthDb;
         engine.check(vp_engine_set_params(engine.h, &p));
+        // per-stream values set since the last setParams: pushed again after the broadcast above (unchanged values cost nothing)
+        if (!streamParams.empty()) engine.check(vp_engine_set_stream_params(engine.h, 0, S, streamParams.data()));
         engine.check(vp_engine_process_host(engine.h, blocks, inVoice, inSynthL, inSynthR, outL, outR, stride));
         beginBlock();
     }
@@ -146,6 +163,7 @@ private:
     friend class PitchProcess;
     void beginBlock() { vocRequested = pitchRequested = false; dryVoiceDb = drySynthDb = -60.0f; }
     vp_params params;
+    std::vector<vp_stream_params> streamParams;  // [S] once setStreamParams was called, else empty
     vp_sizes sizes{};
     int B = 0, S = 0, maxBlocks = 1, blocks = 1;
     double sampleRate = 0;
@@ -233,6 +251,11 @@ public:
     void processBlock(const float* voice, const float* synthL, const float* synthR, float* outL, float* outR, size_t stride,
                       int nBlocks = 1) {
         myBuffer.setParams(params);
+        // one parameter tree per instance: pushed after setParams, which broadcasts; each stream then has its own dry mix
+        if (!streamParams.empty()) {
+            if (streamParams.size() != (size_t)myBuffer.getNumStreams()) throw Error(VP_E_ARG, "streamParams must hold one entry per stream");
+            myBuffer.setStreamParams(0, (int)streamParams.size(), streamParams.data());
+        }
         myBuffer.fillInputBuffers(voice, synthL, synthR, stride, nBlocks);   // :212
         if (params.vocBool) vocoderProcess.process(myBuffer);                // :214-215
         if (params.pitchBool) pitchProcess.process(myBuffer);                // :218-221
@@ -243,6 +266,8 @@ public:
     }
 
     vp_params params;   // the ten plug-in parameters (PluginProcessor.cpp:37-73)
+    // optional, one entry per stream: that instance's key and gains (its value tree); empty = params' values for every stream
+    std::vector<vp_stream_params> streamParams;
     std::string windowType = "sine";  // the literal prepareToPlay passes to VocoderProcess::prepare (:173); "hann" = the class's other branch
     MyBuffer myBuffer;
     VocoderProcess vocoderProcess;

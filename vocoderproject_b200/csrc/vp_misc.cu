@@ -9,11 +9,13 @@
 // out = vocoder OLA + pitch OLA (+ gainVoice * delayed voice) (+ gainSynth *
 // delayed synth), cast to float. Output sample u carries input time u - latency.
 // ---------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_mix(VPGeom g, const float* __restrict__ voice, const float* __restrict__ synthL,
-                                             const float* __restrict__ synthR, const float* __restrict__ outV,
-                                             const float* __restrict__ outP, float* __restrict__ outL,
-                                             float* __restrict__ outR) {
+// Each stream mixes with its own dry gains; a path that is off adds nothing (not 0 * x, which would turn -0 into +0).
+__global__ void __launch_bounds__(256) k_mix(VPGeom g, const VPStreamParam* __restrict__ sp, const float* __restrict__ voice,
+                                             const float* __restrict__ synthL, const float* __restrict__ synthR,
+                                             const float* __restrict__ outV, const float* __restrict__ outP,
+                                             float* __restrict__ outL, float* __restrict__ outR) {
     const int s = blockIdx.y;
+    const VPStreamParam p = sp[s];
     const size_t row = (size_t)s * g.stride, wrow = (size_t)s * g.wstride;
     const long long step = (long long)gridDim.x * blockDim.x;
     constexpr int MU = 4;  // independent loads in flight per thread and plane
@@ -33,13 +35,13 @@ __global__ void __launch_bounds__(256) k_mix(VPGeom g, const float* __restrict__
             if (g.vocMix) l += a[k];
             if (g.pitchMix) l += b[k];
             float r = l;
-            if (g.dryOn) {
-                const float d = g.gainVoiceF * vp_x(vp_row(voice, g.histV, s, g), u, g);
+            if (p.dryOn) {
+                const float d = p.gainVoiceF * vp_x(vp_row(voice, g.histV, s, g), u, g);
                 l += d; r += d;
             }
-            if (g.synthOn) {
-                l += g.gainSynthF * vp_x(vp_row(synthL, g.histS, s, g), u, g);
-                r += g.gainSynthF * (synthR ? vp_x(vp_row(synthR, g.histR, s, g), u, g) : vp_x(vp_row(synthL, g.histS, s, g), u, g));
+            if (p.synthOn) {
+                l += p.gainSynthF * vp_x(vp_row(synthL, g.histS, s, g), u, g);
+                r += p.gainSynthF * (synthR ? vp_x(vp_row(synthR, g.histR, s, g), u, g) : vp_x(vp_row(synthL, g.histS, s, g), u, g));
             }
             outL[row + u] = l;
             if (outR) outR[row + u] = r;
@@ -47,7 +49,7 @@ __global__ void __launch_bounds__(256) k_mix(VPGeom g, const float* __restrict__
     }
 }
 
-// The common case -- no dry paths, rows 16-byte aligned -- as 128-bit accesses with 32-bit indexing inside a row: 4 output
+// The common case -- no stream of the call with a dry path on, rows 16-byte aligned -- as 128-bit accesses with 32-bit indexing inside a row: 4 output
 // samples per thread and iteration for 2 loads, 4 adds and 1 (2) stores; the general kernel above spends ~57 instructions
 // per sample on 64-bit index arithmetic (ncu, profiles/ncu_mix_r02e.json), 2.9 % of the whole step's instruction issue.
 template <bool VOC, bool PITCH>
@@ -77,10 +79,10 @@ __global__ void __launch_bounds__(256) k_mix4(const float4* __restrict__ outV, c
     }
 }
 
-void vp_launch_mix(cudaStream_t st, const VPGeom& g, int S, const float* voice, const float* synthL,
+void vp_launch_mix(cudaStream_t st, const VPGeom& g, const VPTables& tb, bool anyDry, int S, const float* voice, const float* synthL,
                    const float* synthR, const float* outV, const float* outP, float* outL, float* outR) {
     auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
-    if (!g.dryOn && !g.synthOn && (g.n & 3) == 0 && (g.stride & 3) == 0 && (g.wstride & 3) == 0 && g.n / 4 < (1LL << 30) && al16(outV) &&
+    if (!anyDry && (g.n & 3) == 0 && (g.stride & 3) == 0 && (g.wstride & 3) == 0 && g.n / 4 < (1LL << 30) && al16(outV) &&
         al16(outP) && al16(outL) && al16(outR)) {
         const int n4 = (int)(g.n / 4);
         int bx = (n4 + 2 * 256 - 1) / (2 * 256);
@@ -100,7 +102,7 @@ void vp_launch_mix(cudaStream_t st, const VPGeom& g, int S, const float* voice, 
     if (bx > 4096) bx = 4096;
     if (bx < 1) bx = 1;
     dim3 grid((unsigned)bx, S);
-    VP_LAUNCH(k_mix<<<grid, 256, 0, st>>>(g, voice, synthL, synthR, outV, outP, outL, outR));
+    VP_LAUNCH(k_mix<<<grid, 256, 0, st>>>(g, tb.sp, voice, synthL, synthR, outV, outP, outL, outR));
 }
 
 // ---------------------------------------------------------------------------

@@ -828,6 +828,7 @@ __global__ void __launch_bounds__(128) k_marks(VPGeom g, VPTables tb, const floa
     const VPRow v = vp_row(voice, g.histV, s, g);
     const uint8_t* gt = gate + (size_t)s * g.nBlocks;
     const int L = g.L, hop = g.hopP, cap = g.anCap;
+    const int lut = tb.sp[s].key * (g.tauMax + 1);  // the note LUT row of this stream's key, read per pitch frame (Notes.cpp:79-110)
     // PitchProcess state (PitchProcess.cpp:76-92), carried from the previous call of this stream
     VPMarkState* cs = carry + s;
     int period = cs->period, prevPeriod = cs->prevPeriod, prevVoicedPeriod = cs->prevVoicedPeriod, periodNew = cs->periodNew;
@@ -984,9 +985,9 @@ __global__ void __launch_bounds__(128) k_marks(VPGeom g, VPTables tb, const floa
             if (nAn > 0) {
                 const int nStOv = __popc(__ballot_sync(0xffffffffu, lane < nPst && pst >= 0));
                 if (voiced) {
-                    beta = tb.lutBeta[period];
-                    periodNew = tb.lutPeriodNew[period];
-                    note = tb.lutNote[period];
+                    beta = tb.lutBeta[lut + period];
+                    periodNew = tb.lutPeriodNew[lut + period];
+                    note = tb.lutNote[lut + period];
                 } else {
                     periodNew = prevVoicedPeriod;
                 }
@@ -1520,10 +1521,13 @@ void vp_launch_pitch_psola(cudaStream_t st, const VPGeom& g, const VPTables& tb,
 #define PI_WARPS 2
 #define PI_ROW 36  // floats per tile row: 32 samples + 4 spare (16-byte aligned rows, conflict-free 128-bit accesses)
 
-template <int P>
+// STREAM_GAIN: each frame scales by its stream's gainPitch from the table; else every stream of the call has the same one,
+// passed as gpCall. Measured on the default workload (same-box A/B against the form that always reads the table): the
+// table form took this kernel from 18.9 to 19.8 ms per step, the argument form is at 18.9 again.
+template <int P, bool STREAM_GAIN>
 __global__ void __launch_bounds__(32 * PI_WARPS, 8) k_pitch_iir(VPGeom g, VPTables tb, const vp_pitch_frame* __restrict__ frames,
                                                              const double* __restrict__ aP, const float* __restrict__ outE,
-                                                             float* __restrict__ outP, long long nFramesTot) {
+                                                             float* __restrict__ outP, long long nFramesTot, double gpCall) {
     // Rows of 36 floats: 16-byte aligned (128-bit copies in, 128-bit reads / writes by the filter thread: a quarter-warp's 8
     // rows start 4 banks apart), and the 4 spare floats of a tout row carry that frame's output range and position for the
     // row-wise write-out. A shared-memory or shuffle instruction costs the scheduler ~3 cycles next to FP64 work
@@ -1570,7 +1574,7 @@ __global__ void __launch_bounds__(32 * PI_WARPS, 8) k_pitch_iir(VPGeom g, VPTabl
         if (nSteps == 0 || meta.y < meta.x) { meta.x = 0; meta.y = 0; meta.z = 0; }  // empty range: hi == lo (the write-out tests i - lo < hi - lo unsigned)
         *reinterpret_cast<int4*>(&tout[warp][lane][32]) = meta;
     }
-    const double gp = (double)g.gainPitchF;
+    const double gp = STREAM_GAIN ? (double)tb.sp[s].gainPitchF : gpCall;  // the frame's stream's gainPitch, read per emitted chunk (PitchProcess.cpp:336)
     const int nSlabs = (L + 31) / 32;
     int maxSteps = nSteps;
 #pragma unroll
@@ -1649,7 +1653,7 @@ __global__ void __launch_bounds__(32 * PI_WARPS, 8) k_pitch_iir(VPGeom g, VPTabl
 }
 
 void vp_launch_pitch_iir(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const vp_pitch_frame* frames,
-                         const double* aP, const float* outE, float* outP) {
+                         const double* aP, const float* outE, float* outP, const float* gainUniform) {
     const long long tot = (long long)S * (g.nFramesP + VP_PC);
     const unsigned grid = (unsigned)((tot + 32 * PI_WARPS - 1) / (32 * PI_WARPS));
     // a warp's 32 frame slots span at most 32 / (nFramesP + VP_PC) + 1 streams: their plane offsets relative to the first
@@ -1658,6 +1662,12 @@ void vp_launch_pitch_iir(cudaStream_t st, const VPGeom& g, const VPTables& tb, i
         if (g_vpLaunchError == cudaSuccess) g_vpLaunchError = cudaErrorInvalidValue;
         return;
     }
-    if (g.ordP == 15) VP_LAUNCH(k_pitch_iir<15><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot));
-    else VP_LAUNCH(k_pitch_iir<0><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot));
+    const double gp = gainUniform ? (double)*gainUniform : 0.0;
+    if (g.ordP == 15) {
+        if (gainUniform) VP_LAUNCH(k_pitch_iir<15, false><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot, gp));
+        else VP_LAUNCH(k_pitch_iir<15, true><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot, gp));
+    } else {
+        if (gainUniform) VP_LAUNCH(k_pitch_iir<0, false><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot, gp));
+        else VP_LAUNCH(k_pitch_iir<0, true><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot, gp));
+    }
 }

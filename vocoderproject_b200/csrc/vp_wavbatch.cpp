@@ -1,10 +1,11 @@
 // vp_wavbatch -- WAV front-end of the batch engine (SURVEY.md 8(f)#3): every line of a manifest is one plug-in
 // instance = one stream,
 //
-//     voice.wav  sidechain.wav  out.wav
+//     voice.wav  sidechain.wav  out.wav  [key=N] [gainVoc=dB] [gainPitch=dB] [gainVoice=dB] [gainSynth=dB]
 //
 // (voice: channel 0 is used, PluginProcessor.cpp:153-157 mono main bus; side-chain: stereo, a mono file feeds both
-// channels). All jobs run as ONE batch on the GPU through the facade's prepareToPlay / processBlock (vp_facade.hpp):
+// channels). The optional tokens are that instance's own key and gains: they override the command-line values for the
+// job, so files in different keys or with different mixes still run as one batch. All jobs run as ONE batch on the GPU through the facade's prepareToPlay / processBlock (vp_facade.hpp):
 // same sample rate for all files, shorter jobs are zero-padded to the longest and trimmed again on output.
 //
 //   vp_wavbatch manifest.txt [--block 1024] [--blocks-per-call 64] [--key 12] [--voc 0|1] [--pitch 0|1]
@@ -26,7 +27,30 @@
 #include "vp_facade.hpp"
 #include "vp_wav.hpp"
 
-struct Job { std::string voice, synth, out; vpb200::WavData v, s; };
+struct Job { std::string voice, synth, out; vpb200::WavData v, s; vp_stream_params sp; };
+
+// "name=value" tokens of a manifest line -> the job's per-instance parameters; false when any token is not one of them
+static bool parse_stream_tokens(std::istringstream& ls, vp_stream_params& sp, bool& any) {
+    std::string tok;
+    while (ls >> tok) {
+        const size_t eq = tok.find('=');
+        if (eq == std::string::npos || eq + 1 == tok.size()) return false;
+        const std::string name = tok.substr(0, eq), val = tok.substr(eq + 1);
+        char* end = nullptr;
+        const double x = strtod(val.c_str(), &end);
+        if (*end != '\0') return false;
+        if (name == "key") {
+            if (x != (double)(int)x) return false;
+            sp.keyPitch = (int)x;
+        } else if (name == "gainVoc") sp.gainVoc = (float)x;
+        else if (name == "gainPitch") sp.gainPitch = (float)x;
+        else if (name == "gainVoice") sp.gainVoice = (float)x;
+        else if (name == "gainSynth") sp.gainSynth = (float)x;
+        else return false;
+        any = true;
+    }
+    return true;
+}
 
 int main(int argc, char** argv) {
     int B = 1024, K = 64, device = 0;
@@ -51,7 +75,8 @@ int main(int argc, char** argv) {
         else if (!strcmp(argv[i], "--help")) {
             printf("usage: vp_wavbatch manifest.txt [--block B] [--blocks-per-call K] [--key 0..12] [--voc 0|1] [--pitch 0|1] "
                    "[--gain-voice dB] [--gain-synth dB] [--gain-voc dB] [--gain-pitch dB] [--pcm16] [--keep-latency] [--device d]\n"
-                   "manifest lines: voice.wav sidechain.wav out.wav\n");
+                   "manifest lines: voice.wav sidechain.wav out.wav [key=N] [gainVoc=dB] [gainPitch=dB] [gainVoice=dB] [gainSynth=dB]\n"
+                   "  (the tokens set that job's key and gains; they override --key / --gain-* for the job)\n");
             return 0;
         } else if (argv[i][0] != '-' && manifest.empty()) manifest = argv[i];
         else { fprintf(stderr, "unknown argument %s\n", argv[i]); return 2; }
@@ -59,6 +84,7 @@ int main(int argc, char** argv) {
     if (manifest.empty() || B <= 0 || K <= 0) { fprintf(stderr, "vp_wavbatch: no manifest (see --help)\n"); return 2; }
     try {
         std::vector<Job> jobs;
+        bool perJob = false;  // some line sets its own key or gains
         {
             std::ifstream mf(manifest);
             if (!mf) throw std::runtime_error("cannot open " + manifest);
@@ -69,6 +95,10 @@ int main(int argc, char** argv) {
                 if (!(ls >> j.voice)) continue;
                 if (j.voice[0] == '#') continue;
                 if (!(ls >> j.synth >> j.out)) throw std::runtime_error("manifest line needs three paths: " + line);
+                j.sp.gainPitch = prm.gainPitch; j.sp.gainVoice = prm.gainVoice; j.sp.gainSynth = prm.gainSynth;
+                j.sp.gainVoc = prm.gainVoc; j.sp.keyPitch = prm.keyPitch;
+                if (!parse_stream_tokens(ls, j.sp, perJob))
+                    throw std::runtime_error("manifest tokens after the paths are key=N gainVoc= gainPitch= gainVoice= gainSynth=: " + line);
                 jobs.push_back(std::move(j));
             }
         }
@@ -87,6 +117,8 @@ int main(int argc, char** argv) {
         vpb200::VocoderBatchProcessor proc(device);
         proc.params = prm;
         proc.prepareToPlay((double)fs, B, S, K);
+        if (perJob)
+            for (const Job& j : jobs) proc.streamParams.push_back(j.sp);
         const size_t lat = keepLatency ? 0 : (size_t)proc.getLatencySamples();
         const size_t m = (size_t)K * B;
         const size_t nCalls = (longest + lat + m - 1) / m;
