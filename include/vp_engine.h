@@ -185,6 +185,23 @@ int vp_engine_get_info(const vp_engine* e, int* streamsPerPass, int* historySamp
  * MyBuffer / VocoderProcess / PitchProcess keep between processBlock calls). */
 int vp_engine_reset(vp_engine* e);
 
+/* Per-stream counterpart of vp_engine_reset, for a host that hands a slot of a running batch to a new plug-in instance
+ * (user, track): streams[0 .. count) continue as streams that have received ZEROS on every input channel since
+ * vp_engine_prepare / vp_engine_reset -- their rings, histories, pitch marks and the frames of theirs still in flight are
+ * forgotten. The frame grids are shared by all streams (vocBool / pitchBool / LPC orders are per engine), so a reset stream
+ * keeps the batch's grid phase: it is exactly a freshly prepared instance only where the grids are in their prepare phase
+ * (no vocBool / pitchBool-off block since prepare, and blocksDone * samplesPerBlock a multiple of both frame hops -- every
+ * 3rd block at 44.1 kHz / 1024). Elsewhere it is what the reference's processBlock gives for zeros up to that block.
+ * Valid after vp_engine_prepare (VP_E_STATE before). count == 0 does nothing; count < 0, streams == NULL with count > 0, or
+ * any index outside [0, nStreams) is VP_E_ARG, and then nothing is queued. Duplicates, and repeated requests before one
+ * process call, act as one. The reset takes effect at the next process call of any kind (process_device, process_host,
+ * process_host_pcm16, stream_block), before its first kernel; a call already issued keeps the state it was issued with.
+ * Does not wait for the GPU. Keeps each stream's vp_stream_params, the engine-wide parameters, the grids, every other
+ * stream (bit for bit) and the records of the most recent call (get_pitch_frames / get_voc_frames); does not clear the
+ * failed mark of a half-done call (only vp_engine_reset / vp_engine_prepare do, and both drop pending stream resets).
+ * Streaming needs no new graph capture for it. Cost: one kernel launch in the next call, none when no reset is pending. */
+int vp_engine_reset_streams(vp_engine* e, const int* streams, int count);
+
 /* Host-only helper (no CUDA): the frame grids a sequence of process calls produces -- call c processes nBlocks[c] blocks
  * with params[c] in force (only vocBool, pitchBool, lpcVoice, lpcSynth matter). For hosts that want to know how many frame
  * records a call will report, and for the CPU tests of the grid bookkeeping. */

@@ -31,7 +31,7 @@ ABI_SYMBOLS = [
     "vp_synth_host", "vp_synth_device", "vp_measure_peaks", "vp_engine_timing_reset", "vp_engine_timer_record",
     "vp_engine_timer_elapsed_ms", "vp_engine_last_timing_counts", "vp_measure_peaks2", "vp_engine_reset", "vp_engine_stream_buffers", "vp_engine_stream_block",
     "vp_engine_stream_stats", "vp_engine_get_info", "vp_engine_reserve_orders", "vp_grid_plan", "vp_engine_set_mode", "vp_engine_process_host_pcm16", "vp_engine_set_window",
-    "vp_engine_set_stream_params", "vp_engine_get_stream_params",
+    "vp_engine_set_stream_params", "vp_engine_get_stream_params", "vp_engine_reset_streams",
 ]
 
 
@@ -142,6 +142,7 @@ def load_library(path=None):
         "vp_measure_peaks": (i, [vp, C.POINTER(dbl), C.POINTER(dbl)]),
         "vp_engine_timing_reset": (i, [vp, i]),
         "vp_engine_reset": (i, [vp]),
+        "vp_engine_reset_streams": (i, [vp, C.POINTER(i), i]),
         "vp_engine_stream_buffers": (i, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]),
         "vp_engine_stream_block": (i, [vp]),
         "vp_engine_stream_stats": (i, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
@@ -291,6 +292,13 @@ class Engine:
     def reset(self):
         """prepareToPlay again: forget every stream's history; the next process call starts at block 0."""
         self._check(self.lib.vp_engine_reset(self.h))
+
+    def reset_streams(self, streams):
+        """Hand the listed streams to new instances: from the next process call on, each continues as a stream that has
+        heard only silence since prepare (its key and gains are kept). The other streams are not touched."""
+        streams = [int(s) for s in streams]
+        arr = (C.c_int * max(len(streams), 1))(*streams)
+        self._check(self.lib.vp_engine_reset_streams(self.h, arr, len(streams)))
 
     # ---- low-latency streaming: one host block per call through pinned buffers and a CUDA graph per block phase ----
     def stream_buffers(self):

@@ -86,7 +86,9 @@ struct VPMarkState {
     int period, prevPeriod, prevVoicedPeriod, periodNew, voiced, prevVoiced, nAn, nSt;
     double beta;
     int an[VP_SLOTS], st[VP_SLOTS];
+    int pad[2];  // a whole number of 16-byte units per stream (k_reset_streams)
 };
+static_assert(sizeof(VPMarkState) % 16 == 0, "k_reset_streams writes 16-byte units");
 
 // One stream's input as seen by a call: x = the samples handed to this call, h = the H samples before them.
 struct VPRow {
@@ -241,6 +243,23 @@ void vp_launch_carry_out(cudaStream_t st, void* carry, const void* ws, int S, in
 // row `srcRow` of every stream's C-row carried store -> slot `dstSlot` of its D-slot store (same row bytes)
 void vp_launch_row_move(cudaStream_t st, void* dst, const void* src, int S, int rowBytes, int C, int srcRow, int D, int dstSlot);
 void vp_launch_marks_silence(cudaStream_t st, VPMarkState* carry, int S);
+// The per-stream state carried from call to call, as k_reset_streams sees it: arrays [nStreams][units * 16 bytes], each with
+// the value a stream that has heard only silence since prepare holds in it.
+#define VP_FILL_ZERO 0    // all bits zero
+#define VP_FILL_GATED 1   // doubles = -1.0: EeSynth of a gated vocoder frame (k_voc_levinson*), which no kernel synthesises
+#define VP_FILL_ONE_AT 2  // zeros, except double oneAt of each stream's run = 1.0 (VPMarkState::beta)
+#define VP_RESET_MAXSEG 16
+struct VPResetSeg {
+    void* base;
+    int units;  // 16-byte units per stream
+    int kind, oneAt;
+};
+struct VPResetSegs {
+    VPResetSeg seg[VP_RESET_MAXSEG];
+    int nSeg, unitsPerStream;
+};
+// one launch: the silent state of streams list[0 .. count) (list == NULL: streams 0 .. count - 1) in every segment
+void vp_launch_reset_streams(cudaStream_t st, const VPResetSegs& segs, const int* list, int count);
 // 16-bit PCM <-> float exactly as vp_wav.hpp converts on the host: x / 32768 in, clamp(rint(x * 32768)) out
 void vp_launch_pcm16_to_float(cudaStream_t st, float* dst, const int16_t* src, long long count);
 void vp_launch_float_to_pcm16(cudaStream_t st, int16_t* dst, const float* src, long long count);

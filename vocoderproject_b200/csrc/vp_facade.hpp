@@ -132,6 +132,9 @@ public:
     void reserveOrders(int maxLpcVoice, int maxLpcSynth) { engine.check(vp_engine_reserve_orders(engine.h, maxLpcVoice, maxLpcSynth)); }
     // prepareToPlay on a running instance: back to the freshly prepared state first
     void restart() { if (B > 0) engine.check(vp_engine_reset(engine.h)); }
+    // prepareToPlay for some instances of the running batch (a slot handed to a new user): from the next block on, each
+    // listed stream continues as one that has heard only silence since prepare; the others are not touched
+    void restartStreams(const int* streams, int count) { engine.check(vp_engine_reset_streams(engine.h, streams, count)); }
     const vp_params& getParams() const { return params; }
 
     // fillInputBuffers(voiceBuffer, synthBuffer): host rows [S][stride]; synth channel 1 may be null when gainSynth is off

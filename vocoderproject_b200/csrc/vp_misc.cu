@@ -162,6 +162,31 @@ void vp_launch_row_move(cudaStream_t st, void* dst, const void* src, int S, int 
                                                                                        rowBytes / 4, C, srcRow, D, dstSlot));
 }
 
+// ---------------------------------------------------------------------------
+// Silent state of listed streams (vp_engine_reset_streams; every stream at prepare / reset): what a stream holds that has
+// received zeros on every input since prepare. The engine lists the carried arrays and their silent values (VPResetSegs);
+// one launch fills all of them. Grid: x over a stream's 16-byte units of all segments, y over the listed streams.
+// ---------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_reset_streams(VPResetSegs segs, const int* __restrict__ list, int count) {
+    const int unit = blockIdx.x * blockDim.x + threadIdx.x;
+    if (unit >= segs.unitsPerStream) return;
+    int j = 0, u = unit;
+    while (u >= segs.seg[j].units) { u -= segs.seg[j].units; ++j; }
+    const VPResetSeg sg = segs.seg[j];
+    double2 v;
+    if (sg.kind == VP_FILL_ONE_AT) v = make_double2(2 * u == sg.oneAt ? 1.0 : 0.0, 2 * u + 1 == sg.oneAt ? 1.0 : 0.0);
+    else v.x = v.y = (sg.kind == VP_FILL_GATED) ? -1.0 : 0.0;
+    for (int i = blockIdx.y; i < count; i += gridDim.y) {
+        const size_t s = list ? (size_t)__ldg(list + i) : (size_t)i;
+        reinterpret_cast<double2*>(sg.base)[s * (size_t)sg.units + u] = v;
+    }
+}
+void vp_launch_reset_streams(cudaStream_t st, const VPResetSegs& segs, const int* list, int count) {
+    if (count <= 0 || segs.unitsPerStream <= 0) return;
+    const dim3 grid((unsigned)((segs.unitsPerStream + 255) / 256), (unsigned)std::min(count, 65535));
+    VP_LAUNCH(k_reset_streams<<<grid, 256, 0, st>>>(segs, list, count));
+}
+
 // PitchProcess::silence() (PitchProcess.cpp:146-158) for every stream: both mark vectors cleared (their storage keeps its
 // values), pitch = prevPitch = 0, period = prevPeriod = 0. prevVoicedPeriod, periodNew and beta are not touched.
 __global__ void __launch_bounds__(128) k_marks_silence(VPMarkState* __restrict__ carry, int S) {
