@@ -148,9 +148,37 @@ int vp_engine_set_params(vp_engine* e, const vp_params* p);
  * emitted chunk, gainVoice / gainSynth per block, keyPitch per pitch frame. vp_engine_reset keeps the values (a plug-in's
  * parameter tree survives prepareToPlay). Setting the values a stream already has costs nothing. The table goes to the
  * device with the next process call: a call already issued (vp_engine_process_device is asynchronous) keeps the values it
- * was issued with. */
+ * was issued with. For changes at arbitrary blocks inside one call see vp_engine_schedule_stream_params. */
 int vp_engine_set_stream_params(vp_engine* e, int firstStream, int count, const vp_stream_params* p);
+/* The values in force at the last block issued (after a call with scheduled changes: at its last block). */
 int vp_engine_get_stream_params(const vp_engine* e, int firstStream, int count, vp_stream_params* out);
+
+/* Block-accurate per-stream automation: stream `stream` takes p from absolute block `block` on (blocks counted since
+ * vp_engine_prepare / vp_engine_reset, the count of vp_call_plan.firstBlock), until its next change. 40 bytes. */
+typedef struct vp_stream_event {
+    int stream;
+    int reserved;     /* 0 */
+    long long block;
+    vp_stream_params p;
+    int pad;          /* 0 */
+} vp_stream_event;
+/* Queues changes for any block not yet issued; a process call of any kind (including vp_engine_stream_block) applies them
+ * at their blocks, where the reference reads each value: a value scheduled for block b applies to every read site whose
+ * delayed-timeline position lies in block b or later -- the start of a vocoder frame (gainVoc), the start of a pitch frame
+ * (keyPitch), the start of a pitch chunk (gainPitch: the whole chunk, also the part past the block's end), the output
+ * sample (gainVoice, gainSynth). The output does not depend on how the blocks are cut into calls: one call, any cut into
+ * several calls, or vp_engine_stream_block block by block give bit-identical output and frame records.
+ * Valid after vp_engine_prepare (VP_E_STATE before). count < 0, events == NULL with count > 0, a stream outside
+ * [0, nStreams) or a block already issued is VP_E_ARG; a value outside the plug-in's range is VP_E_RANGE; on any error
+ * nothing is queued. The same (stream, block) twice: the later one (list order, then call order) wins. An event at the next
+ * block to be issued is exactly vp_engine_set_stream_params before that call. Does not wait for the GPU; a call already
+ * issued keeps its values. vp_engine_set_stream_params / vp_engine_set_params change the value from the next block on and
+ * leave pending events in place (they apply at their blocks); vp_engine_reset and vp_engine_prepare drop every pending
+ * event, vp_engine_reset_streams those of the listed streams. A call with no event inside its blocks costs nothing extra; a
+ * call with events after its first block builds a per-block parameter table (one kernel launch; 32 bytes x nStreams x
+ * nBlocks of device memory, allocated at the first such call outside the workspace budget: VP_E_NOMEM before anything is
+ * issued when it cannot be had). */
+int vp_engine_schedule_stream_params(vp_engine* e, const vp_stream_event* events, int count);
 /* Behaviour at the places where the reference's C++ has undefined behaviour (SURVEY.md App. B U1-U6):
  *   VP_MODE_PARITY  (default) what the reference build actually does: the stale vector slot of PitchProcess.cpp:818 and the
  *                   popped table slot of Notes.cpp:99 are modelled, the other sites keep going and the frame is flagged VP_PF_UB;
@@ -196,7 +224,9 @@ int vp_engine_reset(vp_engine* e);
  * any index outside [0, nStreams) is VP_E_ARG, and then nothing is queued. Duplicates, and repeated requests before one
  * process call, act as one. The reset takes effect at the next process call of any kind (process_device, process_host,
  * process_host_pcm16, stream_block), before its first kernel; a call already issued keeps the state it was issued with.
- * Does not wait for the GPU. Keeps each stream's vp_stream_params, the engine-wide parameters, the grids, every other
+ * Does not wait for the GPU. Keeps each stream's vp_stream_params (the values in force now) but drops the listed streams'
+ * pending vp_engine_schedule_stream_params events: a slot handed to a new user does not inherit the old user's automation
+ * (the other streams keep theirs). Keeps the engine-wide parameters, the grids, every other
  * stream (bit for bit) and the records of the most recent call (get_pitch_frames / get_voc_frames); does not clear the
  * failed mark of a half-done call (only vp_engine_reset / vp_engine_prepare do, and both drop pending stream resets).
  * Streaming needs no new graph capture for it. Cost: one kernel launch in the next call, none when no reset is pending. */

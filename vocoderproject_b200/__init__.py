@@ -31,7 +31,7 @@ ABI_SYMBOLS = [
     "vp_synth_host", "vp_synth_device", "vp_measure_peaks", "vp_engine_timing_reset", "vp_engine_timer_record",
     "vp_engine_timer_elapsed_ms", "vp_engine_last_timing_counts", "vp_measure_peaks2", "vp_engine_reset", "vp_engine_stream_buffers", "vp_engine_stream_block",
     "vp_engine_stream_stats", "vp_engine_get_info", "vp_engine_reserve_orders", "vp_grid_plan", "vp_engine_set_mode", "vp_engine_process_host_pcm16", "vp_engine_set_window",
-    "vp_engine_set_stream_params", "vp_engine_get_stream_params", "vp_engine_reset_streams",
+    "vp_engine_set_stream_params", "vp_engine_get_stream_params", "vp_engine_reset_streams", "vp_engine_schedule_stream_params",
 ]
 
 
@@ -51,6 +51,11 @@ class StreamParams(C.Structure):
 
 
 STREAM_PARAM_FIELDS = tuple(k for k, _ in StreamParams._fields_)
+
+
+class StreamEvent(C.Structure):
+    """vp_stream_event: stream `stream` takes p from absolute block `block` on (blocks since prepare / reset). 40 bytes."""
+    _fields_ = [("stream", C.c_int), ("reserved", C.c_int), ("block", C.c_longlong), ("p", StreamParams), ("pad", C.c_int)]
 
 
 def stream_params(**kw):
@@ -143,6 +148,7 @@ def load_library(path=None):
         "vp_engine_timing_reset": (i, [vp, i]),
         "vp_engine_reset": (i, [vp]),
         "vp_engine_reset_streams": (i, [vp, C.POINTER(i), i]),
+        "vp_engine_schedule_stream_params": (i, [vp, C.POINTER(StreamEvent), i]),
         "vp_engine_stream_buffers": (i, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]),
         "vp_engine_stream_block": (i, [vp]),
         "vp_engine_stream_stats": (i, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
@@ -295,7 +301,8 @@ class Engine:
 
     def reset_streams(self, streams):
         """Hand the listed streams to new instances: from the next process call on, each continues as a stream that has
-        heard only silence since prepare (its key and gains are kept). The other streams are not touched."""
+        heard only silence since prepare (its key and gains are kept, its pending scheduled changes are dropped). The other
+        streams are not touched."""
         streams = [int(s) for s in streams]
         arr = (C.c_int * max(len(streams), 1))(*streams)
         self._check(self.lib.vp_engine_reset_streams(self.h, arr, len(streams)))
@@ -345,6 +352,41 @@ class Engine:
                     if f not in STREAM_PARAM_FIELDS:
                         raise KeyError(f)
         self._check(self.lib.vp_engine_set_stream_params(self.h, int(first), len(items), arr))
+
+    def schedule_stream_params(self, events):
+        """Block-accurate automation: events = [(stream, block, values), ...]; stream `stream` takes the values from absolute
+        block `block` on (blocks since prepare / reset; not one already processed), where the reference reads each of them --
+        also inside one multi-block process call. values is a StreamParams or a dict; the missing fields of a dict are the
+        stream's values just before that block as far as this call can tell: its current values, updated by the earlier
+        events of the same list for that stream at blocks up to that one (events queued by earlier calls are not seen).
+        On an error nothing is queued."""
+        events = list(events)
+        cur = None
+        if any(not isinstance(v, StreamParams) for _, _, v in events):
+            cur = self.stream_params()
+        # for dicts: the mirror of each stream's values, in block order (a stable sort keeps list order within a block)
+        order = sorted(range(len(events)), key=lambda k: (int(events[k][1]), k))
+        last = {}
+        arr = (StreamEvent * max(len(events), 1))()
+        for k in order:
+            s, b, v = events[k]
+            s, b = int(s), int(b)
+            e = arr[k]
+            e.stream, e.block, e.reserved, e.pad = s, b, 0, 0
+            if isinstance(v, StreamParams):
+                C.memmove(C.byref(e.p), C.byref(v), C.sizeof(StreamParams))
+                vals = v.as_dict()
+            else:
+                for f in v:
+                    if f not in STREAM_PARAM_FIELDS:
+                        raise KeyError(f)
+                base = last.get(s) or (cur[s] if 0 <= s < len(cur) else dict(stream_params().as_dict()))
+                vals = dict(base)
+                vals.update(v)
+                for f in STREAM_PARAM_FIELDS:
+                    setattr(e.p, f, vals[f])
+            last[s] = vals
+        self._check(self.lib.vp_engine_schedule_stream_params(self.h, arr, len(events)))
 
     def stream_params(self, first=0, count=None):
         """[dict] of the key and gains of streams first .. first + count - 1 (default: to the last stream)."""

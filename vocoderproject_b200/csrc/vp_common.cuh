@@ -170,8 +170,9 @@ inline cudaError_t vp_take_launch_error() {
 
 // The per-instance parameters of one stream (vp_stream_params) as the kernels read them: gains already converted with
 // decibelsToGain<float>(dB, -59) (PluginProcessor.cpp:226-230, VocoderProcess.cpp:291, PitchProcess.cpp:336), the key, and
-// whether each dry path is mixed in (> -59 dB). Device table [nStreams], indexed by the engine's global stream.
-struct VPStreamParam {
+// whether each dry path is mixed in (> -59 dB). Device table [nStreams], indexed by the engine's global stream; a call with
+// scheduled changes (vp_engine_schedule_stream_params) reads a block-indexed table [nBlocks][nStreams] instead.
+struct __align__(16) VPStreamParam {
     float gainVocF, gainPitchF, gainVoiceF, gainSynthF;
     int key;             // Notes::key 0..12: row of the note LUTs
     int dryOn, synthOn;  // dry voice / dry side-chain mixed in
@@ -188,8 +189,14 @@ struct VPTables {
     const double* lutBeta;   // [13 keys][tauMax+1] per period: closestFreq / pitch   PitchProcess.cpp:594-596
     const int* lutPeriodNew; // [13][tauMax+1] per period: round(period / beta)
     const int* lutNote;      // [13][tauMax+1] per period: snapped note index         Notes.cpp:79-110
-    const VPStreamParam* sp; // per-stream parameters of the pass's streams (table + streamBase): sp[s], s = stream of the pass
+    const VPStreamParam* sp; // per-stream parameters of the pass's streams (table + streamBase): sp[blk * spStride + s], s = stream
+                             // of the pass, blk = call-local block of the read site's delayed-timeline position (vp_sp)
+    int spStride;            // 0: one entry per stream for the whole call; nStreams: a call with scheduled changes
 };
+// the parameters of stream s (of the pass) in force at call-local block blk
+__device__ __forceinline__ const VPStreamParam& vp_sp(const VPTables& tb, int blk, int s) {
+    return tb.sp[(size_t)blk * (size_t)tb.spStride + s];
+}
 
 int vp_gate_carry_rows(const VPGeom& g);
 void vp_launch_gate(cudaStream_t st, const VPGeom& g, int S, const float* voice, const float* synth, uint8_t* gate,
@@ -227,9 +234,12 @@ void vp_launch_pitch_lpc(cudaStream_t st, const VPGeom& g, int S, const float* v
                          double* rP, double* aP);
 void vp_launch_pitch_psola(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const float* voice,
                            vp_pitch_frame* frames, const double* aP, float* outE);
-// gainUniform: the gainPitch (as a gain) every stream of the call has, or NULL to read each stream's from the table
+// gainUniform: the gainPitch (as a gain) every stream has in every block of the call and that every carried chunk was
+// emitted with, or NULL to read each chunk's from the table. pgIn / pgOut [S][VP_PC][4]: the gain each chunk of the carried
+// pitch frames was emitted with, before / after the call (pgOut: the last VP_PC frames of carried ++ new)
 void vp_launch_pitch_iir(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const vp_pitch_frame* frames,
-                         const double* aP, const float* outE, float* outP, const float* gainUniform);
+                         const double* aP, const float* outE, float* outP, const float* gainUniform, const float* pgIn,
+                         float* pgOut);
 // anyDry: some stream of the call has a dry path on (then the general kernel, which tests each stream's own flags)
 void vp_launch_mix(cudaStream_t st, const VPGeom& g, const VPTables& tb, bool anyDry, int S, const float* voice, const float* synthL,
                    const float* synthR, const float* outV, const float* outP, float* outL, float* outR);
@@ -260,6 +270,10 @@ struct VPResetSegs {
 };
 // one launch: the silent state of streams list[0 .. count) (list == NULL: streams 0 .. count - 1) in every segment
 void vp_launch_reset_streams(cudaStream_t st, const VPResetSegs& segs, const int* list, int count);
+// the [nBlocks][S] table of a call with scheduled changes: entry (b, s) = the last event of stream s at or before call-local
+// block b (events of s: evBlk / evVal[off[s] .. off[s + 1]), ascending blocks), else cur[s]
+void vp_launch_expand_stream_params(cudaStream_t st, const VPStreamParam* cur, const int* off, const int* evBlk,
+                                    const VPStreamParam* evVal, VPStreamParam* out, int S, int nBlocks);
 // 16-bit PCM <-> float exactly as vp_wav.hpp converts on the host: x / 32768 in, clamp(rint(x * 32768)) out
 void vp_launch_pcm16_to_float(cudaStream_t st, float* dst, const int16_t* src, long long count);
 void vp_launch_float_to_pcm16(cudaStream_t st, int16_t* dst, const float* src, long long count);

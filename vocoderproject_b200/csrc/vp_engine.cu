@@ -6,6 +6,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <limits.h>
+
 #include <algorithm>
 #include <map>
 #include <string>
@@ -91,6 +93,24 @@ struct vp_engine {
     bool anyDry = false, anySynth = false;  // some stream has a dry path (voice or side-chain) / the dry side-chain on
     bool pitchGainUniform = true;           // every stream has the same gainPitch (k_pitch_iir then takes it as an argument)
     bool capturing = false;                 // a streaming graph is being captured: nothing table-derived may be baked in
+    // ---- scheduled per-stream changes (vp_engine_schedule_stream_params): pending events by (absolute block, stream). A call
+    // takes those at its first block into the [S] table (= vp_engine_set_stream_params before it) and those after it into
+    // callEv; a call with callEv non-empty reads the block-indexed table dSPB [nBlocks][S], which k_expand_stream_params
+    // builds from dSP and the events (uploaded through the pinned staging buffer schPinned; evSchUp marks when that copy
+    // has read it). dSPB is allocated at the first such call, outside the workspace budget.
+    struct CallEvent { int blk, stream; vp_stream_params p; VPStreamParam v; };
+    std::map<std::pair<long long, int>, vp_stream_params> sched;
+    std::vector<CallEvent> callEv;
+    VPStreamParam* dSPB = nullptr;
+    uint8_t *schPinned = nullptr, *dSch = nullptr;
+    size_t schPinnedCap = 0, dSchCap = 0;
+    cudaEvent_t evSchUp = nullptr;
+    // what the call being issued reads (the [S] table or dSPB) and its flags over all of its blocks: some stream has a dry path
+    // on / the dry side-chain on in some block, every stream has gainPitch callPg in every block
+    const VPStreamParam* callSP = nullptr;
+    int callStride = 0;
+    bool callAnyDry = false, callAnySynth = false, callPgUniform = true;
+    float callPg = 0.0f;
     // workspace (device), sized for Sc streams x maxBlocks
     uint8_t* dGate = nullptr;
     double* dGatePart = nullptr;
@@ -102,6 +122,12 @@ struct vp_engine {
     double *cGate = nullptr, *cAV = nullptr, *cAS = nullptr, *cEeS = nullptr, *cG = nullptr, *cGainHist = nullptr;
     vp_pitch_frame* cFrames = nullptr; // [S][VP_PC]
     VPMarkState* cMarks = nullptr;     // [S]
+    // gain each chunk of the carried pitch frames was emitted with, [S][VP_PC][4], read / written by k_pitch_iir: current =
+    // cPG[histCur], the call writes the other one. pgCarry >= 0: every carried chunk of every stream went out with that gain
+    // (then k_pitch_iir may take a uniform gain as its argument); pgCarryAny: nothing has been emitted since prepare / reset.
+    float* cPG[2] = {nullptr, nullptr};
+    float pgCarry = -1.0f;
+    bool pgCarryAny = true;
     // ---- per-stream resets (vp_engine_reset_streams): the streams listed since the last process call (rsMark dedupes), put on
     // the device through the pinned staging list rsPinned, like the parameter table; evRsUp marks when that copy has read it
     std::vector<uint8_t> rsMark;
@@ -320,6 +346,13 @@ static void free_workspace(vp_engine* e) {
                       (void**)&e->cFrames, (void**)&e->cMarks, (void**)&e->oAV, (void**)&e->oAS, (void**)&e->oEeS, (void**)&e->oG};
     for (void** p : cptrs) if (*p) { cudaFree(*p); *p = nullptr; }
     for (int i = 0; i < 2; ++i) for (int j = 0; j < 3; ++j) if (e->cHist[i][j]) { cudaFree(e->cHist[i][j]); e->cHist[i][j] = nullptr; }
+    for (int i = 0; i < 2; ++i) if (e->cPG[i]) { cudaFree(e->cPG[i]); e->cPG[i] = nullptr; }
+    if (e->dSPB) { cudaFree(e->dSPB); e->dSPB = nullptr; }
+    if (e->dSch) { cudaFree(e->dSch); e->dSch = nullptr; }
+    if (e->schPinned) { cudaFreeHost(e->schPinned); e->schPinned = nullptr; }
+    e->dSchCap = e->schPinnedCap = 0;
+    e->sched.clear();
+    e->callEv.clear();
     if (e->spPinned) { cudaFreeHost(e->spPinned); e->spPinned = nullptr; }
     if (e->rsPinned) { cudaFreeHost(e->rsPinned); e->rsPinned = nullptr; }
     void** ptrs[] = {(void**)&e->dSP, (void**)&e->dRsList, (void**)&e->dGate, (void**)&e->dRV, (void**)&e->dRS, (void**)&e->dAV, (void**)&e->dAS, (void**)&e->dEeV,
@@ -362,7 +395,8 @@ extern "C" int vp_engine_create(vp_engine** out, int device) {
         cudaEventCreateWithFlags(&e->evJoin, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreate(&e->evT0) != cudaSuccess || cudaEventCreate(&e->evT1) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->evSpUp, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&e->evRsUp, cudaEventDisableTiming) != cudaSuccess) {
+        cudaEventCreateWithFlags(&e->evRsUp, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&e->evSchUp, cudaEventDisableTiming) != cudaSuccess) {
         cudaGetLastError();
         delete e;
         return VP_E_CUDA;
@@ -400,7 +434,7 @@ extern "C" void vp_engine_destroy(vp_engine* e) {
     cudaEventDestroy(e->evT0); cudaEventDestroy(e->evT1);
     for (int i = 0; i < 8; ++i) cudaEventDestroy(e->evTimer[i]);
     for (auto ev : e->evSide) cudaEventDestroy(ev);
-    cudaEventDestroy(e->evFork); cudaEventDestroy(e->evJoin); cudaEventDestroy(e->evSpUp); cudaEventDestroy(e->evRsUp);
+    cudaEventDestroy(e->evFork); cudaEventDestroy(e->evJoin); cudaEventDestroy(e->evSpUp); cudaEventDestroy(e->evRsUp); cudaEventDestroy(e->evSchUp);
     for (int i = 0; i < 2; ++i) { cudaEventDestroy(e->evYin[i]); cudaEventDestroy(e->evMarks[i]); cudaEventDestroy(e->evSideDone[i]); cudaEventDestroy(e->evMix[i]); }
     cudaStreamDestroy(e->st); cudaStreamDestroy(e->stIn); cudaStreamDestroy(e->stOut); cudaStreamDestroy(e->st2);
     delete e;
@@ -468,16 +502,17 @@ static VPStreamParam stream_table_entry(const vp_stream_params& p) {
     return q;
 }
 
-// streams [first, first + count) take the values p[0 .. count); only a changed table entry makes the next call upload
-static void put_stream_params(vp_engine* e, int first, int count, const vp_stream_params* p, size_t pStep) {
-    bool changed = false;
-    for (int i = 0; i < count; ++i) {
-        const vp_stream_params& v = p[(size_t)i * pStep];
-        const VPStreamParam t = stream_table_entry(v);
-        e->sprm[first + i] = v;
-        if (memcmp(&e->spTab[first + i], &t, sizeof t) != 0) { e->spTab[first + i] = t; changed = true; }
-    }
-    if (!changed) return;
+// stream s takes the values v; true when its table entry changed
+static bool put_one_stream(vp_engine* e, int s, const vp_stream_params& v) {
+    const VPStreamParam t = stream_table_entry(v);
+    e->sprm[s] = v;
+    if (memcmp(&e->spTab[s], &t, sizeof t) == 0) return false;
+    e->spTab[s] = t;
+    return true;
+}
+
+// after table entries changed: the next call uploads the table, the batch-wide flags are recomputed
+static void stream_table_changed(vp_engine* e) {
     e->spDirty = true;
     e->anyDry = e->anySynth = false;
     e->pitchGainUniform = true;
@@ -486,6 +521,13 @@ static void put_stream_params(vp_engine* e, int first, int count, const vp_strea
         e->anySynth = e->anySynth || t.synthOn;
         e->pitchGainUniform = e->pitchGainUniform && t.gainPitchF == e->spTab[0].gainPitchF;
     }
+}
+
+// streams [first, first + count) take the values p[0 .. count); only a changed table entry makes the next call upload
+static void put_stream_params(vp_engine* e, int first, int count, const vp_stream_params* p, size_t pStep) {
+    bool changed = false;
+    for (int i = 0; i < count; ++i) changed = put_one_stream(e, first + i, p[(size_t)i * pStep]) || changed;
+    if (changed) stream_table_changed(e);
 }
 
 static vp_stream_params stream_part(const vp_params& p) {
@@ -508,15 +550,32 @@ static int upload_stream_params(vp_engine* e) {
     return VP_OK;
 }
 
+static bool stream_params_ok(const vp_stream_params& p) {
+    return p.keyPitch >= 0 && p.keyPitch <= 12 && gain_ok(p.gainPitch) && gain_ok(p.gainVoice) && gain_ok(p.gainSynth) &&
+           gain_ok(p.gainVoc);
+}
+
 extern "C" int vp_engine_set_stream_params(vp_engine* e, int firstStream, int count, const vp_stream_params* p) {
     if (!e || !p) return VP_E_ARG;
     if (!e->prepared) return vp_err(e, VP_E_STATE, "vp_engine_prepare has not been called");
     if (firstStream < 0 || count < 0 || firstStream > e->S - count) return vp_err(e, VP_E_ARG, "stream range outside [0, nStreams)");
     for (int i = 0; i < count; ++i)
-        if (p[i].keyPitch < 0 || p[i].keyPitch > 12 || !gain_ok(p[i].gainPitch) || !gain_ok(p[i].gainVoice) ||
-            !gain_ok(p[i].gainSynth) || !gain_ok(p[i].gainVoc))
-            return vp_err(e, VP_E_RANGE, "parameter outside the plug-in's range");
+        if (!stream_params_ok(p[i])) return vp_err(e, VP_E_RANGE, "parameter outside the plug-in's range");
     put_stream_params(e, firstStream, count, p, 1);
+    return VP_OK;
+}
+
+extern "C" int vp_engine_schedule_stream_params(vp_engine* e, const vp_stream_event* ev, int count) {
+    if (!e) return VP_E_ARG;
+    if (!e->prepared) return vp_err(e, VP_E_STATE, "vp_engine_prepare has not been called");
+    if (count < 0 || (count > 0 && !ev)) return vp_err(e, VP_E_ARG, "events must be non-null and count >= 0");
+    for (int i = 0; i < count; ++i) {
+        if (ev[i].stream < 0 || ev[i].stream >= e->S) return vp_err(e, VP_E_ARG, "stream index outside [0, nStreams)");
+        if (ev[i].block < e->gs.blocksDone) return vp_err(e, VP_E_ARG, "event for a block that has already been issued");
+    }
+    for (int i = 0; i < count; ++i)
+        if (!stream_params_ok(ev[i].p)) return vp_err(e, VP_E_RANGE, "parameter outside the plug-in's range");
+    for (int i = 0; i < count; ++i) e->sched[{ev[i].block, ev[i].stream}] = ev[i].p;  // a later (stream, block) replaces an earlier one
     return VP_OK;
 }
 
@@ -599,6 +658,7 @@ static VPResetSegs carried_state(vp_engine* e) {
     add(e->cGainHist, 20 * d, VP_FILL_ZERO, 0);
     add(e->cFrames, (size_t)VP_PC * sizeof(vp_pitch_frame), VP_FILL_ZERO, 0);
     add(e->cMarks, sizeof(VPMarkState), VP_FILL_ONE_AT, (int)(offsetof(VPMarkState, beta) / d));
+    add(e->cPG[e->histCur], (size_t)VP_PC * 4 * sizeof(float), VP_FILL_ZERO, 0);  // (a silent frame has no marks: never emitted)
     add(e->oAV, (size_t)VP_ORPH * (e->capV + 1) * d, VP_FILL_ZERO, 0);
     add(e->oAS, (size_t)VP_ORPH * (e->capS + 1) * d, VP_FILL_ZERO, 0);
     add(e->oEeS, (size_t)VP_ORPH * d, VP_FILL_GATED, 0);
@@ -616,6 +676,8 @@ static int reset_state(vp_engine* e) {
     VP_CUDA_OK(cudaStreamSynchronize(e->st));
     for (int s : e->rsList) e->rsMark[s] = 0;
     e->rsList.clear();
+    e->sched.clear();
+    e->pgCarryAny = true;
     e->gs.B = e->B; e->gs.z = e->sz;
     e->gs.reset();
     e->failed = false;
@@ -639,6 +701,15 @@ extern "C" int vp_engine_reset_streams(vp_engine* e, const int* streams, int cou
         if (streams[i] < 0 || streams[i] >= e->S) return vp_err(e, VP_E_ARG, "stream index outside [0, nStreams)");
     for (int i = 0; i < count; ++i)
         if (!e->rsMark[streams[i]]) { e->rsMark[streams[i]] = 1; e->rsList.push_back(streams[i]); }
+    // the new user of a slot does not inherit the old user's automation
+    if (!e->sched.empty() && count > 0) {
+        std::vector<uint8_t> listed((size_t)e->S, 0);
+        for (int i = 0; i < count; ++i) listed[streams[i]] = 1;
+        for (auto it = e->sched.begin(); it != e->sched.end();) {
+            if (listed[it->first.second]) it = e->sched.erase(it);
+            else ++it;
+        }
+    }
     return VP_OK;
 }
 
@@ -656,6 +727,98 @@ static int apply_stream_resets(vp_engine* e) {
     e->launches++;
     for (int s : e->rsList) e->rsMark[s] = 0;
     e->rsList.clear();
+    return VP_OK;
+}
+
+// Host part of a call's scheduled changes (nothing is issued; what the call needs is allocated here, so that VP_E_NOMEM comes
+// before its first kernel). Events at the call's first block b0 go into the [S] table now: exactly vp_engine_set_stream_params
+// before the call. Events after b0 inside the call are listed in callEv (ascending block, then stream); they make the call
+// read the block-indexed table. The call's flags (dry paths, uniform pitch gain) cover all of its blocks.
+static int plan_schedule(vp_engine* e, int nBlocks) {
+    const long long b0 = e->gs.blocksDone;
+    bool changed = false;
+    for (auto it = e->sched.begin(); it != e->sched.end() && it->first.first == b0;) {  // (no earlier block can be pending)
+        changed = put_one_stream(e, it->first.second, it->second) || changed;
+        it = e->sched.erase(it);
+    }
+    if (changed) stream_table_changed(e);
+    e->callEv.clear();
+    const auto end = e->sched.lower_bound({b0 + nBlocks, INT_MIN});
+    for (auto it = e->sched.begin(); it != end; ++it)
+        e->callEv.push_back({(int)(it->first.first - b0), it->first.second, it->second, stream_table_entry(it->second)});
+    e->callAnyDry = e->anyDry; e->callAnySynth = e->anySynth;
+    e->callPg = e->spTab[0].gainPitchF; e->callPgUniform = e->pitchGainUniform;
+    for (const auto& c : e->callEv) {
+        e->callAnyDry = e->callAnyDry || c.v.dryOn || c.v.synthOn;
+        e->callAnySynth = e->callAnySynth || c.v.synthOn;
+        e->callPgUniform = e->callPgUniform && c.v.gainPitchF == e->callPg;
+    }
+    e->callSP = e->dSP; e->callStride = 0;
+    if (e->callEv.empty()) return VP_OK;
+    if (!e->dSPB) {
+        if (cudaMalloc((void**)&e->dSPB, (size_t)e->S * e->maxBlocks * sizeof(VPStreamParam)) != cudaSuccess) {
+            cudaGetLastError();
+            e->dSPB = nullptr;
+            return vp_err(e, VP_E_NOMEM, "no device memory for the per-block parameter table of a scheduled call");
+        }
+    }
+    const size_t nEv = e->callEv.size();
+    const size_t bytes = (((size_t)(e->S + 1) * 4 + 15) & ~(size_t)15) + ((nEv * 4 + 15) & ~(size_t)15) + nEv * sizeof(VPStreamParam);
+    if (bytes > e->schPinnedCap) {
+        VP_CUDA_OK(cudaEventSynchronize(e->evSchUp));  // the previous upload has read the old buffer
+        if (e->schPinned) cudaFreeHost(e->schPinned);
+        e->schPinned = nullptr; e->schPinnedCap = 0;
+        if (cudaHostAlloc((void**)&e->schPinned, bytes, cudaHostAllocDefault) != cudaSuccess) {
+            cudaGetLastError();
+            e->schPinned = nullptr;
+            return vp_err(e, VP_E_NOMEM, "no pinned host memory for the scheduled events");
+        }
+        e->schPinnedCap = bytes;
+    }
+    if (bytes > e->dSchCap) {
+        if (e->dSch) cudaFree(e->dSch);  // (cudaFree waits for the device: only when the list outgrows the buffer)
+        e->dSch = nullptr; e->dSchCap = 0;
+        if (cudaMalloc((void**)&e->dSch, bytes) != cudaSuccess) {
+            cudaGetLastError();
+            e->dSch = nullptr;
+            return vp_err(e, VP_E_NOMEM, "no device memory for the scheduled events");
+        }
+        e->dSchCap = bytes;
+    }
+    e->callSP = e->dSPB; e->callStride = e->S;
+    return VP_OK;
+}
+
+// Device part, after the [S] table of the call's start is on its way: the events go up through the pinned staging buffer
+// (rewritten only after the previous upload has read it) as per-stream lists, and one kernel builds the [nBlocks][S] table.
+// The host then holds the values in force at the call's last block; they reach dSP with the next call's upload.
+static int issue_schedule(vp_engine* e, int nBlocks) {
+    if (e->callEv.empty()) return VP_OK;
+    const int S = e->S;
+    const size_t nEv = e->callEv.size();
+    const size_t offB = ((size_t)(S + 1) * 4 + 15) & ~(size_t)15, blkB = (nEv * 4 + 15) & ~(size_t)15;
+    const size_t bytes = offB + blkB + nEv * sizeof(VPStreamParam);
+    VP_CUDA_OK(cudaEventSynchronize(e->evSchUp));
+    int* off = reinterpret_cast<int*>(e->schPinned);
+    int* blk = reinterpret_cast<int*>(e->schPinned + offB);
+    VPStreamParam* val = reinterpret_cast<VPStreamParam*>(e->schPinned + offB + blkB);
+    for (int i = 0; i <= S; ++i) off[i] = 0;
+    for (const auto& c : e->callEv) off[c.stream + 1]++;
+    for (int i = 0; i < S; ++i) off[i + 1] += off[i];
+    {   // stable counting sort by stream: each stream's events keep their ascending blocks
+        std::vector<int> pos(off, off + S);
+        for (const auto& c : e->callEv) { const int k = pos[c.stream]++; blk[k] = c.blk; val[k] = c.v; }
+    }
+    VP_CUDA_OK(cudaMemcpyAsync(e->dSch, e->schPinned, bytes, cudaMemcpyHostToDevice, e->st));
+    VP_CUDA_OK(cudaEventRecord(e->evSchUp, e->st));
+    vp_launch_expand_stream_params(e->st, e->dSP, reinterpret_cast<const int*>(e->dSch), reinterpret_cast<const int*>(e->dSch + offB),
+                                   reinterpret_cast<const VPStreamParam*>(e->dSch + offB + blkB), e->dSPB, S, nBlocks);
+    e->launches++;
+    bool changed = false;
+    for (const auto& c : e->callEv) changed = put_one_stream(e, c.stream, c.p) || changed;  // ascending blocks: the last one stays
+    if (changed) stream_table_changed(e);
+    const long long b0 = e->gs.blocksDone;
+    e->sched.erase(e->sched.begin(), e->sched.lower_bound({b0 + nBlocks, INT_MIN}));
     return VP_OK;
 }
 
@@ -763,6 +926,10 @@ extern "C" int vp_engine_prepare(vp_engine* e, double fs, int B, int S, int maxB
     if ((rc = wsalloc(e, &e->cGainHist, (size_t)S * 20))) return rc;
     if ((rc = wsalloc(e, &e->cFrames, (size_t)S * VP_PC))) return rc;
     if ((rc = wsalloc(e, &e->cMarks, (size_t)S))) return rc;
+    for (int i = 0; i < 2; ++i) {
+        if ((rc = wsalloc(e, &e->cPG[i], (size_t)S * VP_PC * 4))) return rc;
+        VP_CUDA_OK(cudaMemset(e->cPG[i], 0, (size_t)S * VP_PC * 4 * sizeof(float)));
+    }
     // every stream starts from the engine's parameters
     if ((rc = wsalloc(e, &e->dSP, (size_t)S))) return rc;
     VP_CUDA_OK(cudaHostAlloc((void**)&e->spPinned, (size_t)S * sizeof(VPStreamParam), cudaHostAllocDefault));
@@ -865,7 +1032,7 @@ static void pass_init(vp_engine* e, PassCtx& c, const VPGeom& gIO, int Sp, int s
                       const float* synthR, float* outL, float* outR) {
     c.g = gIO;
     c.tb = VPTables{e->dWV, e->dWS ? e->dWS : e->dWV, e->dStP, e->dHann, e->dHannOff, e->dLutBeta, e->dLutPeriodNew, e->dLutNote,
-                    e->dSP + streamBase};
+                    e->callSP + streamBase, e->callStride};
     c.Sp = Sp;
     c.sb = (size_t)streamBase;
     const int hc = e->histCur;
@@ -1000,9 +1167,12 @@ static int pass_P(vp_engine* e, PassCtx& c) {
         stage_mark(e, ST_PLPC);
         vp_launch_pitch_psola(st, g, c.tb, Sp, c.voice, e->dFrames, e->dAP, e->dOutE);
         stage_mark(e, ST_PFRAME);
+        // one gain for every chunk of the call: every stream has it in every block, and the carried chunks went out with it
         // (a captured graph reads the table: a gain change between blocks must not need a new capture)
-        const bool uniform = e->pitchGainUniform && !e->capturing;
-        vp_launch_pitch_iir(st, g, c.tb, Sp, e->dFrames, e->dAP, e->dOutE, e->dOutP, uniform ? &e->spTab[0].gainPitchF : nullptr);
+        const bool uniform = e->callPgUniform && (e->pgCarryAny || e->pgCarry == e->callPg) && !e->capturing;
+        const int hc = e->histCur;
+        vp_launch_pitch_iir(st, g, c.tb, Sp, e->dFrames, e->dAP, e->dOutE, e->dOutP, uniform ? &e->callPg : nullptr,
+                            e->cPG[hc] + c.sb * VP_PC * 4, e->cPG[hc ^ 1] + c.sb * VP_PC * 4);
         stage_mark(e, ST_PIIR);
         e->launches += 4;
         e->yinFrames += (size_t)Sp * g.nFramesP;
@@ -1085,7 +1255,7 @@ static int pass_M(vp_engine* e, PassCtx& c) {
     const size_t sb = c.sb;
     const int hc = e->histCur;
     const long long rowsP = g.nFramesP + VP_PC;
-    vp_launch_mix(st, g, c.tb, e->anyDry, Sp, c.voice, c.synthL, c.synthR, e->dOutV, e->dOutP, c.outL, c.outR);
+    vp_launch_mix(st, g, c.tb, e->callAnyDry, Sp, c.voice, c.synthL, c.synthR, e->dOutV, e->dOutP, c.outL, c.outR);
     e->launches++;
     stage_mark(e, ST_MIX);
     if (g.pitchMix) vp_launch_carry_out(st, e->cFrames + sb * VP_PC, e->dFrames, Sp, (int)sizeof(vp_pitch_frame), (int)sizeof(vp_pitch_frame), VP_PC, g.nFramesP, rowsP);
@@ -1302,6 +1472,11 @@ static void begin_call(vp_engine* e) {
 static void finish_call(vp_engine* e, const VPGeom& g) {
     grid_finish(e->gs, g);
     e->histCur ^= 1;
+    // the frames carried out: all their emitted chunks went out with callPg if the call had it throughout and they start in
+    // the call (or the chunks before it had it as well)
+    const bool same = e->callPgUniform && (e->pgCarryAny || e->pgCarry == e->callPg || g.nFramesP >= VP_PC);
+    e->pgCarry = same ? e->callPg : -1.0f;
+    e->pgCarryAny = false;
 }
 
 static int check_process_args(vp_engine* e, int nBlocks, const float* voice, const float* synthL, const float* synthR,
@@ -1336,7 +1511,9 @@ extern "C" int vp_engine_process_device(vp_engine* e, int nBlocks, const float* 
         if (ranges_overlap(outL, span, outR, span)) return vp_err(e, VP_E_ARG, "outL and outR must not overlap");
     }
     VP_CUDA_OK(cudaSetDevice(e->device));
+    if ((rc = plan_schedule(e, nBlocks))) return rc;
     if ((rc = upload_stream_params(e))) return rc;
+    if ((rc = issue_schedule(e, nBlocks))) return rc;
     if ((rc = apply_stream_resets(e))) return rc;
     begin_call(e);
     VPGeom g;
@@ -1393,8 +1570,9 @@ static int process_host_impl(vp_engine* e, int nBlocks, const void* voiceV, cons
     int rc = check_process_args(e, nBlocks, (const float*)voiceV, (const float*)synthLV, (const float*)synthRV, (float*)outLV, stride);
     if (rc) return rc;
     VP_CUDA_OK(cudaSetDevice(e->device));
+    if ((rc = plan_schedule(e, nBlocks))) return rc;
     const long long n = (long long)nBlocks * e->B;
-    const bool synthOn = e->anySynth;
+    const bool synthOn = e->callAnySynth;  // (some block of some stream has the dry side-chain on)
     const size_t esz = pcm16 ? sizeof(int16_t) : sizeof(float);
     const char *voice = (const char*)voiceV, *synthL = (const char*)synthLV, *synthR = (const char*)synthRV;
     char *outL = (char*)outLV, *outR = (char*)outRV;
@@ -1428,6 +1606,7 @@ static int process_host_impl(vp_engine* e, int nBlocks, const void* voiceV, cons
         }
     }
     if ((rc = upload_stream_params(e))) return rc;
+    if ((rc = issue_schedule(e, nBlocks))) return rc;
     if ((rc = apply_stream_resets(e))) return rc;
     begin_call(e);
     e->sidePending = e->mixPending = false;
@@ -1538,8 +1717,10 @@ extern "C" int vp_engine_stream_buffers(vp_engine* e, float** voice, float** syn
 extern "C" int vp_engine_stream_block(vp_engine* e) {
     if (!e) return VP_E_ARG;
     if (!e->prepared || !e->sHostV) return vp_err(e, VP_E_STATE, "call vp_engine_prepare and vp_engine_stream_buffers first");
-    if (e->anySynth) return vp_err(e, VP_E_ARG, "streaming mode carries side-chain channel 0 only: gainSynth must be off on every stream");
     VP_CUDA_OK(cudaSetDevice(e->device));
+    // the block's scheduled changes go into the [S] table here (a one-block call has no event after its first block)
+    { int rc = plan_schedule(e, 1); if (rc) return rc; }
+    if (e->anySynth) return vp_err(e, VP_E_ARG, "streaming mode carries side-chain channel 0 only: gainSynth must be off on every stream");
     // per-stream key and gains are table data: a change is uploaded here, outside the graph, and needs no new capture
     // so are per-stream resets: one kernel before the graph, the block phase (the graph's key) does not change
     { int rc = upload_stream_params(e); if (!rc) rc = apply_stream_resets(e); if (rc) return rc; }
@@ -1551,7 +1732,7 @@ extern "C" int vp_engine_stream_block(vp_engine* e) {
     e->lastG = g;
     // everything that shapes the launch sequence or is baked into kernel arguments
     std::vector<long long> key = {e->gs.blocksDone > 0 ? 1 : 0, e->histCur, g.offV, g.offP, g.nFramesV, g.nFramesP, g.kV0, g.synV, g.synS,
-                                  g.vocOn, g.pitchOn, g.vocMix, g.pitchMix, e->anyDry};
+                                  g.vocOn, g.pitchOn, g.vocMix, g.pitchMix, e->callAnyDry};
     for (int j = 0; j < VP_ORPH; ++j) { key.push_back(g.orphPos[j]); key.push_back(g.orphOrdV[j]); key.push_back(g.orphOrdS[j]); }
     for (int j = 0; j < VP_PC; ++j) { key.push_back(g.carryPosP[j]); key.push_back(g.carryLimP[j]); }
     auto it = e->graphs.find(key);

@@ -135,6 +135,13 @@ public:
     // prepareToPlay for some instances of the running batch (a slot handed to a new user): from the next block on, each
     // listed stream continues as one that has heard only silence since prepare; the others are not touched
     void restartStreams(const int* streams, int count) { engine.check(vp_engine_reset_streams(engine.h, streams, count)); }
+    // automation at block accuracy: each event gives one stream its key and gains from an absolute block on (blocks counted
+    // since prepare / restart); the engine applies them where the reference reads each value, also inside one multi-block call.
+    // Pending events survive setParams / setStreamParams (which change the value from the next block on); restart drops them,
+    // restartStreams those of the listed streams
+    void scheduleStreamParams(const vp_stream_event* events, int count) {
+        engine.check(vp_engine_schedule_stream_params(engine.h, events, count));
+    }
     const vp_params& getParams() const { return params; }
 
     // fillInputBuffers(voiceBuffer, synthBuffer): host rows [S][stride]; synth channel 1 may be null when gainSynth is off

@@ -9,13 +9,15 @@
 // out = vocoder OLA + pitch OLA (+ gainVoice * delayed voice) (+ gainSynth *
 // delayed synth), cast to float. Output sample u carries input time u - latency.
 // ---------------------------------------------------------------------------
-// Each stream mixes with its own dry gains; a path that is off adds nothing (not 0 * x, which would turn -0 into +0).
-__global__ void __launch_bounds__(256) k_mix(VPGeom g, const VPStreamParam* __restrict__ sp, const float* __restrict__ voice,
+// Each stream mixes with its own dry gains, those of the output sample's block (PluginProcessor.cpp:226-230 reads them per
+// block); a path that is off adds nothing (not 0 * x, which would turn -0 into +0).
+__global__ void __launch_bounds__(256) k_mix(VPGeom g, VPTables tb, const float* __restrict__ voice,
                                              const float* __restrict__ synthL, const float* __restrict__ synthR,
                                              const float* __restrict__ outV, const float* __restrict__ outP,
                                              float* __restrict__ outL, float* __restrict__ outR) {
     const int s = blockIdx.y;
-    const VPStreamParam p = sp[s];
+    const VPStreamParam p0 = tb.sp[s];
+    const bool perBlock = tb.spStride != 0;
     const size_t row = (size_t)s * g.stride, wrow = (size_t)s * g.wstride;
     const long long step = (long long)gridDim.x * blockDim.x;
     constexpr int MU = 4;  // independent loads in flight per thread and plane
@@ -35,6 +37,7 @@ __global__ void __launch_bounds__(256) k_mix(VPGeom g, const VPStreamParam* __re
             if (g.vocMix) l += a[k];
             if (g.pitchMix) l += b[k];
             float r = l;
+            const VPStreamParam p = perBlock ? vp_sp(tb, (int)(u / g.B), s) : p0;
             if (p.dryOn) {
                 const float d = p.gainVoiceF * vp_x(vp_row(voice, g.histV, s, g), u, g);
                 l += d; r += d;
@@ -102,7 +105,40 @@ void vp_launch_mix(cudaStream_t st, const VPGeom& g, const VPTables& tb, bool an
     if (bx > 4096) bx = 4096;
     if (bx < 1) bx = 1;
     dim3 grid((unsigned)bx, S);
-    VP_LAUNCH(k_mix<<<grid, 256, 0, st>>>(g, tb.sp, voice, synthL, synthR, outV, outP, outL, outR));
+    VP_LAUNCH(k_mix<<<grid, 256, 0, st>>>(g, tb, voice, synthL, synthR, outV, outP, outL, outR));
+}
+
+// ---------------------------------------------------------------------------
+// Block-indexed parameter table of a call with scheduled changes (vp_engine_schedule_stream_params): out[b][s] = the value
+// stream s has in force at call-local block b -- its last event at or before b, else its value at the call's start cur[s].
+// Grid: x over streams (a warp writes 32 consecutive 32-byte entries of one block row), y over tiles of EX_TILE blocks; a
+// thread finds the value at its tile's start by binary search in its stream's events and walks the tile.
+// ---------------------------------------------------------------------------
+#define EX_TILE 64
+__global__ void __launch_bounds__(128) k_expand_stream_params(const VPStreamParam* __restrict__ cur, const int* __restrict__ off,
+                                                              const int* __restrict__ evBlk, const VPStreamParam* __restrict__ evVal,
+                                                              VPStreamParam* __restrict__ out, int S, int nBlocks) {
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= S) return;
+    const int b0 = blockIdx.y * EX_TILE, b1 = min(b0 + EX_TILE, nBlocks);
+    const int k0 = off[s], k1 = off[s + 1];
+    int lo = k0, hi = k1;  // first event after b0
+    while (lo < hi) {
+        const int m = (lo + hi) >> 1;
+        if (evBlk[m] <= b0) lo = m + 1;
+        else hi = m;
+    }
+    VPStreamParam v = (lo > k0) ? evVal[lo - 1] : cur[s];
+    int k = lo;
+    for (int b = b0; b < b1; ++b) {
+        if (k < k1 && evBlk[k] == b) v = evVal[k++];
+        out[(size_t)b * S + s] = v;
+    }
+}
+void vp_launch_expand_stream_params(cudaStream_t st, const VPStreamParam* cur, const int* off, const int* evBlk,
+                                    const VPStreamParam* evVal, VPStreamParam* out, int S, int nBlocks) {
+    const dim3 grid((unsigned)((S + 127) / 128), (unsigned)((nBlocks + EX_TILE - 1) / EX_TILE));
+    VP_LAUNCH(k_expand_stream_params<<<grid, 128, 0, st>>>(cur, off, evBlk, evVal, out, S, nBlocks));
 }
 
 // ---------------------------------------------------------------------------

@@ -700,7 +700,7 @@ __device__ __forceinline__ int vs_skew(int pos, int hop, int sk) { return pos + 
 // PROCESSED frames, newest first (a gated frame -- EeSynth < 0 -- neither shifts the histories nor gets a gain).
 // One thread per frame scans back over this call's frames and, if the call started fewer than 10 processed frames
 // ago, continues into the stream's carried histories hist[s] = {EeVoice[10], EeSynth[10]} (newest first).
-__global__ void __launch_bounds__(128) k_voc_gain(VPGeom g, const VPStreamParam* __restrict__ sp, const double* __restrict__ EeV,
+__global__ void __launch_bounds__(128) k_voc_gain(VPGeom g, VPTables tb, const double* __restrict__ EeV,
                                                   const double* __restrict__ EeS, double* __restrict__ G, double* __restrict__ Gs,
                                                   const double* __restrict__ hist, long long tot) {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -721,9 +721,10 @@ __global__ void __launch_bounds__(128) k_voc_gain(VPGeom g, const VPStreamParam*
         gain = sqrt(sv / ss);
     }
     G[row0 + k] = gain;
-    // what the synthesis applies: g times the frame's own gainVoc (its stream's, read once per frame, VocoderProcess.cpp:
-    // 291-294), so a frame that is finished by a later call keeps the gain of the block it was started in
-    Gs[row0 + k] = gain * (double)sp[s].gainVocF;
+    // what the synthesis applies: g times the frame's own gainVoc (its stream's, read once per frame in the block the frame
+    // starts in, VocoderProcess.cpp:291-294), so a frame that is finished by a later call keeps the gain of that block
+    const int blk = (int)(((long long)k * g.hopV + g.offV) / g.B);
+    Gs[row0 + k] = gain * (double)vp_sp(tb, blk, s).gainVocF;
 }
 
 // the carried histories after this call: the 10 newest processed frames of (old history ++ this call's frames)
@@ -746,7 +747,7 @@ __global__ void __launch_bounds__(64) k_voc_gain_carry(VPGeom g, const double* _
 void vp_launch_voc_gain(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const double* EeV, const double* EeS, double* G,
                         double* Gs, double* hist) {
     const long long tot = (long long)S * g.nFramesV;
-    if (tot > 0) VP_LAUNCH(k_voc_gain<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(g, tb.sp, EeV, EeS, G, Gs, hist, tot));
+    if (tot > 0) VP_LAUNCH(k_voc_gain<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(g, tb, EeV, EeS, G, Gs, hist, tot));
     VP_LAUNCH(k_voc_gain_carry<<<(S + 63) / 64, 64, 0, st>>>(g, EeV, EeS, hist, S));
 }
 
