@@ -10,8 +10,9 @@
  *
  * Semantics. One "stream" is one plug-in instance (1 mono voice + stereo
  * side-chain in, stereo out). Each stream has its own key and gains
- * (vp_stream_params, vp_engine_set_stream_params); the remaining parameters
- * (LPC orders, vocBool / pitchBool, window, mode) are one set per engine.
+ * (vp_stream_params, vp_engine_set_stream_params) and its own vocoder LPC
+ * orders (vp_stream_orders, vp_engine_set_stream_orders); the remaining
+ * parameters (lpcPitch, vocBool / pitchBool, window, mode) are one set per engine.
  * vp_engine_prepare is prepareToPlay(sampleRate,
  * samplesPerBlock) for every stream; each vp_engine_process* call is, per
  * stream, nBlocks further consecutive processBlock calls. Results do
@@ -57,13 +58,20 @@ typedef struct vp_params {
 } vp_params;
 
 /* The per-instance part of vp_params: what one stream's plug-in instance holds in its parameter tree and the engine reads
- * per stream. Only these five are per stream: the others (lpcVoice, lpcSynth, lpcPitch, vocBool, pitchBool, the window and
- * the mode) stay per engine, because the frame grids are host state every stream shares (a bypassed block freezes them) and
- * the orders select the tuned kernels and size the coefficient rows. 20 bytes. */
+ * per stream. These five and the two vocoder orders (vp_stream_orders) are per stream. The others stay per engine: vocBool
+ * and pitchBool move the frame grids, which are host state every stream shares (a bypassed block freezes them); lpcPitch is
+ * read in prepare only and sizes the pitch kernels; the window and the mode are prepare-time choices. 20 bytes. */
 typedef struct vp_stream_params {
     float gainPitch, gainVoice, gainSynth, gainVoc; /* dB, [-60, 6]; the dry paths are on above -59 dB */
     int keyPitch;                                   /* 0..12 */
 } vp_stream_params;
+
+/* The vocoder's two LPC orders of one stream (VocoderProcess.cpp:193-194, read at every vocoder frame start): they set the
+ * stream's timbre and move no frame grid. 8 bytes. */
+typedef struct vp_stream_orders {
+    int lpcVoice;  /* [2, 100] */
+    int lpcSynth;  /* [2, 30] */
+} vp_stream_orders;
 
 /* Sizes prepareToPlay derives from the sample rate
  * (PluginProcessor.cpp:160-176, PitchProcess.cpp:100-107, MyBuffer.cpp:46-48). */
@@ -138,8 +146,9 @@ int vp_engine_prepare(vp_engine* e, double sampleRate, int samplesPerBlock, int 
  * freezes relative to the block, frames in flight still come out), a block with pitchBool off is PitchProcess::silence()
  * (PluginProcessor.cpp:214-221, PitchProcess.cpp:146-158). lpcPitch is read in PitchProcess::prepare only (:70): a change on
  * a running stream is ignored until the next vp_engine_prepare, as in the reference.
- * The five per-instance fields (gainPitch, gainVoice, gainSynth, gainVoc, keyPitch) are written to EVERY stream, replacing
- * what vp_engine_set_stream_params set: a caller that never sets streams one by one has one parameter set for the batch. */
+ * The five per-instance fields (gainPitch, gainVoice, gainSynth, gainVoc, keyPitch) and the orders lpcVoice / lpcSynth are
+ * written to EVERY stream, replacing what vp_engine_set_stream_params / vp_engine_set_stream_orders set: a caller that never
+ * sets streams one by one has one parameter set for the batch. */
 int vp_engine_set_params(vp_engine* e, const vp_params* p);
 /* Per-stream key and gains: streams firstStream .. firstStream + count - 1 take p[0 .. count). Valid after vp_engine_prepare,
  * which sets every stream from the engine's vp_params (VP_E_STATE before). A range outside [0, nStreams) is VP_E_ARG; a
@@ -179,6 +188,37 @@ typedef struct vp_stream_event {
  * nBlocks of device memory, allocated at the first such call outside the workspace budget: VP_E_NOMEM before anything is
  * issued when it cannot be had). */
 int vp_engine_schedule_stream_params(vp_engine* e, const vp_stream_event* events, int count);
+
+/* Per-stream vocoder orders: streams firstStream .. firstStream + count - 1 take o[0 .. count). Valid after vp_engine_prepare,
+ * which sets every stream from the engine's vp_params (VP_E_STATE before). A range outside [0, nStreams) or o == NULL is
+ * VP_E_ARG; an order outside the plug-in's ranges ([2, 100] / [2, 30]) is VP_E_RANGE; an order above what the workspace was
+ * sized for (the orders at vp_engine_prepare or vp_engine_reserve_orders, at least 40 / 5) is VP_E_STATE. On any error no
+ * stream changes. A new value takes effect from the next block on, at the start of each vocoder frame (VocoderProcess.cpp:
+ * 193-194): frames in flight keep the order they started with. Setting the values a stream already has costs nothing;
+ * vp_engine_reset and vp_engine_reset_streams keep them. A call in which every stream has the same orders in every block runs
+ * exactly the kernels an engine with those orders in its vp_params runs; otherwise the Levinson kernels solve each frame at
+ * its own orders, and every stream's coefficient rows are as wide as the widest (zero padded: a call whose orders are all
+ * <= 40 / <= 5 keeps the tuned autocorrelation and synthesis kernels). */
+int vp_engine_set_stream_orders(vp_engine* e, int firstStream, int count, const vp_stream_orders* o);
+/* The values in force at the last block issued (after a call with scheduled changes: at its last block). */
+int vp_engine_get_stream_orders(const vp_engine* e, int firstStream, int count, vp_stream_orders* out);
+
+/* Block-accurate order automation: stream `stream` takes o from absolute block `block` on. 24 bytes. */
+typedef struct vp_stream_order_event {
+    int stream;
+    int reserved;     /* 0 */
+    long long block;
+    vp_stream_orders o;
+} vp_stream_order_event;
+/* The rules of vp_engine_schedule_stream_params, for the orders: a value scheduled at block b applies to every vocoder frame
+ * whose delayed-timeline start lies in block b or later; one call, any cut into calls, and vp_engine_stream_block give
+ * bit-identical output and frame records. VP_E_STATE before vp_engine_prepare; VP_E_ARG for count < 0, a NULL list, a stream
+ * outside [0, nStreams) or a block already issued; VP_E_RANGE / VP_E_STATE for values as vp_engine_set_stream_orders; on any
+ * error nothing is queued. The same (stream, block) twice: the later one wins. vp_engine_set_stream_orders /
+ * vp_engine_set_params change the value from the next block on and leave pending events in place; vp_engine_reset and
+ * vp_engine_prepare drop every pending event, vp_engine_reset_streams those of the listed streams. Order and parameter events
+ * share the per-block table of a call (see vp_engine_schedule_stream_params for its cost). */
+int vp_engine_schedule_stream_orders(vp_engine* e, const vp_stream_order_event* events, int count);
 /* Behaviour at the places where the reference's C++ has undefined behaviour (SURVEY.md App. B U1-U6):
  *   VP_MODE_PARITY  (default) what the reference build actually does: the stale vector slot of PitchProcess.cpp:818 and the
  *                   popped table slot of Notes.cpp:99 are modelled, the other sites keep going and the frame is flagged VP_PF_UB;
@@ -216,7 +256,7 @@ int vp_engine_reset(vp_engine* e);
 /* Per-stream counterpart of vp_engine_reset, for a host that hands a slot of a running batch to a new plug-in instance
  * (user, track): streams[0 .. count) continue as streams that have received ZEROS on every input channel since
  * vp_engine_prepare / vp_engine_reset -- their rings, histories, pitch marks and the frames of theirs still in flight are
- * forgotten. The frame grids are shared by all streams (vocBool / pitchBool / LPC orders are per engine), so a reset stream
+ * forgotten. The frame grids are shared by all streams (vocBool / pitchBool are per engine), so a reset stream
  * keeps the batch's grid phase: it is exactly a freshly prepared instance only where the grids are in their prepare phase
  * (no vocBool / pitchBool-off block since prepare, and blocksDone * samplesPerBlock a multiple of both frame hops -- every
  * 3rd block at 44.1 kHz / 1024). Elsewhere it is what the reference's processBlock gives for zeros up to that block.
@@ -228,13 +268,16 @@ int vp_engine_reset(vp_engine* e);
  * pending vp_engine_schedule_stream_params events: a slot handed to a new user does not inherit the old user's automation
  * (the other streams keep theirs). Keeps the engine-wide parameters, the grids, every other
  * stream (bit for bit) and the records of the most recent call (get_pitch_frames / get_voc_frames); does not clear the
- * failed mark of a half-done call (only vp_engine_reset / vp_engine_prepare do, and both drop pending stream resets).
+ * failed mark of a half-done call (only vp_engine_reset / vp_engine_prepare do, and both drop pending stream resets). The
+ * listed streams keep their vp_stream_orders and drop their pending vp_engine_schedule_stream_orders events as well.
  * Streaming needs no new graph capture for it. Cost: one kernel launch in the next call, none when no reset is pending. */
 int vp_engine_reset_streams(vp_engine* e, const int* streams, int count);
 
 /* Host-only helper (no CUDA): the frame grids a sequence of process calls produces -- call c processes nBlocks[c] blocks
  * with params[c] in force (only vocBool, pitchBool, lpcVoice, lpcSynth matter). For hosts that want to know how many frame
- * records a call will report, and for the CPU tests of the grid bookkeeping. */
+ * records a call will report, and for the CPU tests of the grid bookkeeping. The orders are the engine-wide ones: the plan
+ * describes a batch whose streams all have params[c]'s lpcVoice / lpcSynth (rowOrderV / rowOrderS of a call with per-stream
+ * orders are the widest of its streams, at least 40 / 5). */
 typedef struct vp_call_plan {
     long long firstBlock;        /* blocks processed before this call */
     int offV, nFramesV;          /* first new vocoder frame (samples after the call's start) and how many start in the call */

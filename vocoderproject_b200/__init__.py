@@ -32,6 +32,7 @@ ABI_SYMBOLS = [
     "vp_engine_timer_elapsed_ms", "vp_engine_last_timing_counts", "vp_measure_peaks2", "vp_engine_reset", "vp_engine_stream_buffers", "vp_engine_stream_block",
     "vp_engine_stream_stats", "vp_engine_get_info", "vp_engine_reserve_orders", "vp_grid_plan", "vp_engine_set_mode", "vp_engine_process_host_pcm16", "vp_engine_set_window",
     "vp_engine_set_stream_params", "vp_engine_get_stream_params", "vp_engine_reset_streams", "vp_engine_schedule_stream_params",
+    "vp_engine_set_stream_orders", "vp_engine_get_stream_orders", "vp_engine_schedule_stream_orders",
 ]
 
 
@@ -56,6 +57,22 @@ STREAM_PARAM_FIELDS = tuple(k for k, _ in StreamParams._fields_)
 class StreamEvent(C.Structure):
     """vp_stream_event: stream `stream` takes p from absolute block `block` on (blocks since prepare / reset). 40 bytes."""
     _fields_ = [("stream", C.c_int), ("reserved", C.c_int), ("block", C.c_longlong), ("p", StreamParams), ("pad", C.c_int)]
+
+
+class StreamOrders(C.Structure):
+    """vp_stream_orders: the vocoder's two LPC orders of one stream. 8 bytes."""
+    _fields_ = [("lpcVoice", C.c_int), ("lpcSynth", C.c_int)]
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k, _ in self._fields_}
+
+
+STREAM_ORDER_FIELDS = tuple(k for k, _ in StreamOrders._fields_)
+
+
+class StreamOrderEvent(C.Structure):
+    """vp_stream_order_event: stream `stream` takes the orders o from absolute block `block` on. 24 bytes."""
+    _fields_ = [("stream", C.c_int), ("reserved", C.c_int), ("block", C.c_longlong), ("o", StreamOrders)]
 
 
 def stream_params(**kw):
@@ -149,6 +166,9 @@ def load_library(path=None):
         "vp_engine_reset": (i, [vp]),
         "vp_engine_reset_streams": (i, [vp, C.POINTER(i), i]),
         "vp_engine_schedule_stream_params": (i, [vp, C.POINTER(StreamEvent), i]),
+        "vp_engine_set_stream_orders": (i, [vp, i, i, C.POINTER(StreamOrders)]),
+        "vp_engine_get_stream_orders": (i, [vp, i, i, C.POINTER(StreamOrders)]),
+        "vp_engine_schedule_stream_orders": (i, [vp, C.POINTER(StreamOrderEvent), i]),
         "vp_engine_stream_buffers": (i, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]),
         "vp_engine_stream_block": (i, [vp]),
         "vp_engine_stream_stats": (i, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
@@ -332,7 +352,7 @@ class Engine:
         self._check(self.lib.vp_engine_set_mode(self.h, int(mode)))
 
     def set_params(self, params):
-        """Engine-wide parameters; the key and gains go to every stream (replacing per-stream values)."""
+        """Engine-wide parameters; the key, the gains and the vocoder orders go to every stream (replacing per-stream values)."""
         self._check(self.lib.vp_engine_set_params(self.h, C.byref(params)))
         self.params = params
 
@@ -395,6 +415,63 @@ class Engine:
         arr = (StreamParams * max(int(count), 1))()
         self._check(self.lib.vp_engine_get_stream_params(self.h, int(first), int(count), arr))
         return [arr[k].as_dict() for k in range(int(count))]
+
+    def set_stream_orders(self, first, items):
+        """Vocoder orders (lpcVoice, lpcSynth) of streams first .. first + len(items) - 1; items are StreamOrders, dicts
+        (missing fields keep the stream's current value) or (lpcVoice, lpcSynth) pairs. Takes effect from the next block on,
+        at each vocoder frame start."""
+        items = list(items)
+        cur = self.stream_orders(first, len(items)) if any(isinstance(it, dict) for it in items) else None
+        arr = (StreamOrders * max(len(items), 1))()
+        for k, it in enumerate(items):
+            if isinstance(it, StreamOrders):
+                C.memmove(C.byref(arr[k]), C.byref(it), C.sizeof(StreamOrders))
+            elif isinstance(it, dict):
+                for f in it:
+                    if f not in STREAM_ORDER_FIELDS:
+                        raise KeyError(f)
+                for f in STREAM_ORDER_FIELDS:
+                    setattr(arr[k], f, int(it[f] if f in it else cur[k][f]))
+            else:
+                arr[k].lpcVoice, arr[k].lpcSynth = int(it[0]), int(it[1])
+        self._check(self.lib.vp_engine_set_stream_orders(self.h, int(first), len(items), arr))
+
+    def stream_orders(self, first=0, count=None):
+        """[dict] of the vocoder orders of streams first .. first + count - 1 (default: to the last stream)."""
+        if count is None:
+            count = self.n_streams - int(first)
+        arr = (StreamOrders * max(int(count), 1))()
+        self._check(self.lib.vp_engine_get_stream_orders(self.h, int(first), int(count), arr))
+        return [arr[k].as_dict() for k in range(int(count))]
+
+    def schedule_stream_orders(self, events):
+        """Block-accurate order automation: events = [(stream, block, orders), ...] with the rules of
+        schedule_stream_params; orders is a StreamOrders, a (lpcVoice, lpcSynth) pair or a dict whose missing fields are
+        the stream's orders just before that block as far as this call can tell. On an error nothing is queued."""
+        events = list(events)
+        cur = self.stream_orders() if any(isinstance(v, dict) for _, _, v in events) else None
+        order = sorted(range(len(events)), key=lambda k: (int(events[k][1]), k))
+        last = {}
+        arr = (StreamOrderEvent * max(len(events), 1))()
+        for k in order:
+            s, b, v = events[k]
+            s, b = int(s), int(b)
+            e = arr[k]
+            e.stream, e.block, e.reserved = s, b, 0
+            if isinstance(v, StreamOrders):
+                vals = v.as_dict()
+            elif isinstance(v, dict):
+                for f in v:
+                    if f not in STREAM_ORDER_FIELDS:
+                        raise KeyError(f)
+                base = last.get(s) or (cur[s] if 0 <= s < len(cur) else {"lpcVoice": 40, "lpcSynth": 5})
+                vals = dict(base)
+                vals.update(v)
+            else:
+                vals = {"lpcVoice": int(v[0]), "lpcSynth": int(v[1])}
+            e.o.lpcVoice, e.o.lpcSynth = int(vals["lpcVoice"]), int(vals["lpcSynth"])
+            last[s] = vals
+        self._check(self.lib.vp_engine_schedule_stream_orders(self.h, arr, len(events)))
 
     # ---- host-buffer API (what a plug-in host calls) ----
     def process(self, voice, synthL, synthR=None, want_right=True):

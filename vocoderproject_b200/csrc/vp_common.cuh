@@ -28,7 +28,9 @@ struct VPGeom {
     long long pstride; // same for the pitch path
     int nFramesV;      // vocoder frames with start < n   (VocoderProcess.cpp:176)
     int nFramesP;      // pitch frames with start < n     (PitchProcess.cpp:169)
-    int ordV, ordS, ordP;
+    int ordV, ordS, ordP;  // analysis row orders of the call's frames (every frame's own order when ordTab is 0)
+    int ordTab;            // 1: the streams' orders differ -- the Levinson kernels take each frame's own orders from the
+                           // parameter table at its start block (VPStreamParam::ordV / ordS <= ordV / ordS)
     int vocOn, pitchOn;
     double yinEps;  // relative margin below which the FP32 YIN decision is re-done in FP64
     // ---- continuation (consecutive process calls = consecutive processBlock calls). Kernels work in CALL-LOCAL
@@ -176,8 +178,9 @@ struct __align__(16) VPStreamParam {
     float gainVocF, gainPitchF, gainVoiceF, gainSynthF;
     int key;             // Notes::key 0..12: row of the note LUTs
     int dryOn, synthOn;  // dry voice / dry side-chain mixed in
-    int pad;
+    int16_t ordV, ordS;  // vocoder LPC orders (vp_stream_orders): read by the Levinson kernels when VPGeom::ordTab is set
 };
+static_assert(sizeof(VPStreamParam) == 32, "one table entry is 32 bytes");
 
 // ---- kernel launchers (one per .cu file) -------------------------------------
 struct VPTables {

@@ -27,8 +27,8 @@ thread_local cudaError_t g_vpLaunchError = cudaSuccess;  // per host thread: eng
 
 // ---------------------------------------------------------------------------
 // Frame grids: absolute positions on the delayed timeline. Every stream of an engine shares them (the parameters that move
-// the grids -- vocBool, pitchBool, the LPC orders -- are per engine; only the key and the gains are per stream), so this is
-// plain host state; it is what VocoderProcess::startSample, PitchProcess::startSample and
+// the grids -- vocBool, pitchBool -- are per engine; the key, the gains and the vocoder orders are per stream and move no
+// grid), so this is plain host state; it is what VocoderProcess::startSample, PitchProcess::startSample and
 // PitchProcess::nChunk are in the reference, plus the bookkeeping of the frames that outlive the call they started in.
 // Pure host logic (no CUDA): vp_grid_plan runs it stand-alone.
 // ---------------------------------------------------------------------------
@@ -38,7 +38,7 @@ struct GridState {
     long long blocksDone = 0;          // host blocks processed since prepare / reset
     long long nextFrameV = 0;          // start of the next vocoder frame = block start + VocoderProcess::startSample
     int alignedV = 0;                  // carried vocoder frames that lie on the current grid: carry rows VP_VC - alignedV .. VP_VC - 1
-    int alignedOrdV[VP_VC] = {0}, alignedOrdS[VP_VC] = {0};  // their analysis orders, by carry row
+    int alignedOrdV[VP_VC] = {0}, alignedOrdS[VP_VC] = {0};  // their analysis row orders (largest over the streams), by carry row
     long long orphAbs[VP_ORPH];        // frames left off the grid by a vocBool-off stretch: absolute start, -1 = free slot
     int orphOrdV[VP_ORPH] = {0}, orphOrdS[VP_ORPH] = {0};
     long long nextChunkP = 0;          // start of the next pitch chunk = block start + PitchProcess::startSample
@@ -85,21 +85,27 @@ struct vp_engine {
     // ---- per-stream parameters (vp_engine_set_stream_params): what each stream's plug-in instance holds, in dB, and the
     // table the kernels read (spTab on the host, dSP on the device, [S]). A changed table goes up through the pinned staging
     // buffer spPinned on the engine's stream before the next call's first kernel; evSpUp marks when that copy has read it.
+    // The vocoder orders of each stream (vp_engine_set_stream_orders) are kept beside them (sord) and ride in the same table.
     std::vector<vp_stream_params> sprm;
+    std::vector<vp_stream_orders> sord;
     std::vector<VPStreamParam> spTab;
     VPStreamParam *spPinned = nullptr, *dSP = nullptr;
     cudaEvent_t evSpUp = nullptr;
     bool spDirty = false;
     bool anyDry = false, anySynth = false;  // some stream has a dry path (voice or side-chain) / the dry side-chain on
     bool pitchGainUniform = true;           // every stream has the same gainPitch (k_pitch_iir then takes it as an argument)
+    bool ordUniform = true;                 // every stream has the orders of spTab[0]
+    int ordMaxV = 0, ordMaxS = 0;           // largest orders over the streams
     bool capturing = false;                 // a streaming graph is being captured: nothing table-derived may be baked in
     // ---- scheduled per-stream changes (vp_engine_schedule_stream_params): pending events by (absolute block, stream). A call
     // takes those at its first block into the [S] table (= vp_engine_set_stream_params before it) and those after it into
     // callEv; a call with callEv non-empty reads the block-indexed table dSPB [nBlocks][S], which k_expand_stream_params
     // builds from dSP and the events (uploaded through the pinned staging buffer schPinned; evSchUp marks when that copy
-    // has read it). dSPB is allocated at the first such call, outside the workspace budget.
-    struct CallEvent { int blk, stream; vp_stream_params p; VPStreamParam v; };
-    std::map<std::pair<long long, int>, vp_stream_params> sched;
+    // has read it). dSPB is allocated at the first such call, outside the workspace budget. Parameter and order events
+    // (vp_engine_schedule_stream_orders) of one (block, stream) share an entry; a CallEvent holds the full values in force.
+    struct Pending { bool hasP = false, hasO = false; vp_stream_params p; vp_stream_orders o; };
+    struct CallEvent { int blk, stream; vp_stream_params p; vp_stream_orders o; VPStreamParam v; };
+    std::map<std::pair<long long, int>, Pending> sched;
     std::vector<CallEvent> callEv;
     VPStreamParam* dSPB = nullptr;
     uint8_t *schPinned = nullptr, *dSch = nullptr;
@@ -111,6 +117,9 @@ struct vp_engine {
     int callStride = 0;
     bool callAnyDry = false, callAnySynth = false, callPgUniform = true;
     float callPg = 0.0f;
+    // the call's vocoder orders: every stream has callOrdV / callOrdS in every block (callOrdTab false), else the largest
+    bool callOrdTab = false;
+    int callOrdV = 0, callOrdS = 0;
     // workspace (device), sized for Sc streams x maxBlocks
     uint8_t* dGate = nullptr;
     double* dGatePart = nullptr;
@@ -492,20 +501,22 @@ extern "C" int vp_engine_reserve_orders(vp_engine* e, int maxLpcVoice, int maxLp
     return VP_OK;
 }
 
-static VPStreamParam stream_table_entry(const vp_stream_params& p) {
+static VPStreamParam stream_table_entry(const vp_stream_params& p, const vp_stream_orders& o) {
     VPStreamParam q;
     memset(&q, 0, sizeof q);
     q.gainVocF = db_to_gain(p.gainVoc); q.gainPitchF = db_to_gain(p.gainPitch);
     q.gainVoiceF = db_to_gain(p.gainVoice); q.gainSynthF = db_to_gain(p.gainSynth);
     q.key = p.keyPitch;
     q.dryOn = p.gainVoice > -59.0f; q.synthOn = p.gainSynth > -59.0f;
+    q.ordV = (int16_t)o.lpcVoice; q.ordS = (int16_t)o.lpcSynth;
     return q;
 }
 
-// stream s takes the values v; true when its table entry changed
-static bool put_one_stream(vp_engine* e, int s, const vp_stream_params& v) {
-    const VPStreamParam t = stream_table_entry(v);
+// stream s takes the values v and the orders o; true when its table entry changed
+static bool put_one_stream(vp_engine* e, int s, const vp_stream_params& v, const vp_stream_orders& o) {
+    const VPStreamParam t = stream_table_entry(v, o);
     e->sprm[s] = v;
+    e->sord[s] = o;
     if (memcmp(&e->spTab[s], &t, sizeof t) == 0) return false;
     e->spTab[s] = t;
     return true;
@@ -515,18 +526,26 @@ static bool put_one_stream(vp_engine* e, int s, const vp_stream_params& v) {
 static void stream_table_changed(vp_engine* e) {
     e->spDirty = true;
     e->anyDry = e->anySynth = false;
-    e->pitchGainUniform = true;
+    e->pitchGainUniform = e->ordUniform = true;
+    e->ordMaxV = e->ordMaxS = 0;
     for (const VPStreamParam& t : e->spTab) {
         e->anyDry = e->anyDry || t.dryOn || t.synthOn;
         e->anySynth = e->anySynth || t.synthOn;
         e->pitchGainUniform = e->pitchGainUniform && t.gainPitchF == e->spTab[0].gainPitchF;
+        e->ordUniform = e->ordUniform && t.ordV == e->spTab[0].ordV && t.ordS == e->spTab[0].ordS;
+        e->ordMaxV = std::max(e->ordMaxV, (int)t.ordV); e->ordMaxS = std::max(e->ordMaxS, (int)t.ordS);
     }
 }
 
-// streams [first, first + count) take the values p[0 .. count); only a changed table entry makes the next call upload
-static void put_stream_params(vp_engine* e, int first, int count, const vp_stream_params* p, size_t pStep) {
+// streams [first, first + count) take the values p[0 .. count) (p == NULL: keep theirs) and the orders o[0 .. count)
+// (o == NULL: keep theirs); only a changed table entry makes the next call upload
+static void put_streams(vp_engine* e, int first, int count, const vp_stream_params* p, size_t pStep, const vp_stream_orders* o,
+                        size_t oStep) {
     bool changed = false;
-    for (int i = 0; i < count; ++i) changed = put_one_stream(e, first + i, p[(size_t)i * pStep]) || changed;
+    for (int i = 0; i < count; ++i) {
+        const int s = first + i;
+        changed = put_one_stream(e, s, p ? p[(size_t)i * pStep] : e->sprm[s], o ? o[(size_t)i * oStep] : e->sord[s]) || changed;
+    }
     if (changed) stream_table_changed(e);
 }
 
@@ -534,6 +553,22 @@ static vp_stream_params stream_part(const vp_params& p) {
     vp_stream_params q;
     q.gainPitch = p.gainPitch; q.gainVoice = p.gainVoice; q.gainSynth = p.gainSynth; q.gainVoc = p.gainVoc; q.keyPitch = p.keyPitch;
     return q;
+}
+static vp_stream_orders order_part(const vp_params& p) { return vp_stream_orders{p.lpcVoice, p.lpcSynth}; }
+
+// VP_E_RANGE outside the plug-in's ranges, VP_E_STATE above what the workspace rows were sized for
+static int check_orders(vp_engine* e, const vp_stream_orders* o, size_t step, int count) {
+    for (int i = 0; i < count; ++i) {
+        const vp_stream_orders& q = o[(size_t)i * step];
+        if (q.lpcVoice < 2 || q.lpcVoice > 100 || q.lpcSynth < 2 || q.lpcSynth > 30) return vp_err(e, VP_E_RANGE, "order outside the plug-in's range");
+    }
+    for (int i = 0; i < count; ++i) {
+        const vp_stream_orders& q = o[(size_t)i * step];
+        if (q.lpcVoice > e->capV || q.lpcSynth > e->capS)
+            return vp_err(e, VP_E_STATE, "lpcVoice / lpcSynth beyond what vp_engine_prepare sized: vp_engine_reserve_orders before "
+                                         "vp_engine_prepare");
+    }
+    return VP_OK;
 }
 
 // The table goes up before the first kernel of a call, on the engine's stream. The staging buffer is rewritten only after
@@ -561,21 +596,65 @@ extern "C" int vp_engine_set_stream_params(vp_engine* e, int firstStream, int co
     if (firstStream < 0 || count < 0 || firstStream > e->S - count) return vp_err(e, VP_E_ARG, "stream range outside [0, nStreams)");
     for (int i = 0; i < count; ++i)
         if (!stream_params_ok(p[i])) return vp_err(e, VP_E_RANGE, "parameter outside the plug-in's range");
-    put_stream_params(e, firstStream, count, p, 1);
+    put_streams(e, firstStream, count, p, 1, nullptr, 0);
     return VP_OK;
 }
 
-extern "C" int vp_engine_schedule_stream_params(vp_engine* e, const vp_stream_event* ev, int count) {
-    if (!e) return VP_E_ARG;
+extern "C" int vp_engine_set_stream_orders(vp_engine* e, int firstStream, int count, const vp_stream_orders* o) {
+    if (!e || !o) return VP_E_ARG;
+    if (!e->prepared) return vp_err(e, VP_E_STATE, "vp_engine_prepare has not been called");
+    if (firstStream < 0 || count < 0 || firstStream > e->S - count) return vp_err(e, VP_E_ARG, "stream range outside [0, nStreams)");
+    const int rc = check_orders(e, o, 1, count);
+    if (rc) return rc;
+    put_streams(e, firstStream, count, nullptr, 0, o, 1);
+    return VP_OK;
+}
+
+extern "C" int vp_engine_get_stream_orders(const vp_engine* e, int firstStream, int count, vp_stream_orders* out) {
+    if (!e || !out) return VP_E_ARG;
+    if (!e->prepared) return VP_E_STATE;
+    if (firstStream < 0 || count < 0 || firstStream > e->S - count) return VP_E_ARG;
+    for (int i = 0; i < count; ++i) out[i] = e->sord[firstStream + i];
+    return VP_OK;
+}
+
+static_assert(sizeof(vp_stream_order_event) == 24 && sizeof(vp_stream_order_event) % sizeof(vp_stream_orders) == 0 &&
+              offsetof(vp_stream_order_event, o) % sizeof(vp_stream_orders) == 0, "event orders are checked as a strided list");
+
+// the checks every schedule call shares: state, list, streams, blocks not yet issued
+template <typename Ev>
+static int check_events(vp_engine* e, const Ev* ev, int count) {
     if (!e->prepared) return vp_err(e, VP_E_STATE, "vp_engine_prepare has not been called");
     if (count < 0 || (count > 0 && !ev)) return vp_err(e, VP_E_ARG, "events must be non-null and count >= 0");
     for (int i = 0; i < count; ++i) {
         if (ev[i].stream < 0 || ev[i].stream >= e->S) return vp_err(e, VP_E_ARG, "stream index outside [0, nStreams)");
         if (ev[i].block < e->gs.blocksDone) return vp_err(e, VP_E_ARG, "event for a block that has already been issued");
     }
+    return VP_OK;
+}
+
+extern "C" int vp_engine_schedule_stream_params(vp_engine* e, const vp_stream_event* ev, int count) {
+    if (!e) return VP_E_ARG;
+    int rc = check_events(e, ev, count);
+    if (rc) return rc;
     for (int i = 0; i < count; ++i)
         if (!stream_params_ok(ev[i].p)) return vp_err(e, VP_E_RANGE, "parameter outside the plug-in's range");
-    for (int i = 0; i < count; ++i) e->sched[{ev[i].block, ev[i].stream}] = ev[i].p;  // a later (stream, block) replaces an earlier one
+    for (int i = 0; i < count; ++i) {  // a later (stream, block) replaces an earlier one
+        vp_engine::Pending& q = e->sched[{ev[i].block, ev[i].stream}];
+        q.hasP = true; q.p = ev[i].p;
+    }
+    return VP_OK;
+}
+
+extern "C" int vp_engine_schedule_stream_orders(vp_engine* e, const vp_stream_order_event* ev, int count) {
+    if (!e) return VP_E_ARG;
+    int rc = check_events(e, ev, count);
+    if (rc) return rc;
+    if ((rc = check_orders(e, count > 0 ? &ev[0].o : nullptr, sizeof(vp_stream_order_event) / sizeof(vp_stream_orders), count))) return rc;
+    for (int i = 0; i < count; ++i) {
+        vp_engine::Pending& q = e->sched[{ev[i].block, ev[i].stream}];
+        q.hasO = true; q.o = ev[i].o;
+    }
     return VP_OK;
 }
 
@@ -618,9 +697,10 @@ extern "C" int vp_engine_set_params(vp_engine* e, const vp_params* p) {
         double freq[128];
         e->sz.nFreq = notes_table(q.keyPitch, 100.0, 800.0, freq);
     }
-    // the per-instance part goes to every stream (a caller that never sets streams one by one gets one parameter set)
+    // the per-instance part and the orders go to every stream (a caller that never sets streams one by one gets one set)
     const vp_stream_params sp = stream_part(q);
-    put_stream_params(e, 0, (int)e->sprm.size(), &sp, 0);
+    const vp_stream_orders so = order_part(q);
+    put_streams(e, 0, (int)e->sprm.size(), &sp, 0, &so, 0);
     return VP_OK;
 }
 
@@ -738,21 +818,45 @@ static int plan_schedule(vp_engine* e, int nBlocks) {
     const long long b0 = e->gs.blocksDone;
     bool changed = false;
     for (auto it = e->sched.begin(); it != e->sched.end() && it->first.first == b0;) {  // (no earlier block can be pending)
-        changed = put_one_stream(e, it->first.second, it->second) || changed;
+        const int s = it->first.second;
+        const vp_engine::Pending& q = it->second;
+        changed = put_one_stream(e, s, q.hasP ? q.p : e->sprm[s], q.hasO ? q.o : e->sord[s]) || changed;
         it = e->sched.erase(it);
     }
     if (changed) stream_table_changed(e);
     e->callEv.clear();
     const auto end = e->sched.lower_bound({b0 + nBlocks, INT_MIN});
-    for (auto it = e->sched.begin(); it != end; ++it)
-        e->callEv.push_back({(int)(it->first.first - b0), it->first.second, it->second, stream_table_entry(it->second)});
+    {   // each event carries the full values in force from its block on: a parameter event keeps the stream's orders at that
+        // block, an order event its parameters (ascending blocks: the stream's previous event in the list is the one before)
+        std::map<int, size_t> lastOf;
+        for (auto it = e->sched.begin(); it != end; ++it) {
+            const int s = it->first.second;
+            const vp_engine::Pending& q = it->second;
+            const auto prev = lastOf.find(s);
+            vp_stream_params p = prev != lastOf.end() ? e->callEv[prev->second].p : e->sprm[s];
+            vp_stream_orders o = prev != lastOf.end() ? e->callEv[prev->second].o : e->sord[s];
+            if (q.hasP) p = q.p;
+            if (q.hasO) o = q.o;
+            lastOf[s] = e->callEv.size();
+            e->callEv.push_back({(int)(it->first.first - b0), s, p, o, stream_table_entry(p, o)});
+        }
+    }
     e->callAnyDry = e->anyDry; e->callAnySynth = e->anySynth;
     e->callPg = e->spTab[0].gainPitchF; e->callPgUniform = e->pitchGainUniform;
+    e->callOrdV = e->spTab[0].ordV; e->callOrdS = e->spTab[0].ordS;
+    bool ordUniform = e->ordUniform;
+    int maxV = e->ordMaxV, maxS = e->ordMaxS;
     for (const auto& c : e->callEv) {
         e->callAnyDry = e->callAnyDry || c.v.dryOn || c.v.synthOn;
         e->callAnySynth = e->callAnySynth || c.v.synthOn;
         e->callPgUniform = e->callPgUniform && c.v.gainPitchF == e->callPg;
+        ordUniform = ordUniform && c.v.ordV == e->callOrdV && c.v.ordS == e->callOrdS;
+        maxV = std::max(maxV, (int)c.v.ordV); maxS = std::max(maxS, (int)c.v.ordS);
     }
+    // orders that differ between streams or blocks: rows as wide as the widest (at least the tuned kernels' 40 / 5), each
+    // frame solved at its own orders
+    e->callOrdTab = !ordUniform;
+    if (e->callOrdTab) { e->callOrdV = std::max(maxV, 40); e->callOrdS = std::max(maxS, 5); }
     e->callSP = e->dSP; e->callStride = 0;
     if (e->callEv.empty()) return VP_OK;
     if (!e->dSPB) {
@@ -815,7 +919,7 @@ static int issue_schedule(vp_engine* e, int nBlocks) {
                                    reinterpret_cast<const VPStreamParam*>(e->dSch + offB + blkB), e->dSPB, S, nBlocks);
     e->launches++;
     bool changed = false;
-    for (const auto& c : e->callEv) changed = put_one_stream(e, c.stream, c.p) || changed;  // ascending blocks: the last one stays
+    for (const auto& c : e->callEv) changed = put_one_stream(e, c.stream, c.p, c.o) || changed;  // ascending blocks: the last one stays
     if (changed) stream_table_changed(e);
     const long long b0 = e->gs.blocksDone;
     e->sched.erase(e->sched.begin(), e->sched.lower_bound({b0 + nBlocks, INT_MIN}));
@@ -938,10 +1042,9 @@ extern "C" int vp_engine_prepare(vp_engine* e, double fs, int B, int S, int maxB
     e->rsMark.assign((size_t)S, 0);
     e->rsList.clear();
     e->sprm.assign((size_t)S, stream_part(e->prm));
-    e->spTab.assign((size_t)S, stream_table_entry(e->sprm[0]));
-    e->spDirty = true;
-    e->anyDry = e->spTab[0].dryOn || e->spTab[0].synthOn; e->anySynth = e->spTab[0].synthOn != 0;
-    e->pitchGainUniform = true;
+    e->sord.assign((size_t)S, order_part(e->prm));
+    e->spTab.assign((size_t)S, stream_table_entry(e->sprm[0], e->sord[0]));
+    stream_table_changed(e);
     e->capV = capV; e->capS = capS; e->capP = capP;
     if ((rc = reset_state(e))) return rc;
     e->launches = e->yinRechecked = e->yinFrames = 0;
@@ -992,7 +1095,8 @@ static int make_geom(vp_engine* e, int nBlocks, size_t stride, VPGeom* g) {
     g->wstride = (long long)e->maxBlocks * e->B;
     g->vstride = g->pstride = g->wstride;
     g->vocOn = e->prm.vocBool != 0; g->pitchOn = e->prm.pitchBool != 0;
-    g->ordV = e->prm.lpcVoice; g->ordS = e->prm.lpcSynth; g->ordP = e->capP;
+    g->ordV = e->callOrdV; g->ordS = e->callOrdS; g->ordP = e->capP;  // (plan_schedule: the streams' orders in this call)
+    g->ordTab = e->callOrdTab;
     g->H = e->H;
     g->defined = e->mode == VP_MODE_DEFINED;
     grid_geom(e->gs, g);
@@ -1731,8 +1835,9 @@ extern "C" int vp_engine_stream_block(vp_engine* e) {
     e->lastBlocks = 1;
     e->lastG = g;
     // everything that shapes the launch sequence or is baked into kernel arguments
+    // (per-stream orders are table data; whether they differ, and the row orders, select the kernels)
     std::vector<long long> key = {e->gs.blocksDone > 0 ? 1 : 0, e->histCur, g.offV, g.offP, g.nFramesV, g.nFramesP, g.kV0, g.synV, g.synS,
-                                  g.vocOn, g.pitchOn, g.vocMix, g.pitchMix, e->callAnyDry};
+                                  g.vocOn, g.pitchOn, g.vocMix, g.pitchMix, e->callAnyDry, g.ordV, g.ordS, g.ordTab};
     for (int j = 0; j < VP_ORPH; ++j) { key.push_back(g.orphPos[j]); key.push_back(g.orphOrdV[j]); key.push_back(g.orphOrdS[j]); }
     for (int j = 0; j < VP_PC; ++j) { key.push_back(g.carryPosP[j]); key.push_back(g.carryLimP[j]); }
     auto it = e->graphs.find(key);

@@ -110,10 +110,12 @@ public:
         engine.check(vp_engine_prepare(engine.h, sampleRate, B, S, maxBlocks, 0));
         beginBlock();
     }
-    // the engine-wide parameters; the key and gains go to every stream (and replace what setStreamParams set)
+    // the engine-wide parameters; the key, the gains and the vocoder orders go to every stream (and replace what
+    // setStreamParams / setStreamOrders set)
     void setParams(const vp_params& p) {
         params = p;
         streamParams.clear();
+        streamOrders.clear();
         engine.check(vp_engine_set_params(engine.h, &params));
     }
     // key and gains of streams first .. first + count - 1 (after prepare); kept until the next setParams
@@ -124,6 +126,16 @@ public:
             engine.check(vp_engine_get_stream_params(engine.h, 0, S, streamParams.data()));
         } else {
             for (int i = 0; i < count; ++i) streamParams[(size_t)(first + i)] = p[i];
+        }
+    }
+    // vocoder orders (lpcVoice, lpcSynth) of streams first .. first + count - 1 (after prepare); kept until the next setParams
+    void setStreamOrders(int first, int count, const vp_stream_orders* o) {
+        engine.check(vp_engine_set_stream_orders(engine.h, first, count, o));
+        if (streamOrders.empty()) {
+            streamOrders.resize((size_t)S);
+            engine.check(vp_engine_get_stream_orders(engine.h, 0, S, streamOrders.data()));
+        } else {
+            for (int i = 0; i < count; ++i) streamOrders[(size_t)(first + i)] = o[i];
         }
     }
     // largest lpcVoice / lpcSynth that may be set while the streams run (before prepare; VocoderProcess.cpp:50-57 sizes its
@@ -141,6 +153,10 @@ public:
     // restartStreams those of the listed streams
     void scheduleStreamParams(const vp_stream_event* events, int count) {
         engine.check(vp_engine_schedule_stream_params(engine.h, events, count));
+    }
+    // the same for the vocoder orders: each event gives one stream its lpcVoice / lpcSynth from an absolute block on
+    void scheduleStreamOrders(const vp_stream_order_event* events, int count) {
+        engine.check(vp_engine_schedule_stream_orders(engine.h, events, count));
     }
     const vp_params& getParams() const { return params; }
 
@@ -160,6 +176,7 @@ public:
         engine.check(vp_engine_set_params(engine.h, &p));
         // per-stream values set since the last setParams: pushed again after the broadcast above (unchanged values cost nothing)
         if (!streamParams.empty()) engine.check(vp_engine_set_stream_params(engine.h, 0, S, streamParams.data()));
+        if (!streamOrders.empty()) engine.check(vp_engine_set_stream_orders(engine.h, 0, S, streamOrders.data()));
         engine.check(vp_engine_process_host(engine.h, blocks, inVoice, inSynthL, inSynthR, outL, outR, stride));
         beginBlock();
     }
@@ -174,6 +191,7 @@ private:
     void beginBlock() { vocRequested = pitchRequested = false; dryVoiceDb = drySynthDb = -60.0f; }
     vp_params params;
     std::vector<vp_stream_params> streamParams;  // [S] once setStreamParams was called, else empty
+    std::vector<vp_stream_orders> streamOrders;  // [S] once setStreamOrders was called, else empty
     vp_sizes sizes{};
     int B = 0, S = 0, maxBlocks = 1, blocks = 1;
     double sampleRate = 0;
@@ -266,6 +284,10 @@ public:
             if (streamParams.size() != (size_t)myBuffer.getNumStreams()) throw Error(VP_E_ARG, "streamParams must hold one entry per stream");
             myBuffer.setStreamParams(0, (int)streamParams.size(), streamParams.data());
         }
+        if (!streamOrders.empty()) {
+            if (streamOrders.size() != (size_t)myBuffer.getNumStreams()) throw Error(VP_E_ARG, "streamOrders must hold one entry per stream");
+            myBuffer.setStreamOrders(0, (int)streamOrders.size(), streamOrders.data());
+        }
         myBuffer.fillInputBuffers(voice, synthL, synthR, stride, nBlocks);   // :212
         if (params.vocBool) vocoderProcess.process(myBuffer);                // :214-215
         if (params.pitchBool) pitchProcess.process(myBuffer);                // :218-221
@@ -278,6 +300,9 @@ public:
     vp_params params;   // the ten plug-in parameters (PluginProcessor.cpp:37-73)
     // optional, one entry per stream: that instance's key and gains (its value tree); empty = params' values for every stream
     std::vector<vp_stream_params> streamParams;
+    // optional, one entry per stream: that instance's lpcVoice / lpcSynth; empty = params' orders for every stream (orders
+    // above params' need maxLpcVoice / maxLpcSynth at prepareToPlay)
+    std::vector<vp_stream_orders> streamOrders;
     std::string windowType = "sine";  // the literal prepareToPlay passes to VocoderProcess::prepare (:173); "hann" = the class's other branch
     MyBuffer myBuffer;
     VocoderProcess vocoderProcess;

@@ -517,7 +517,6 @@ __device__ void lev_solve(const double* r, double* a, int order) {
 __device__ double fir_energy(const double* r, const double* a, int order, int wlen, const double* __restrict__ xt) {
     double q = r[0];
     for (int k = 1; k <= order; ++k) q = fma(a[k], r[k], q);
-    double E = q * (double)wlen;
     // tail of the full convolution: i = wlen + d, d = 0..order-1, taps k = d+1..order on xw[wlen + d - k]
     double tail = 0.0;
     for (int d = 0; d < order; ++d) {
@@ -525,7 +524,9 @@ __device__ double fir_energy(const double* r, const double* a, int order, int wl
         for (int k = d + 1; k <= order; ++k) e = fma(a[k], xt[order + d - k], e);
         tail = fma(e, e, tail);
     }
-    E -= tail;
+    // q wlen rounded on its own, then the tail subtracted (spelled out: k_voc_levinson_static's per-frame form must round
+    // exactly like this for the orders that run here)
+    const double E = __dsub_rn(__dmul_rn(q, (double)wlen), tail);
     return E > 0.0 ? E : 0.0;
 }
 
@@ -537,24 +538,28 @@ __global__ void __launch_bounds__(128) k_voc_levinson(VPGeom g, VPTables tb, con
     if (idx >= (long long)S * g.nFramesV) return;
     const int s = (int)(idx / g.nFramesV), k = (int)(idx - (long long)s * g.nFramesV);
     const size_t row = vp_vrow(g, s, k);
+    const int b = (int)(((unsigned)k * (unsigned)g.hopV + (unsigned)g.offV) / (unsigned)g.B);  // block of the frame's start
+    // the frame's own orders: the stream's at its start block (VocoderProcess.cpp:193-194) when the call's streams differ;
+    // the rows are g.ordV / g.ordS wide, and their tails hold the LAST g.ordV / g.ordS windowed samples
+    int pv = g.ordV, ps = g.ordS;
+    if (g.ordTab) { const VPStreamParam& q = vp_sp(tb, b, s); pv = q.ordV; ps = q.ordS; }
     double r[VP_ORDER_MAX + 1], a[VP_ORDER_MAX + 1];
     {
         const double* rp = rV + (size_t)idx * vp_rowlen(g.ordV);
-        for (int m = 0; m <= g.ordV; ++m) r[m] = rp[m] / (double)g.wlenV;
-        lev_solve(r, a, g.ordV);
+        for (int m = 0; m <= pv; ++m) r[m] = rp[m] / (double)g.wlenV;
+        lev_solve(r, a, pv);
         double* ap = aV + row * (g.synV + 1);
-        for (int m = 0; m <= g.synV; ++m) ap[m] = (m <= g.ordV) ? a[m] : 0.0;  // zero padded up to the call's row order
-        EeV[row] = fir_energy(r, a, g.ordV, g.wlenV, rp + g.ordV + 1);
+        for (int m = 0; m <= g.synV; ++m) ap[m] = (m <= pv) ? a[m] : 0.0;  // zero padded up to the call's row order
+        EeV[row] = fir_energy(r, a, pv, g.wlenV, rp + g.ordV + 1 + (g.ordV - pv));
     }
     {
         const double* rp = rS + (size_t)idx * vp_rowlen(g.ordS);
-        for (int m = 0; m <= g.ordS; ++m) r[m] = rp[m] / (double)g.wlenV;
-        lev_solve(r, a, g.ordS);
+        for (int m = 0; m <= ps; ++m) r[m] = rp[m] / (double)g.wlenV;
+        lev_solve(r, a, ps);
         double* ap = aS + row * (g.synS + 1);
-        for (int m = 0; m <= g.synS; ++m) ap[m] = (m <= g.ordS) ? a[m] : 0.0;
-        const double eS = fir_energy(r, a, g.ordS, g.wlenV, rp + g.ordS + 1);
+        for (int m = 0; m <= g.synS; ++m) ap[m] = (m <= ps) ? a[m] : 0.0;
+        const double eS = fir_energy(r, a, ps, g.wlenV, rp + g.ordS + 1 + (g.ordS - ps));
         // a frame skipped by the silence gate (VocoderProcess.cpp:199-204) is marked with EeSynth = -1
-        const int b = (int)(((unsigned)k * (unsigned)g.hopV + (unsigned)g.offV) / (unsigned)g.B);
         const bool gated = (gate[(size_t)s * g.nBlocks + b] & (VP_GATE_VOICE | VP_GATE_SYNTH)) != 0;
         EeS[row] = gated ? -1.0 : eS;
     }
@@ -562,9 +567,14 @@ __global__ void __launch_bounds__(128) k_voc_levinson(VPGeom g, VPTables tb, con
 
 // rp / ap / xt point into SHARED memory (row of this thread, odd stride): the CTA stages them with coalesced,
 // batched global accesses, because 232 registers per thread leave no room to keep dozens of global loads in flight.
+// ord <= P: the frame's own order. The recursion stops there and the taps beyond it are +0.0, so the energy sums below
+// append exact zero terms (fma(+0, x, e) == e) after the real ones: bit-identical to solving at order `ord` (lev_solve /
+// fir_energy); the tail samples xt[P + d - k] are the same windowed samples wlen + d - k whatever the row's width.
+// fused: E = q wlen - tail in one rounding, as this kernel has always computed it at its own orders; else the product is
+// rounded first, as fir_energy does -- a frame gets the rounding of the kernel a call at its orders alone would run.
 template <int P>
 __device__ __forceinline__ double lev_energy_static(const double* __restrict__ rp, double* __restrict__ ap, int wlen,
-                                                    const double* __restrict__ xts) {
+                                                    const double* __restrict__ xts, int ord, bool fused) {
     double r[P + 1], a[P + 1];
     const double dw = (double)wlen, iw = 1.0 / dw;
 #pragma unroll
@@ -577,27 +587,28 @@ __device__ __forceinline__ double lev_energy_static(const double* __restrict__ r
         a[1] = r[1] / r[0];
 #pragma unroll
         for (int p = 2; p <= P; ++p) {
-            double rho = 0.0, ra = 0.0;
+            if (p <= ord) {
+                double rho = 0.0, ra = 0.0;
 #pragma unroll
-            for (int i = 1; i < p; ++i) { rho = fma(r[p - i], a[i], rho); ra = fma(r[i], a[i], ra); }
-            const double k = (r[p] - rho) / (r[0] - ra);
+                for (int i = 1; i < p; ++i) { rho = fma(r[p - i], a[i], rho); ra = fma(r[i], a[i], ra); }
+                const double k = (r[p] - rho) / (r[0] - ra);
 #pragma unroll
-            for (int i = 1; 2 * i <= p; ++i) {
-                const double t1 = a[i], t2 = a[p - i];
-                a[i] = fma(-k, t2, t1);
-                if (i != p - i) a[p - i] = fma(-k, t1, t2);
+                for (int i = 1; 2 * i <= p; ++i) {
+                    const double t1 = a[i], t2 = a[p - i];
+                    a[i] = fma(-k, t2, t1);
+                    if (i != p - i) a[p - i] = fma(-k, t1, t2);
+                }
+                a[p] = k;
             }
-            a[p] = k;
         }
 #pragma unroll
-        for (int i = 1; i <= P; ++i) a[i] = -a[i];
+        for (int i = 1; i <= P; ++i) a[i] = (i <= ord) ? -a[i] : 0.0;
     }
 #pragma unroll
     for (int m = 0; m <= P; ++m) ap[m] = a[m];
     double q = r[0];
 #pragma unroll
     for (int k = 1; k <= P; ++k) q = fma(a[k], r[k], q);
-    double E = q * (double)wlen;
     double xt[P];  // xt[t] = windowed sample wlen - P + t
 #pragma unroll
     for (int t = 0; t < P; ++t) xt[t] = xts[t];
@@ -609,13 +620,15 @@ __device__ __forceinline__ double lev_energy_static(const double* __restrict__ r
         for (int k = d + 1; k <= P; ++k) e = fma(a[k], xt[P + d - k], e);
         tail = fma(e, e, tail);
     }
-    E -= tail;
+    const double E = fused ? fma(q, dw, -tail) : __dsub_rn(__dmul_rn(q, dw), tail);
     return E > 0.0 ? E : 0.0;
 }
 
 #define LV_THREADS 64
 
-template <int PV, int PS>
+// TAB: the call's streams have different orders (g.ordTab) -- each frame is solved at its own. A separate instantiation:
+// at uniform 40 / 5 the per-frame form measured 2.1 ms per step slower (21.6 vs 19.5 ms, profiles/ab_stream_orders_r06.txt).
+template <int PV, int PS, bool TAB>
 __global__ void __launch_bounds__(LV_THREADS) k_voc_levinson_static(VPGeom g, VPTables tb, const float* __restrict__ voice,
                                                                     const float* __restrict__ synth, const uint8_t* __restrict__ gate,
                                                                     const double* __restrict__ rV, const double* __restrict__ rS,
@@ -644,13 +657,17 @@ __global__ void __launch_bounds__(LV_THREADS) k_voc_levinson_static(VPGeom g, VP
         const size_t orow = vp_vrow(g, s, k);
         sRow[tid] = orow;
         double* row = sR + tid * RS;
-        const double eS = lev_energy_static<PS>(row + RV, row + RV, wlen, row + RV + PS + 1);
+        const int b = (int)(((unsigned)k * (unsigned)g.hopV + (unsigned)g.offV) / (unsigned)g.B);  // block of the frame's start
+        // the frame's own orders when the call's streams differ (VocoderProcess.cpp:193-194: read at the frame start)
+        int pv = PV, ps = PS;
+        if (TAB) { const VPStreamParam& q = vp_sp(tb, b, s); pv = q.ordV; ps = q.ordS; }
+        const bool fused = pv == PV && ps == PS;  // (other orders alone run k_voc_levinson)
+        const double eS = lev_energy_static<PS>(row + RV, row + RV, wlen, row + RV + PS + 1, ps, fused);
         // a frame skipped by the silence gate (VocoderProcess.cpp:199-204) is marked with EeSynth = -1: the synthesis
         // kernel then needs no gate lookups for its 10-frame energy history
-        const int b = (int)(((unsigned)k * (unsigned)g.hopV + (unsigned)g.offV) / (unsigned)g.B);
         const bool gated = (gate[(size_t)s * g.nBlocks + b] & (VP_GATE_VOICE | VP_GATE_SYNTH)) != 0;
         EeS[orow] = gated ? -1.0 : eS;
-        EeV[orow] = lev_energy_static<PV>(row, row, wlen, row + PV + 1);
+        EeV[orow] = lev_energy_static<PV>(row, row, wlen, row + PV + 1, pv, fused);
     }
     __syncthreads();
     // coalesced coefficient rows out; the workspace row of each frame (carry rows per stream in front) was noted by its thread
@@ -668,12 +685,18 @@ void vp_launch_voc_levinson(cudaStream_t st, const VPGeom& g, const VPTables& tb
                             const float* synth, const uint8_t* gate, const double* rV, const double* rS, double* aV,
                             double* aS, double* EeV, double* EeS) {
     const long long tot = (long long)S * g.nFramesV;
+    // (a call with per-stream orders all <= 40 / <= 5 has 40 / 5 rows and takes this kernel too, in its per-frame form)
     if (g.ordV == 40 && g.ordS == 5 && g.synV == 40 && g.synS == 5 && g.wlenV >= 40)
     {
         const size_t smem = (size_t)LV_THREADS * ((vp_rowlen(40) + vp_rowlen(5)) | 1) * sizeof(double);
-        cudaFuncSetAttribute(k_voc_levinson_static<40, 5>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        VP_LAUNCH(k_voc_levinson_static<40, 5><<<(unsigned)((tot + LV_THREADS - 1) / LV_THREADS), LV_THREADS, smem, st>>>(
-            g, tb, voice, synth, gate, rV, rS, aV, aS, EeV, EeS, tot));
+        const unsigned grid = (unsigned)((tot + LV_THREADS - 1) / LV_THREADS);
+        if (g.ordTab) {
+            cudaFuncSetAttribute(k_voc_levinson_static<40, 5, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+            VP_LAUNCH(k_voc_levinson_static<40, 5, true><<<grid, LV_THREADS, smem, st>>>(g, tb, voice, synth, gate, rV, rS, aV, aS, EeV, EeS, tot));
+        } else {
+            cudaFuncSetAttribute(k_voc_levinson_static<40, 5, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+            VP_LAUNCH(k_voc_levinson_static<40, 5, false><<<grid, LV_THREADS, smem, st>>>(g, tb, voice, synth, gate, rV, rS, aV, aS, EeV, EeS, tot));
+        }
     }
     else
         VP_LAUNCH(k_voc_levinson<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(g, tb, gate, rV, rS, aV, aS, EeV, EeS, S));

@@ -2,10 +2,11 @@
 // instance = one stream,
 //
 //     voice.wav  sidechain.wav  out.wav  [key=N] [gainVoc=dB] [gainPitch=dB] [gainVoice=dB] [gainSynth=dB]
+//                                        [lpcVoice=N] [lpcSynth=N]
 //
 // (voice: channel 0 is used, PluginProcessor.cpp:153-157 mono main bus; side-chain: stereo, a mono file feeds both
-// channels). The optional tokens are that instance's own key and gains: they override the command-line values for the
-// job, so files in different keys or with different mixes still run as one batch. All jobs run as ONE batch on the GPU through the facade's prepareToPlay / processBlock (vp_facade.hpp):
+// channels). The optional tokens are that instance's own key, gains and vocoder orders: they override the command-line
+// values for the job, so files in different keys, with different mixes or timbres still run as one batch. All jobs run as ONE batch on the GPU through the facade's prepareToPlay / processBlock (vp_facade.hpp):
 // same sample rate for all files, shorter jobs are zero-padded to the longest and trimmed again on output.
 //
 //   vp_wavbatch manifest.txt [--block 1024] [--blocks-per-call 64] [--key 12] [--voc 0|1] [--pitch 0|1]
@@ -27,10 +28,11 @@
 #include "vp_facade.hpp"
 #include "vp_wav.hpp"
 
-struct Job { std::string voice, synth, out; vpb200::WavData v, s; vp_stream_params sp; };
+struct Job { std::string voice, synth, out; vpb200::WavData v, s; vp_stream_params sp; vp_stream_orders so; };
 
-// "name=value" tokens of a manifest line -> the job's per-instance parameters; false when any token is not one of them
-static bool parse_stream_tokens(std::istringstream& ls, vp_stream_params& sp, bool& any) {
+// "name=value" tokens of a manifest line -> the job's per-instance parameters; false when any token is not one of them.
+// any / anyOrd: some token set a key or gain / an order
+static bool parse_stream_tokens(std::istringstream& ls, vp_stream_params& sp, vp_stream_orders& so, bool& any, bool& anyOrd) {
     std::string tok;
     while (ls >> tok) {
         const size_t eq = tok.find('=');
@@ -42,6 +44,11 @@ static bool parse_stream_tokens(std::istringstream& ls, vp_stream_params& sp, bo
         if (name == "key") {
             if (x != (double)(int)x) return false;
             sp.keyPitch = (int)x;
+        } else if (name == "lpcVoice" || name == "lpcSynth") {
+            if (x != (double)(int)x) return false;
+            (name == "lpcVoice" ? so.lpcVoice : so.lpcSynth) = (int)x;
+            anyOrd = true;
+            continue;
         } else if (name == "gainVoc") sp.gainVoc = (float)x;
         else if (name == "gainPitch") sp.gainPitch = (float)x;
         else if (name == "gainVoice") sp.gainVoice = (float)x;
@@ -75,8 +82,9 @@ int main(int argc, char** argv) {
         else if (!strcmp(argv[i], "--help")) {
             printf("usage: vp_wavbatch manifest.txt [--block B] [--blocks-per-call K] [--key 0..12] [--voc 0|1] [--pitch 0|1] "
                    "[--gain-voice dB] [--gain-synth dB] [--gain-voc dB] [--gain-pitch dB] [--pcm16] [--keep-latency] [--device d]\n"
-                   "manifest lines: voice.wav sidechain.wav out.wav [key=N] [gainVoc=dB] [gainPitch=dB] [gainVoice=dB] [gainSynth=dB]\n"
-                   "  (the tokens set that job's key and gains; they override --key / --gain-* for the job)\n");
+                   "manifest lines: voice.wav sidechain.wav out.wav [key=N] [gainVoc=dB] [gainPitch=dB] [gainVoice=dB] [gainSynth=dB] "
+                   "[lpcVoice=N] [lpcSynth=N]\n"
+                   "  (the tokens set that job's key, gains and vocoder orders; they override --key / --gain-* for the job)\n");
             return 0;
         } else if (argv[i][0] != '-' && manifest.empty()) manifest = argv[i];
         else { fprintf(stderr, "unknown argument %s\n", argv[i]); return 2; }
@@ -84,7 +92,7 @@ int main(int argc, char** argv) {
     if (manifest.empty() || B <= 0 || K <= 0) { fprintf(stderr, "vp_wavbatch: no manifest (see --help)\n"); return 2; }
     try {
         std::vector<Job> jobs;
-        bool perJob = false;  // some line sets its own key or gains
+        bool perJob = false, perJobOrd = false;  // some line sets its own key or gains / its own orders
         {
             std::ifstream mf(manifest);
             if (!mf) throw std::runtime_error("cannot open " + manifest);
@@ -97,8 +105,10 @@ int main(int argc, char** argv) {
                 if (!(ls >> j.synth >> j.out)) throw std::runtime_error("manifest line needs three paths: " + line);
                 j.sp.gainPitch = prm.gainPitch; j.sp.gainVoice = prm.gainVoice; j.sp.gainSynth = prm.gainSynth;
                 j.sp.gainVoc = prm.gainVoc; j.sp.keyPitch = prm.keyPitch;
-                if (!parse_stream_tokens(ls, j.sp, perJob))
-                    throw std::runtime_error("manifest tokens after the paths are key=N gainVoc= gainPitch= gainVoice= gainSynth=: " + line);
+                j.so.lpcVoice = prm.lpcVoice; j.so.lpcSynth = prm.lpcSynth;
+                if (!parse_stream_tokens(ls, j.sp, j.so, perJob, perJobOrd))
+                    throw std::runtime_error("manifest tokens after the paths are key=N gainVoc= gainPitch= gainVoice= gainSynth= "
+                                             "lpcVoice=N lpcSynth=N: " + line);
                 jobs.push_back(std::move(j));
             }
         }
@@ -116,9 +126,13 @@ int main(int argc, char** argv) {
         const int S = (int)jobs.size();
         vpb200::VocoderBatchProcessor proc(device);
         proc.params = prm;
-        proc.prepareToPlay((double)fs, B, S, K);
+        int maxV = 0, maxS = 0;  // the workspace rows are sized for the largest order of the manifest
+        for (const Job& j : jobs) { maxV = std::max(maxV, j.so.lpcVoice); maxS = std::max(maxS, j.so.lpcSynth); }
+        proc.prepareToPlay((double)fs, B, S, K, maxV, maxS);
         if (perJob)
             for (const Job& j : jobs) proc.streamParams.push_back(j.sp);
+        if (perJobOrd)
+            for (const Job& j : jobs) proc.streamOrders.push_back(j.so);
         const size_t lat = keepLatency ? 0 : (size_t)proc.getLatencySamples();
         const size_t m = (size_t)K * B;
         const size_t nCalls = (longest + lat + m - 1) / m;
