@@ -14,17 +14,30 @@
 //   d[k]  = sum_{i<L} (x[q+i] - x[q+i+k])^2,  q = p - tauMax,  k < tauMax
 //   d'[k] = d[k] * k / sum_{j<=k} d[j]
 // Direct (a-b)^2 form: all terms positive, so FP32 accumulation keeps ~1e-6
-// relative accuracy even in deep minima. Thread tile: R consecutive lags x one
-// i-range, sliding window of R samples in registers (2 LDS per 2R FP32 ops;
-// odd R -> conflict-free window loads). CMND prefix sum, threshold search and
-// descent run on warp 0 in FP64. A frame whose deciding comparisons are within
-// yinEps (relative) is queued for the FP64 re-check kernel, which runs the same
-// code with T = double.
+// relative accuracy even in deep minima -- as long as the squares stay normal
+// floats. Below 2^-126 rounding is absolute (gradual underflow: up to 2^-150
+// per FFMA, squares under 2^-149 vanish), so d[k] also carries an error of up
+// to L 2^-150 that no relative margin covers (a frame of samples near 2^-75
+// has d[k] ~ 2^-140 and is decided on noise). Thread tile: R consecutive lags
+// x one i-range, sliding window of R samples in registers (2 LDS per 2R FP32
+// ops; odd R -> conflict-free window loads). CMND prefix sum, threshold search
+// and descent run on warp 0 in FP64. A frame whose deciding comparisons are
+// within yinEps (relative) or within the bound that the absolute error of d
+// puts on d' is queued for the FP64 re-check kernel, which runs the same code
+// with T = double (products of floats are normal doubles: no underflow term).
 // ===========================================================================
 #define YF_RECHECK 1u
 #define YF_NEAR 2u
 #define YF_UB 4u
 #define YF_DONE64 8u
+
+// Exclusive prefix over the lanes of a warp from the inclusive one: the previous lane's inclusive sum. (Not inclusive minus
+// own: where a lane's own lags are loud and the lags before them tiny -- a frame that ends where loud audio begins -- the
+// subtraction cancels and leaves rounding noise of the loud sum where the tiny prefix should be.)
+__device__ __forceinline__ double yin_lane_exclusive(double incl, int lane) {
+    const double prev = __shfl_up_sync(0xffffffffu, incl, 1);
+    return lane == 0 ? 0.0 : prev;
+}
 
 template <int R, typename T, bool MASK>
 __device__ __forceinline__ void yin_round(const float* __restrict__ xs, int nb, int nEnd, int k0, T* W, T* acc) {
@@ -78,8 +91,13 @@ __global__ void __launch_bounds__(512) k_yin(VPGeom g, const float* __restrict__
         const VPRow v = vp_row(voice, g.histV, s, g);
         const long long q = p - tauMax;
         __syncthreads();
-        for (int j = threadIdx.x; j < xsLen; j += blockDim.x) xs[j] = (j < L + tauMax) ? vp_x(v, q + j, g) : 0.0f;
-        __syncthreads();
+        int nzLoc = 0;
+        for (int j = threadIdx.x; j < xsLen; j += blockDim.x) {
+            const float x = (j < L + tauMax) ? vp_x(v, q + j, g) : 0.0f;
+            xs[j] = x;
+            nzLoc |= x != 0.0f;
+        }
+        const bool nonzero = __syncthreads_or(nzLoc) != 0;  // an all-zero frame is exact: d = 0, no error term
         {
             const int lt = threadIdx.x % LT, ig = threadIdx.x / LT;
             const int iLen = ((L + IG - 1) / IG + R - 1) / R * R;  // multiple of R
@@ -105,8 +123,14 @@ __global__ void __launch_bounds__(512) k_yin(VPGeom g, const float* __restrict__
         __syncthreads();
         if (threadIdx.x < 32) {
             const int lane = threadIdx.x;
+            const bool is64 = sizeof(T) == 8;
             const int per = (tauMax + 31) / 32;
             const int kA = lane * per, kB = min(kA + per, tauMax);
+            // FP32: absolute error bound of each d[k] from gradual underflow (L FFMAs, 2^-150 each, 25 % head room; the
+            // subtraction is exact where it underflows), and ep[k] = the resulting bound on d'[k] (part[] is free now)
+            const double eAbs = (!is64 && nonzero) ? (double)L * 0x1p-150 * 1.25 : 0.0;
+            double* ep = reinterpret_cast<double*>(part);
+            bool unsafe = false;
             // cumulative mean normalisation (PitchProcess.cpp:396-402); d'[0] = 1 and the sum starts at k = 1
             double loc = 0.0;
             for (int k = max(kA, 1); k < kB; ++k) loc += dp[k];
@@ -116,11 +140,17 @@ __global__ void __launch_bounds__(512) k_yin(VPGeom g, const float* __restrict__
                 const double t = __shfl_up_sync(0xffffffffu, incl, o);
                 if (lane >= o) incl += t;
             }
-            double run = incl - loc;
+            double run = yin_lane_exclusive(incl, lane);
             const double total = __shfl_sync(0xffffffffu, incl, 31);
             for (int k = max(kA, 1); k < kB; ++k) {
                 run += dp[k];
-                dp[k] = dp[k] * ((double)k / run);
+                const double dn = dp[k] * ((double)k / run);
+                if (eAbs > 0.0) {
+                    const double runE = eAbs * k;
+                    if (run > 2.0 * runE) ep[k] = (eAbs * ((double)k / run) + fabs(dn) * (runE / run)) * 1.01;
+                    else { ep[k] = 1e300; if (k >= g.tauMin) unsafe = true; }  // the sum itself is not resolved
+                }
+                dp[k] = dn;
             }
             if (lane == 0) dp[0] = 1.0;
             __syncwarp();
@@ -144,18 +174,26 @@ __global__ void __launch_bounds__(512) k_yin(VPGeom g, const float* __restrict__
                 for (int o = 16; o > 0; o >>= 1) stop = min(stop, __shfl_xor_sync(0xffffffffu, stop, o));
                 per_ = stop;
                 for (int k = max(kA, g.tauMin); k < kB; ++k) {
-                    if (k <= first) margin = fmin(margin, fabs(dp[k] - tol) / tol);
-                    if (k >= first && k <= stop && k + 1 < tauMax)
+                    if (k <= first) {
+                        margin = fmin(margin, fabs(dp[k] - tol) / tol);
+                        if (eAbs > 0.0 && !(fabs(dp[k] - tol) > ep[k])) unsafe = true;
+                    }
+                    if (k >= first && k <= stop && k + 1 < tauMax) {
                         margin = fmin(margin, fabs(dp[k + 1] - dp[k]) / fmax(fabs(dp[k]), 1e-300));
+                        if (eAbs > 0.0 && !(fabs(dp[k + 1] - dp[k]) > ep[k] + ep[k + 1])) unsafe = true;
+                    }
                 }
             } else if (total > 0.0) {
-                for (int k = max(kA, g.tauMin); k < kB; ++k) margin = fmin(margin, fabs(dp[k] - tol) / tol);
+                for (int k = max(kA, g.tauMin); k < kB; ++k) {
+                    margin = fmin(margin, fabs(dp[k] - tol) / tol);
+                    if (eAbs > 0.0 && !(fabs(dp[k] - tol) > ep[k])) unsafe = true;
+                }
             }
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) margin = fmin(margin, __shfl_xor_sync(0xffffffffu, margin, o));
+            unsafe = __any_sync(0xffffffffu, unsafe);
             if (lane == 0) {
-                const bool is64 = sizeof(T) == 8;
-                if (margin < (is64 ? 1e-12 : g.yinEps)) fl |= is64 ? YF_NEAR : YF_RECHECK;
+                if (margin < (is64 ? 1e-12 : g.yinEps) || unsafe) fl |= is64 ? YF_NEAR : YF_RECHECK;
                 if (is64) fl |= YF_DONE64;
                 period[fidx] = per_;
                 yflags[fidx] = fl;
@@ -228,8 +266,13 @@ void vp_launch_yin_recheck(cudaStream_t st, const VPGeom& g, int S, const float*
 //                  window loads; the a[n] load is a broadcast), 15-deep register window.
 //   k_yin_decide : one warp per frame, FP64: energies by running sums, CMND, threshold search and
 //                  descent, each deciding comparison checked against a rigorous bound on the FP32
-//                  accumulation error of C(k) (|err d[k]| <= c 2^-24 (A + B(k))); a frame with any
-//                  comparison inside its bound goes to the FP64 direct-form kernel above.
+//                  accumulation error of C(k),
+//                    |err d[k]| <= yin_corr_beta(c) (A + B(k)) + yin_corr_abs(c)   (0 where A + B(k) = 0):
+//                  a relative part for the roundings of normal floats and an absolute one for gradual
+//                  underflow (products and sums below 2^-126 round to multiples of 2^-149, products
+//                  below 2^-150 vanish: without it a frame of samples near 2^-70 is decided on noise,
+//                  with d[k] far outside the relative part). A frame with any comparison inside its
+//                  bound goes to the FP64 direct-form kernel above.
 // ===========================================================================
 #define YC_R 15
 #define YC_LAGS (32 * YC_R)  // lags per warp pass
@@ -373,6 +416,12 @@ __global__ void __launch_bounds__(32 * YC_CH, 4) k_yin_corr(VPGeom g, const floa
 __host__ __device__ inline double yin_corr_beta(int c) {
     return (double)(YC_SUB + c / YC_SUB + 4) * 5.9604644775390625e-08 * 1.25;
 }
+// absolute bound on |err d[k]| from gradual underflow: an FP32 rounding into the subnormal range is off by up to 2^-150
+// whatever the size of its result. C(k) = 4 chunk partials of c FFMAs + c / YC_SUB + 2 adds (k_yin_corr); x 2 for the 2 C
+// in d, 25 % head room. (A and B(k) are double sums of exact products: no underflow.)
+__host__ __device__ inline double yin_corr_abs(int c) {
+    return 2.0 * 4.0 * (double)(c + c / YC_SUB + 2) * 0x1p-150 * 1.25;
+}
 
 #define YD_WARPS 4
 
@@ -423,15 +472,15 @@ __global__ void __launch_bounds__(32 * YD_WARPS) k_yin_decide(VPGeom g, const fl
     double inc = locDelta;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) { const double t = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += t; }
-    double run = inc - locDelta;  // sum of deltas before kA
-    const double beta = yin_corr_beta(c);
+    double run = yin_lane_exclusive(inc, lane);  // sum of deltas before kA
+    const double beta = yin_corr_beta(c), eAbs = yin_corr_abs(c);
     double locD = 0.0, locE = 0.0;
     for (int k = kA; k < kB; ++k) {
         const double Bk = A + run;
         const double h = xhi[k], l = xlo[k];
         run += h * h - l * l;
         const double d = (k == 0) ? 0.0 : (A + Bk) - 2.0 * dp[k];
-        const double e = beta * (A + Bk);
+        const double e = (A + Bk > 0.0) ? fma(beta, A + Bk, eAbs) : 0.0;  // A + B(k) = 0: all samples 0, C(k) exact
         dp[k] = d;
         er[k] = e;
         if (k >= 1) { locD += d; locE += e; }
@@ -442,7 +491,7 @@ __global__ void __launch_bounds__(32 * YD_WARPS) k_yin_decide(VPGeom g, const fl
         const double t = __shfl_up_sync(0xffffffffu, incD, o), t2 = __shfl_up_sync(0xffffffffu, incE, o);
         if (lane >= o) { incD += t; incE += t2; }
     }
-    double runD = incD - locD, runE = incE - locE;
+    double runD = yin_lane_exclusive(incD, lane), runE = yin_lane_exclusive(incE, lane);
     const double total = __shfl_sync(0xffffffffu, incD, 31);
     const double energy = __shfl_sync(0xffffffffu, incE, 31);
     bool shaky = false;  // cumulative sum not resolved against its own error bound
@@ -593,15 +642,15 @@ __global__ void __launch_bounds__(256, (PER <= 9) ? YD9_CTAS : 2) k_yin_decide_r
     double inc = locDelta;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) { const double t = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += t; }
-    double run = inc - locDelta;
-    const double beta = yin_corr_beta(g.c);
+    double run = yin_lane_exclusive(inc, lane);  // sum of deltas before kA
+    const double beta = yin_corr_beta(g.c), eAbs = yin_corr_abs(g.c);
     double locD = 0.0, locE = 0.0;
 #pragma unroll
     for (int j = 0; j < PER; ++j) {
         const int k = kA + j;
         const double Bk = A + run;
         run += en[j];
-        double d = (A + Bk) - 2.0 * dn[j], e = beta * (A + Bk);
+        double d = (A + Bk) - 2.0 * dn[j], e = (A + Bk > 0.0) ? fma(beta, A + Bk, eAbs) : 0.0;  // 0: all samples 0, C(k) exact
         if (k == 0 || k >= kEnd) { d = 0.0; e = 0.0; }
         dn[j] = d;
         en[j] = e;
@@ -614,7 +663,7 @@ __global__ void __launch_bounds__(256, (PER <= 9) ? YD9_CTAS : 2) k_yin_decide_r
         const double t = __shfl_up_sync(0xffffffffu, incD, o), t2 = __shfl_up_sync(0xffffffffu, incE, o);
         if (lane >= o) { incD += t; incE += t2; }
     }
-    double runD = incD - locD, runE = incE - locE;
+    double runD = yin_lane_exclusive(incD, lane), runE = yin_lane_exclusive(incE, lane);
     const double total = __shfl_sync(0xffffffffu, incD, 31);
     const double energy = __shfl_sync(0xffffffffu, incE, 31);
     bool shaky = false;
