@@ -33,6 +33,7 @@ ABI_SYMBOLS = [
     "vp_engine_stream_stats", "vp_engine_get_info", "vp_engine_reserve_orders", "vp_grid_plan", "vp_engine_set_mode", "vp_engine_process_host_pcm16", "vp_engine_set_window",
     "vp_engine_set_stream_params", "vp_engine_get_stream_params", "vp_engine_reset_streams", "vp_engine_schedule_stream_params",
     "vp_engine_set_stream_orders", "vp_engine_get_stream_orders", "vp_engine_schedule_stream_orders",
+    "vp_engine_reserve_pitch_order", "vp_engine_set_stream_pitch_orders", "vp_engine_get_stream_pitch_orders",
 ]
 
 
@@ -169,6 +170,9 @@ def load_library(path=None):
         "vp_engine_set_stream_orders": (i, [vp, i, i, C.POINTER(StreamOrders)]),
         "vp_engine_get_stream_orders": (i, [vp, i, i, C.POINTER(StreamOrders)]),
         "vp_engine_schedule_stream_orders": (i, [vp, C.POINTER(StreamOrderEvent), i]),
+        "vp_engine_reserve_pitch_order": (i, [vp, i]),
+        "vp_engine_set_stream_pitch_orders": (i, [vp, i, i, C.POINTER(i)]),
+        "vp_engine_get_stream_pitch_orders": (i, [vp, i, i, C.POINTER(i), C.POINTER(i)]),
         "vp_engine_stream_buffers": (i, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]),
         "vp_engine_stream_block": (i, [vp]),
         "vp_engine_stream_stats": (i, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
@@ -273,7 +277,7 @@ class Engine:
     process(...) ~ nBlocks consecutive processBlock calls per stream."""
 
     def __init__(self, sample_rate, block, n_streams, max_blocks, params=None, device=0, workspace_bytes=0, reserve_orders=None,
-                 window=VP_WINDOW_SINE):
+                 window=VP_WINDOW_SINE, reserve_pitch_order=None):
         self.lib = load_library()
         self.h = C.c_void_p()
         rc = self.lib.vp_engine_create(C.byref(self.h), int(device))
@@ -286,6 +290,8 @@ class Engine:
             self._check(self.lib.vp_engine_set_window(self.h, int(window)))
         if reserve_orders:  # (maxLpcVoice, maxLpcSynth) that set_params may be given while the streams run
             self._check(self.lib.vp_engine_reserve_orders(self.h, int(reserve_orders[0]), int(reserve_orders[1])))
+        if reserve_pitch_order:  # largest lpcPitch that set_stream_pitch_orders may be given
+            self._check(self.lib.vp_engine_reserve_pitch_order(self.h, int(reserve_pitch_order)))
         self._check(self.lib.vp_engine_set_params(self.h, C.byref(self.params)))
         self._check(self.lib.vp_engine_prepare(self.h, self.sample_rate, self.block, self.n_streams, self.max_blocks,
                                                int(workspace_bytes)))
@@ -443,6 +449,24 @@ class Engine:
         arr = (StreamOrders * max(int(count), 1))()
         self._check(self.lib.vp_engine_get_stream_orders(self.h, int(first), int(count), arr))
         return [arr[k].as_dict() for k in range(int(count))]
+
+    def set_stream_pitch_orders(self, first, values):
+        """lpcPitch of streams first .. first + len(values) - 1: the order each starts with. In force from the next process
+        call for a stream that has processed no block since its last start (prepare, reset, or a pending reset_streams of
+        it); any other stream keeps its order until its next start."""
+        values = [int(v) for v in values]
+        arr = (C.c_int * max(len(values), 1))(*values)
+        self._check(self.lib.vp_engine_set_stream_pitch_orders(self.h, int(first), len(values), arr))
+
+    def stream_pitch_orders(self, first=0, count=None):
+        """(in_force, next): lists of the lpcPitch each of streams first .. first + count - 1 runs its next block at, and the
+        one it takes at its next start (default count: to the last stream)."""
+        if count is None:
+            count = self.n_streams - int(first)
+        a = (C.c_int * max(int(count), 1))()
+        b = (C.c_int * max(int(count), 1))()
+        self._check(self.lib.vp_engine_get_stream_pitch_orders(self.h, int(first), int(count), a, b))
+        return [a[k] for k in range(int(count))], [b[k] for k in range(int(count))]
 
     def schedule_stream_orders(self, events):
         """Block-accurate order automation: events = [(stream, block, orders), ...] with the rules of

@@ -31,6 +31,8 @@ struct VPGeom {
     int ordV, ordS, ordP;  // analysis row orders of the call's frames (every frame's own order when ordTab is 0)
     int ordTab;            // 1: the streams' orders differ -- the Levinson kernels take each frame's own orders from the
                            // parameter table at its start block (VPStreamParam::ordV / ordS <= ordV / ordS)
+    int ordTabP;           // 1: the streams' pitch orders differ -- rows are ordP + 1 wide (zero padded), the pitch Levinson and
+                           // all-pole kernels take each frame's own order from VPTables::ordP (<= ordP)
     int vocOn, pitchOn;
     double yinEps;  // relative margin below which the FP32 YIN decision is re-done in FP64
     // ---- continuation (consecutive process calls = consecutive processBlock calls). Kernels work in CALL-LOCAL
@@ -195,6 +197,8 @@ struct VPTables {
     const VPStreamParam* sp; // per-stream parameters of the pass's streams (table + streamBase): sp[blk * spStride + s], s = stream
                              // of the pass, blk = call-local block of the read site's delayed-timeline position (vp_sp)
     int spStride;            // 0: one entry per stream for the whole call; nStreams: a call with scheduled changes
+    const int16_t* ordP;     // lpcPitch in force for each stream of the pass (vp_engine_set_stream_pitch_orders), read when
+                             // VPGeom::ordTabP is set: fixed between two starts of a stream, so one entry per stream and call
 };
 // the parameters of stream s (of the pass) in force at call-local block blk
 __device__ __forceinline__ const VPStreamParam& vp_sp(const VPTables& tb, int blk, int s) {
@@ -233,8 +237,8 @@ void vp_launch_yin_recheck(cudaStream_t st, const VPGeom& g, int S, const float*
 void vp_launch_marks(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const float* voice,
                      const uint8_t* gate, const int* period, const uint32_t* yflags, vp_pitch_frame* frames,
                      VPMarkState* carry);
-void vp_launch_pitch_lpc(cudaStream_t st, const VPGeom& g, int S, const float* voice, const vp_pitch_frame* frames,
-                         double* rP, double* aP);
+void vp_launch_pitch_lpc(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const float* voice,
+                         const vp_pitch_frame* frames, double* rP, double* aP);
 void vp_launch_pitch_psola(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const float* voice,
                            vp_pitch_frame* frames, const double* aP, float* outE);
 // gainUniform: the gainPitch (as a gain) every stream has in every block of the call and that every carried chunk was

@@ -27,7 +27,7 @@ thread_local cudaError_t g_vpLaunchError = cudaSuccess;  // per host thread: eng
 
 // ---------------------------------------------------------------------------
 // Frame grids: absolute positions on the delayed timeline. Every stream of an engine shares them (the parameters that move
-// the grids -- vocBool, pitchBool -- are per engine; the key, the gains and the vocoder orders are per stream and move no
+// the grids -- vocBool, pitchBool -- are per engine; the key, the gains and the LPC orders are per stream and move no
 // grid), so this is plain host state; it is what VocoderProcess::startSample, PitchProcess::startSample and
 // PitchProcess::nChunk are in the reference, plus the bookkeeping of the frames that outlive the call they started in.
 // Pure host logic (no CUDA): vp_grid_plan runs it stand-alone.
@@ -97,6 +97,15 @@ struct vp_engine {
     bool ordUniform = true;                 // every stream has the orders of spTab[0]
     int ordMaxV = 0, ordMaxS = 0;           // largest orders over the streams
     bool capturing = false;                 // a streaming graph is being captured: nothing table-derived may be baked in
+    // ---- per-stream lpcPitch (vp_engine_set_stream_pitch_orders), read when a stream starts (PitchProcess::prepare, :70):
+    // pordNext = the order each stream starts with, pordIn = the order its next block runs at. pordIn changes only for a
+    // stream that has processed no block since its start, so no frame in flight ever sees a change. It goes up with the
+    // parameter table (through pordPinned, behind evSpUp) into dOrdP [S], which the kernels read when the orders differ.
+    std::vector<int> pordIn, pordNext;
+    int16_t *pordPinned = nullptr, *dOrdP = nullptr;
+    bool pordDirty = false;
+    bool pordUniform = true;  // every stream has pordIn[0]
+    int pordMax = 0;          // largest pordIn
     // ---- scheduled per-stream changes (vp_engine_schedule_stream_params): pending events by (absolute block, stream). A call
     // takes those at its first block into the [S] table (= vp_engine_set_stream_params before it) and those after it into
     // callEv; a call with callEv non-empty reads the block-indexed table dSPB [nBlocks][S], which k_expand_stream_params
@@ -182,6 +191,7 @@ struct vp_engine {
     int passCount = 0;      // passes of the current call
     int capV = 0, capS = 0, capP = 0;  // LPC orders the workspace was sized for
     int reserveV = 0, reserveS = 0;    // vp_engine_reserve_orders: largest lpcVoice / lpcSynth that may be set mid-stream
+    int reserveP = 0;                  // vp_engine_reserve_pitch_order: largest per-stream lpcPitch
     GridState gs;                      // frame grids and carried-frame bookkeeping (host side, shared by all streams)
     double *oAV = nullptr, *oAS = nullptr, *oEeS = nullptr, *oG = nullptr;  // orphan store [S][VP_ORPH][...]
     std::vector<cudaEvent_t> ev;
@@ -363,8 +373,9 @@ static void free_workspace(vp_engine* e) {
     e->sched.clear();
     e->callEv.clear();
     if (e->spPinned) { cudaFreeHost(e->spPinned); e->spPinned = nullptr; }
+    if (e->pordPinned) { cudaFreeHost(e->pordPinned); e->pordPinned = nullptr; }
     if (e->rsPinned) { cudaFreeHost(e->rsPinned); e->rsPinned = nullptr; }
-    void** ptrs[] = {(void**)&e->dSP, (void**)&e->dRsList, (void**)&e->dGate, (void**)&e->dRV, (void**)&e->dRS, (void**)&e->dAV, (void**)&e->dAS, (void**)&e->dEeV,
+    void** ptrs[] = {(void**)&e->dSP, (void**)&e->dOrdP, (void**)&e->dRsList, (void**)&e->dGate, (void**)&e->dRV, (void**)&e->dRS, (void**)&e->dAV, (void**)&e->dAS, (void**)&e->dEeV,
                      (void**)&e->dEeS, (void**)&e->dG, (void**)&e->dGs, (void**)&e->dPeriod, (void**)&e->dList, (void**)&e->dListCount,
                      (void**)&e->dYFlags, (void**)&e->dFrames, (void**)&e->dAP, (void**)&e->dOutE, (void**)&e->dOutV,
                      (void**)&e->dOutP, (void**)&e->dFramesAll, (void**)&e->dGateAll, (void**)&e->dEeVAll, (void**)&e->dEeSAll,
@@ -501,6 +512,61 @@ extern "C" int vp_engine_reserve_orders(vp_engine* e, int maxLpcVoice, int maxLp
     return VP_OK;
 }
 
+extern "C" int vp_engine_reserve_pitch_order(vp_engine* e, int maxLpcPitch) {
+    if (!e) return VP_E_ARG;
+    if (maxLpcPitch < 0 || maxLpcPitch > 100) return vp_err(e, VP_E_RANGE, "order outside the plug-in's range");
+    if (e->prepared && maxLpcPitch > e->capP && e->gs.blocksDone > 0)
+        return vp_err(e, VP_E_STATE, "vp_engine_reserve_pitch_order on a running stream: call it before vp_engine_prepare");
+    e->reserveP = maxLpcPitch;
+    if (e->prepared && maxLpcPitch > e->capP) e->prepared = false;
+    return VP_OK;
+}
+
+// after pordIn changed: the next call uploads the orders, the batch-wide flags are recomputed
+static void pitch_orders_changed(vp_engine* e) {
+    e->pordDirty = true;
+    e->pordUniform = true;
+    e->pordMax = 0;
+    for (int p : e->pordIn) {
+        e->pordUniform = e->pordUniform && p == e->pordIn[0];
+        e->pordMax = std::max(e->pordMax, p);
+    }
+}
+
+extern "C" int vp_engine_set_stream_pitch_orders(vp_engine* e, int firstStream, int count, const int* lpcPitch) {
+    if (!e) return VP_E_ARG;
+    if (!e->prepared) return vp_err(e, VP_E_STATE, "vp_engine_prepare has not been called");
+    if (firstStream < 0 || count < 0 || firstStream > e->S - count || (count > 0 && !lpcPitch))
+        return vp_err(e, VP_E_ARG, "stream range outside [0, nStreams), or NULL values");
+    for (int i = 0; i < count; ++i)
+        if (lpcPitch[i] < 2 || lpcPitch[i] > 100) return vp_err(e, VP_E_RANGE, "order outside the plug-in's range");
+    for (int i = 0; i < count; ++i)
+        if (lpcPitch[i] > e->capP)
+            return vp_err(e, VP_E_STATE, "lpcPitch beyond what vp_engine_prepare sized: vp_engine_reserve_pitch_order before vp_engine_prepare");
+    // a stream that has processed no block since its start (none since prepare / reset, or a reset of it pending) starts with
+    // the new value at the next call; any other stream keeps its order until its next start
+    const bool fresh = e->gs.blocksDone == 0;
+    bool changed = false;
+    for (int i = 0; i < count; ++i) {
+        const int s = firstStream + i;
+        e->pordNext[s] = lpcPitch[i];
+        if ((fresh || e->rsMark[s]) && e->pordIn[s] != lpcPitch[i]) { e->pordIn[s] = lpcPitch[i]; changed = true; }
+    }
+    if (changed) pitch_orders_changed(e);
+    return VP_OK;
+}
+
+extern "C" int vp_engine_get_stream_pitch_orders(const vp_engine* e, int firstStream, int count, int* inForce, int* next) {
+    if (!e) return VP_E_ARG;
+    if (!e->prepared) return VP_E_STATE;
+    if (firstStream < 0 || count < 0 || firstStream > e->S - count) return VP_E_ARG;
+    for (int i = 0; i < count; ++i) {
+        if (inForce) inForce[i] = e->pordIn[firstStream + i];
+        if (next) next[i] = e->pordNext[firstStream + i];
+    }
+    return VP_OK;
+}
+
 static VPStreamParam stream_table_entry(const vp_stream_params& p, const vp_stream_orders& o) {
     VPStreamParam q;
     memset(&q, 0, sizeof q);
@@ -574,14 +640,21 @@ static int check_orders(vp_engine* e, const vp_stream_orders* o, size_t step, in
 // The table goes up before the first kernel of a call, on the engine's stream. The staging buffer is rewritten only after
 // the previous upload has read it: a call that is still queued (vp_engine_process_device returns before it runs) keeps the
 // values it was issued with.
+// The per-stream lpcPitch values travel the same way.
 static int upload_stream_params(vp_engine* e) {
-    if (!e->spDirty) return VP_OK;
-    const size_t bytes = e->spTab.size() * sizeof(VPStreamParam);
+    if (!e->spDirty && !e->pordDirty) return VP_OK;
     VP_CUDA_OK(cudaEventSynchronize(e->evSpUp));
-    memcpy(e->spPinned, e->spTab.data(), bytes);
-    VP_CUDA_OK(cudaMemcpyAsync(e->dSP, e->spPinned, bytes, cudaMemcpyHostToDevice, e->st));
+    if (e->spDirty) {
+        const size_t bytes = e->spTab.size() * sizeof(VPStreamParam);
+        memcpy(e->spPinned, e->spTab.data(), bytes);
+        VP_CUDA_OK(cudaMemcpyAsync(e->dSP, e->spPinned, bytes, cudaMemcpyHostToDevice, e->st));
+    }
+    if (e->pordDirty) {
+        for (size_t s = 0; s < e->pordIn.size(); ++s) e->pordPinned[s] = (int16_t)e->pordIn[s];
+        VP_CUDA_OK(cudaMemcpyAsync(e->dOrdP, e->pordPinned, e->pordIn.size() * sizeof(int16_t), cudaMemcpyHostToDevice, e->st));
+    }
     VP_CUDA_OK(cudaEventRecord(e->evSpUp, e->st));
-    e->spDirty = false;
+    e->spDirty = e->pordDirty = false;
     return VP_OK;
 }
 
@@ -673,12 +746,13 @@ extern "C" int vp_engine_set_params(vp_engine* e, const vp_params* p) {
     vp_params q = *p;
     const bool running = e->prepared && e->gs.blocksDone > 0;
     // lpcPitch is read in PitchProcess::prepare only (PitchProcess.cpp:70): a change on a running stream has no effect until
-    // the next prepareToPlay, exactly as in the reference
-    if (running) q.lpcPitch = e->capP;
+    // the next prepareToPlay, exactly as in the reference. It is the engine-wide value every stream gets at vp_engine_prepare;
+    // the per-stream values (vp_engine_set_stream_pitch_orders) are never overwritten here.
+    if (running) q.lpcPitch = e->prm.lpcPitch;
     // The workspace rows are sized for capV / capS (the orders at vp_engine_prepare, or vp_engine_reserve_orders). On a running
     // stream an order within that range takes effect at the next vocoder frame (VocoderProcess.cpp:193-194); beyond it the
     // reference would run past its orderMax vectors (its assert at :141-147) and the engine refuses.
-    if (e->prepared && (q.lpcVoice > e->capV || q.lpcSynth > e->capS || q.lpcPitch != e->capP)) {
+    if (e->prepared && (q.lpcVoice > e->capV || q.lpcSynth > e->capS || q.lpcPitch != e->prm.lpcPitch)) {
         if (running)
             return vp_err(e, VP_E_STATE, "lpcVoice / lpcSynth beyond what vp_engine_prepare sized: vp_engine_reserve_orders before "
                                          "vp_engine_prepare, or vp_engine_reset, set the parameters, vp_engine_prepare");
@@ -748,7 +822,8 @@ static VPResetSegs carried_state(vp_engine* e) {
 static_assert((VP_PC * sizeof(vp_pitch_frame)) % 16 == 0 && offsetof(VPMarkState, beta) % sizeof(double) == 0,
               "carried records are whole 16-byte units");
 
-// prepareToPlay state for every stream; pending per-stream resets are dropped (they are part of it)
+// prepareToPlay state for every stream; pending per-stream resets are dropped (they are part of it); every stream starts
+// with its set lpcPitch
 static int reset_state(vp_engine* e) {
     e->histCur = 0;  // (the other history buffer is written in full by the next call before it is read)
     vp_launch_reset_streams(e->st, carried_state(e), nullptr, e->S);
@@ -756,6 +831,7 @@ static int reset_state(vp_engine* e) {
     VP_CUDA_OK(cudaStreamSynchronize(e->st));
     for (int s : e->rsList) e->rsMark[s] = 0;
     e->rsList.clear();
+    if (e->pordIn != e->pordNext) { e->pordIn = e->pordNext; pitch_orders_changed(e); }
     e->sched.clear();
     e->pgCarryAny = true;
     e->gs.B = e->B; e->gs.z = e->sz;
@@ -779,8 +855,14 @@ extern "C" int vp_engine_reset_streams(vp_engine* e, const int* streams, int cou
     if (count < 0 || (count > 0 && !streams)) return vp_err(e, VP_E_ARG, "streams must be non-null and count >= 0");
     for (int i = 0; i < count; ++i)
         if (streams[i] < 0 || streams[i] >= e->S) return vp_err(e, VP_E_ARG, "stream index outside [0, nStreams)");
-    for (int i = 0; i < count; ++i)
-        if (!e->rsMark[streams[i]]) { e->rsMark[streams[i]] = 1; e->rsList.push_back(streams[i]); }
+    bool ordChanged = false;
+    for (int i = 0; i < count; ++i) {
+        const int s = streams[i];
+        if (!e->rsMark[s]) { e->rsMark[s] = 1; e->rsList.push_back(s); }
+        // the stream starts at the next call: with its set lpcPitch (PitchProcess::prepare)
+        if (e->pordIn[s] != e->pordNext[s]) { e->pordIn[s] = e->pordNext[s]; ordChanged = true; }
+    }
+    if (ordChanged) pitch_orders_changed(e);
     // the new user of a slot does not inherit the old user's automation
     if (!e->sched.empty() && count > 0) {
         std::vector<uint8_t> listed((size_t)e->S, 0);
@@ -946,7 +1028,8 @@ extern "C" int vp_engine_prepare(vp_engine* e, double fs, int B, int S, int maxB
     int nV, nP;
     frame_counts(z, n, &nV, &nP);
     nV += 1; nP += 1;  // a frame grid that a vocBool / pitchBool-off stretch has shifted can put one more frame into a call
-    const int capV = std::max(std::max(e->prm.lpcVoice, e->reserveV), 40), capS = std::max(std::max(e->prm.lpcSynth, e->reserveS), 5), capP = e->prm.lpcPitch;
+    const int capV = std::max(std::max(e->prm.lpcVoice, e->reserveV), 40), capS = std::max(std::max(e->prm.lpcSynth, e->reserveS), 5);
+    const int capP = std::max(e->prm.lpcPitch, e->reserveP);
     {
         const char* ym = getenv("VP_YIN_MODE");
         e->yinDirect = (ym && strcmp(ym, "direct") == 0) ? 1 : 0;
@@ -1045,6 +1128,13 @@ extern "C" int vp_engine_prepare(vp_engine* e, double fs, int B, int S, int maxB
     e->sord.assign((size_t)S, order_part(e->prm));
     e->spTab.assign((size_t)S, stream_table_entry(e->sprm[0], e->sord[0]));
     stream_table_changed(e);
+    // every stream starts with the engine's lpcPitch; dOrdP is read only once the orders differ, and any change uploads it whole
+    if ((rc = wsalloc(e, &e->dOrdP, (size_t)S))) return rc;
+    VP_CUDA_OK(cudaHostAlloc((void**)&e->pordPinned, (size_t)S * sizeof(int16_t), cudaHostAllocDefault));
+    e->pordIn.assign((size_t)S, e->prm.lpcPitch);
+    e->pordNext = e->pordIn;
+    pitch_orders_changed(e);
+    e->pordDirty = false;
     e->capV = capV; e->capS = capS; e->capP = capP;
     if ((rc = reset_state(e))) return rc;
     e->launches = e->yinRechecked = e->yinFrames = 0;
@@ -1095,8 +1185,12 @@ static int make_geom(vp_engine* e, int nBlocks, size_t stride, VPGeom* g) {
     g->wstride = (long long)e->maxBlocks * e->B;
     g->vstride = g->pstride = g->wstride;
     g->vocOn = e->prm.vocBool != 0; g->pitchOn = e->prm.pitchBool != 0;
-    g->ordV = e->callOrdV; g->ordS = e->callOrdS; g->ordP = e->capP;  // (plan_schedule: the streams' orders in this call)
+    g->ordV = e->callOrdV; g->ordS = e->callOrdS;  // (plan_schedule: the streams' orders in this call)
     g->ordTab = e->callOrdTab;
+    // pitch: every stream at one order -- exactly the kernels of an engine prepared with it; else rows as wide as the widest
+    // order, at least 16 doubles when the workspace holds them (the P = 15 residual path then serves every order <= 15)
+    g->ordTabP = !e->pordUniform;
+    g->ordP = e->pordUniform ? e->pordIn[0] : std::max(e->pordMax, std::min(15, e->capP));
     g->H = e->H;
     g->defined = e->mode == VP_MODE_DEFINED;
     grid_geom(e->gs, g);
@@ -1136,7 +1230,7 @@ static void pass_init(vp_engine* e, PassCtx& c, const VPGeom& gIO, int Sp, int s
                       const float* synthR, float* outL, float* outR) {
     c.g = gIO;
     c.tb = VPTables{e->dWV, e->dWS ? e->dWS : e->dWV, e->dStP, e->dHann, e->dHannOff, e->dLutBeta, e->dLutPeriodNew, e->dLutNote,
-                    e->callSP + streamBase, e->callStride};
+                    e->callSP + streamBase, e->callStride, e->dOrdP + streamBase};
     c.Sp = Sp;
     c.sb = (size_t)streamBase;
     const int hc = e->histCur;
@@ -1267,7 +1361,7 @@ static int pass_P(vp_engine* e, PassCtx& c) {
         stage_mark(e, ST_OTHER);  // whatever of the mark chain was not hidden under the vocoder kernels
     }
     if (g.pitchMix) {
-        vp_launch_pitch_lpc(st, g, Sp, c.voice, e->dFrames, e->dRP, e->dAP);
+        vp_launch_pitch_lpc(st, g, c.tb, Sp, c.voice, e->dFrames, e->dRP, e->dAP);
         stage_mark(e, ST_PLPC);
         vp_launch_pitch_psola(st, g, c.tb, Sp, c.voice, e->dFrames, e->dAP, e->dOutE);
         stage_mark(e, ST_PFRAME);
@@ -1835,9 +1929,10 @@ extern "C" int vp_engine_stream_block(vp_engine* e) {
     e->lastBlocks = 1;
     e->lastG = g;
     // everything that shapes the launch sequence or is baked into kernel arguments
-    // (per-stream orders are table data; whether they differ, and the row orders, select the kernels)
+    // (per-stream orders are table data; whether they differ, and the row orders, select the kernels -- the pitch orders as
+    // well: a reset that gives a stream a new lpcPitch changes at most that signature)
     std::vector<long long> key = {e->gs.blocksDone > 0 ? 1 : 0, e->histCur, g.offV, g.offP, g.nFramesV, g.nFramesP, g.kV0, g.synV, g.synS,
-                                  g.vocOn, g.pitchOn, g.vocMix, g.pitchMix, e->callAnyDry, g.ordV, g.ordS, g.ordTab};
+                                  g.vocOn, g.pitchOn, g.vocMix, g.pitchMix, e->callAnyDry, g.ordV, g.ordS, g.ordTab, g.ordP, g.ordTabP};
     for (int j = 0; j < VP_ORPH; ++j) { key.push_back(g.orphPos[j]); key.push_back(g.orphOrdV[j]); key.push_back(g.orphOrdS[j]); }
     for (int j = 0; j < VP_PC; ++j) { key.push_back(g.carryPosP[j]); key.push_back(g.carryLimP[j]); }
     auto it = e->graphs.find(key);

@@ -142,6 +142,18 @@ public:
     // vectors for the ends of the parameter ranges: 100 / 30)
     void setWindow(bool hann) { engine.check(vp_engine_set_window(engine.h, hann ? VP_WINDOW_HANN : VP_WINDOW_SINE)); }
     void reserveOrders(int maxLpcVoice, int maxLpcSynth) { engine.check(vp_engine_reserve_orders(engine.h, maxLpcVoice, maxLpcSynth)); }
+    // largest per-stream lpcPitch (before prepare; 0 = params.lpcPitch)
+    void reservePitchOrder(int maxLpcPitch) { engine.check(vp_engine_reserve_pitch_order(engine.h, maxLpcPitch)); }
+    // lpcPitch of streams first .. first + count - 1 (after prepare): read when a stream starts (PitchProcess.cpp:70) -- at
+    // once for a stream that has processed nothing since prepare / restart / its restartStreams, else at its next start.
+    // setParams does not touch it (nothing to push again per block)
+    void setStreamPitchOrders(int first, int count, const int* lpcPitch) {
+        engine.check(vp_engine_set_stream_pitch_orders(engine.h, first, count, lpcPitch));
+    }
+    // the order each stream runs its next block at / takes at its next start (either pointer may be null)
+    void getStreamPitchOrders(int first, int count, int* inForce, int* next) const {
+        engine.check(vp_engine_get_stream_pitch_orders(engine.h, first, count, inForce, next));
+    }
     // prepareToPlay on a running instance: back to the freshly prepared state first
     void restart() { if (B > 0) engine.check(vp_engine_reset(engine.h)); }
     // prepareToPlay for some instances of the running batch (a slot handed to a new user): from the next block on, each
@@ -253,9 +265,10 @@ class VocoderBatchProcessor {
 public:
     explicit VocoderBatchProcessor(int device = 0) : myBuffer(device) { vp_default_params(&params); }
 
-    // maxLpcVoice / maxLpcSynth: the largest orders the parameters may take while the streams run (0 = the current ones)
+    // maxLpcVoice / maxLpcSynth: the largest orders the parameters may take while the streams run (0 = the current ones);
+    // maxLpcPitch: the largest per-stream lpcPitch (myBuffer.setStreamPitchOrders; 0 = params.lpcPitch)
     void prepareToPlay(double sampleRate, int samplesPerBlock, int nStreams, int maxBlocksPerCall = 1, int maxLpcVoice = 0,
-                       int maxLpcSynth = 0) {
+                       int maxLpcSynth = 0, int maxLpcPitch = 0) {
         const double ratioSR = sampleRate / 44100.0;                       // :160
         const int hopVoc = (int)std::floor(128.0 * ratioSR);               // :163
         const int wlenVoc = 4 * hopVoc;                                    // :164
@@ -264,6 +277,7 @@ public:
         const double silenceDb = -60.0;                                    // :148
         myBuffer.restart();
         myBuffer.reserveOrders(maxLpcVoice, maxLpcSynth);
+        myBuffer.reservePitchOrder(maxLpcPitch);
         myBuffer.setParams(params);
         pitchProcess.prepare(sampleRate, 100.0, 800.0, frameLenPitch, hopPitch, samplesPerBlock, silenceDb);   // :172
         vocoderProcess.prepare(wlenVoc, hopVoc, windowType, silenceDb);                                         // :173

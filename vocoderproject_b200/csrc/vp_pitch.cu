@@ -1234,19 +1234,21 @@ __global__ void __launch_bounds__(32 * PA_WARPS) k_pitch_autocorr(VPGeom g, cons
     }
 }
 
+// P > 0: every frame has order P; P == 0: order g.ordP, or with g.ordTabP each frame its stream's own order (rows stay
+// g.ordP + 1 wide, the taps beyond the frame's order are written as zeros). Both forms run the same FMA sequence and
+// vp_div_const is the correctly rounded x / L, so a frame solved here at order 15 has the bits of k_pitch_levinson<15>.
 template <int P>
-__global__ void __launch_bounds__(128) k_pitch_levinson(VPGeom g, const vp_pitch_frame* __restrict__ frames,
+__global__ void __launch_bounds__(128) k_pitch_levinson(VPGeom g, const int16_t* __restrict__ ordTab, const vp_pitch_frame* __restrict__ frames,
                                                         const double* __restrict__ rP, double* __restrict__ aP, long long nFramesTot) {
     const long long fidx = (long long)blockIdx.x * blockDim.x + threadIdx.x;  // slot index over [S][nFramesP + VP_PC]
     if (fidx >= nFramesTot) return;
-    {
-        const int s = (int)(fidx / (g.nFramesP + VP_PC)), f = (int)(fidx - (long long)s * (g.nFramesP + VP_PC)) - VP_PC;
-        if (!pf_live(g, frames + fidx, f)) return;
-    }
+    const int s = (int)(fidx / (g.nFramesP + VP_PC)), f = (int)(fidx - (long long)s * (g.nFramesP + VP_PC)) - VP_PC;
+    if (!pf_live(g, frames + fidx, f)) return;
     constexpr int PM = (P > 0) ? P : VP_ORDER_MAX;
-    const int ord = (P > 0) ? P : g.ordP;
+    const int row = (P > 0) ? P : g.ordP;
+    const int ord = (P > 0) ? P : (g.ordTabP ? (int)ordTab[s] : g.ordP);
     double r[PM + 1], a[PM + 1];
-    const double* rp = rP + (size_t)fidx * (size_t)(ord + 1);
+    const double* rp = rP + (size_t)fidx * (size_t)(row + 1);
     if (P > 0) {
 #pragma unroll
         for (int m = 0; m <= PM; ++m) r[m] = vp_div_const(rp[m], (double)g.L, 1.0 / (double)g.L);
@@ -1296,12 +1298,13 @@ __global__ void __launch_bounds__(128) k_pitch_levinson(VPGeom g, const vp_pitch
             for (int i = 1; i <= ord; ++i) a[i] = -a[i];
         }
     }
-    double* ap = aP + (size_t)fidx * (size_t)(ord + 1);
+    double* ap = aP + (size_t)fidx * (size_t)(row + 1);
     if (P > 0) {
 #pragma unroll
         for (int i = 0; i <= PM; ++i) ap[i] = a[i];
     } else {
         for (int i = 0; i <= ord; ++i) ap[i] = a[i];
+        for (int i = ord + 1; i <= row; ++i) ap[i] = 0.0;
     }
 }
 
@@ -1528,8 +1531,12 @@ __global__ void __launch_bounds__(PF_THREADS, 7) k_pitch_psola(VPGeom g, VPTable
     if (ub && tid == 0) rec->flags = flags | VP_PF_UB;
 }
 
-void vp_launch_pitch_lpc(cudaStream_t st, const VPGeom& g, int S, const float* voice, const vp_pitch_frame* frames,
-                         double* rP, double* aP) {
+// Rows of g.ordP + 1: with g.ordTabP the widest order of the call (at least 15 when the rows can hold it), and each frame
+// solved at its own. The autocorrelation's lag sums do not depend on how many lags are computed (the segmentation depends on
+// L only), and the residual in k_pitch_psola sums taps 0 .. g.ordP in ascending order, where a zero tap leaves the sum as it
+// is: both run unchanged on padded rows, and a row of order <= 15 padded to 16 keeps the P = 15 register path.
+void vp_launch_pitch_lpc(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const float* voice,
+                         const vp_pitch_frame* frames, double* rP, double* aP) {
     const long long tot = (long long)S * (g.nFramesP + VP_PC);
     int segLen = (g.L + PA_SEGS - 1) / PA_SEGS;
     if ((segLen & 1) == 0) ++segLen;  // odd -> the 16 segments of a half-warp hit 16 distinct 64-bit banks
@@ -1538,8 +1545,8 @@ void vp_launch_pitch_lpc(cudaStream_t st, const VPGeom& g, int S, const float* v
     const size_t smem = (size_t)PA_WARPS * xdLen * sizeof(double);
     cudaFuncSetAttribute(k_pitch_autocorr, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     VP_LAUNCH(k_pitch_autocorr<<<(unsigned)((tot + PA_WARPS - 1) / PA_WARPS), 32 * PA_WARPS, smem, st>>>(g, voice, frames, rP, segLen, xdLen, tot));
-    if (g.ordP == 15) VP_LAUNCH(k_pitch_levinson<15><<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(g, frames, rP, aP, tot));
-    else VP_LAUNCH(k_pitch_levinson<0><<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(g, frames, rP, aP, tot));
+    if (g.ordP == 15 && !g.ordTabP) VP_LAUNCH(k_pitch_levinson<15><<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(g, tb.ordP, frames, rP, aP, tot));
+    else VP_LAUNCH(k_pitch_levinson<0><<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(g, tb.ordP, frames, rP, aP, tot));
 }
 
 void vp_launch_pitch_psola(cudaStream_t st, const VPGeom& g, const VPTables& tb, int S, const float* voice,
@@ -1579,6 +1586,10 @@ void vp_launch_pitch_psola(cudaStream_t st, const VPGeom& g, const VPTables& tb,
 // as gpCall. Measured on the default workload (same-box A/B against the form that always reads the table): the table form
 // took this kernel from 18.9 to 19.8 ms per step, the argument form is at 18.9 again.
 // Both forms store the gains of the chunks of the frames the next call carries (pgOut, the last VP_PC of carried ++ new).
+// P = 15: transposed direct form II in registers; P = 0: direct form with a circular history at order g.ordP. The two round
+// differently, so a call whose streams have different orders (g.ordTabP) runs P = -1: each frame takes the form and the order
+// a call at its stream's order alone would run -- the transposed form (its own 16 registers) at 15, else the direct form.
+// Frames of different forms share a warp only where a stream boundary falls inside its 32 slots.
 template <int P, bool STREAM_GAIN>
 __global__ void __launch_bounds__(32 * PI_WARPS, 8) k_pitch_iir(VPGeom g, VPTables tb, const vp_pitch_frame* __restrict__ frames,
                                                              const double* __restrict__ aP, const float* __restrict__ outE,
@@ -1596,7 +1607,8 @@ __global__ void __launch_bounds__(32 * PI_WARPS, 8) k_pitch_iir(VPGeom g, VPTabl
     if (f0 >= nFramesTot) return;
     const long long fidx = f0 + lane;
     const int L = g.L, c = g.c;
-    const int order = (P > 0) ? P : g.ordP;
+    const int row = (P > 0) ? P : g.ordP;  // row width - 1
+    int order = row;
     bool active = false;
     int s = 0, f = 0, nSteps = 0;
     if (fidx < nFramesTot) {  // slot index over [S][nFramesP + VP_PC]
@@ -1606,14 +1618,25 @@ __global__ void __launch_bounds__(32 * PI_WARPS, 8) k_pitch_iir(VPGeom g, VPTabl
         const long long p = vp_ppos(g, f);
         const int lim = vp_plim(g, f);
         for (int n = 0; n < lim; ++n) if (p + (long long)n * c < g.n) nSteps += c;  // chunks handled up to the end of this call
+        if (P < 0) order = tb.ordP[s];
     }
     if (!active) nSteps = 0;
     constexpr int PA = (P > 0) ? P : VP_ORDER_MAX;
-    double a[PA + 1], h[PA + 1];  // P > 0: h[k] = transposed-form state s_{k+1} (h[PA] stays 0); P == 0: circular output history
+    double a[PA + 1], h[PA + 1];  // P > 0: h[k] = transposed-form state s_{k+1} (h[PA] stays 0); else circular output history
+    constexpr int PT = (P < 0) ? 15 : 0;
+    double at[PT + 1], ht[PT + 1];  // P < 0: coefficients and state of a transposed-form frame (ht[PT] stays 0)
+    const bool tdf = P < 0 && order == 15;
     for (int k = 0; k <= PA; ++k) { a[k] = 0.0; h[k] = 0.0; }
+#pragma unroll
+    for (int k = 0; k <= PT; ++k) { at[k] = 0.0; ht[k] = 0.0; }
     if (active) {
-        const double* ap = aP + (size_t)fidx * (order + 1);
-        for (int k = 0; k <= order; ++k) a[k] = ap[k];
+        const double* ap = aP + (size_t)fidx * (row + 1);
+        if (tdf) {
+#pragma unroll
+            for (int k = 0; k <= PT; ++k) at[k] = ap[k];
+        } else {
+            for (int k = 0; k <= order; ++k) a[k] = ap[k];
+        }
     }
     // frame-relative output range that lands inside this call (positions before 0 went out with an earlier call, beyond n go
     // out with a later one) and the frame's offset in the output plane relative to the warp's first stream: lane fr's values
@@ -1708,6 +1731,10 @@ __global__ void __launch_bounds__(32 * PI_WARPS, 8) k_pitch_iir(VPGeom g, VPTabl
                     acc += h[0];
 #pragma unroll
                     for (int k = 0; k < PA; ++k) h[k] = fma(-a[k + 1], acc, h[k + 1]);
+                } else if (tdf) {  // (the same DFMAs as P = 15)
+                    acc += ht[0];
+#pragma unroll
+                    for (int k = 0; k < PT; ++k) ht[k] = fma(-at[k + 1], acc, ht[k + 1]);
                 } else {
                     for (int k = 1; k <= order && k <= i; ++k) acc = fma(-a[k], h[(i - k) % order], acc);
                     h[i % order] = acc;
@@ -1753,7 +1780,10 @@ void vp_launch_pitch_iir(cudaStream_t st, const VPGeom& g, const VPTables& tb, i
         return;
     }
     const double gp = gainUniform ? (double)*gainUniform : 0.0;
-    if (g.ordP == 15) {
+    if (g.ordTabP) {
+        if (gainUniform) VP_LAUNCH(k_pitch_iir<-1, false><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot, gp, pgIn, pgOut));
+        else VP_LAUNCH(k_pitch_iir<-1, true><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot, gp, pgIn, pgOut));
+    } else if (g.ordP == 15) {
         if (gainUniform) VP_LAUNCH(k_pitch_iir<15, false><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot, gp, pgIn, pgOut));
         else VP_LAUNCH(k_pitch_iir<15, true><<<grid, 32 * PI_WARPS, 0, st>>>(g, tb, frames, aP, outE, outP, tot, gp, pgIn, pgOut));
     } else {

@@ -2,11 +2,12 @@
 // instance = one stream,
 //
 //     voice.wav  sidechain.wav  out.wav  [key=N] [gainVoc=dB] [gainPitch=dB] [gainVoice=dB] [gainSynth=dB]
-//                                        [lpcVoice=N] [lpcSynth=N]
+//                                        [lpcVoice=N] [lpcSynth=N] [lpcPitch=N]
 //
 // (voice: channel 0 is used, PluginProcessor.cpp:153-157 mono main bus; side-chain: stereo, a mono file feeds both
-// channels). The optional tokens are that instance's own key, gains and vocoder orders: they override the command-line
-// values for the job, so files in different keys, with different mixes or timbres still run as one batch. All jobs run as ONE batch on the GPU through the facade's prepareToPlay / processBlock (vp_facade.hpp):
+// channels). The optional tokens are that instance's own key, gains, vocoder orders and pitch-corrector order: they
+// override the command-line values for the job, so files in different keys, with different mixes or timbres still run as
+// one batch. All jobs run as ONE batch on the GPU through the facade's prepareToPlay / processBlock (vp_facade.hpp):
 // same sample rate for all files, shorter jobs are zero-padded to the longest and trimmed again on output.
 //
 //   vp_wavbatch manifest.txt [--block 1024] [--blocks-per-call 64] [--key 12] [--voc 0|1] [--pitch 0|1]
@@ -28,11 +29,12 @@
 #include "vp_facade.hpp"
 #include "vp_wav.hpp"
 
-struct Job { std::string voice, synth, out; vpb200::WavData v, s; vp_stream_params sp; vp_stream_orders so; };
+struct Job { std::string voice, synth, out; vpb200::WavData v, s; vp_stream_params sp; vp_stream_orders so; int lpcPitch; };
 
 // "name=value" tokens of a manifest line -> the job's per-instance parameters; false when any token is not one of them.
-// any / anyOrd: some token set a key or gain / an order
-static bool parse_stream_tokens(std::istringstream& ls, vp_stream_params& sp, vp_stream_orders& so, bool& any, bool& anyOrd) {
+// any / anyOrd / anyPitch: some token set a key or gain / a vocoder order / lpcPitch
+static bool parse_stream_tokens(std::istringstream& ls, vp_stream_params& sp, vp_stream_orders& so, int& lpcPitch, bool& any,
+                                bool& anyOrd, bool& anyPitch) {
     std::string tok;
     while (ls >> tok) {
         const size_t eq = tok.find('=');
@@ -48,6 +50,11 @@ static bool parse_stream_tokens(std::istringstream& ls, vp_stream_params& sp, vp
             if (x != (double)(int)x) return false;
             (name == "lpcVoice" ? so.lpcVoice : so.lpcSynth) = (int)x;
             anyOrd = true;
+            continue;
+        } else if (name == "lpcPitch") {
+            if (x != (double)(int)x) return false;
+            lpcPitch = (int)x;
+            anyPitch = true;
             continue;
         } else if (name == "gainVoc") sp.gainVoc = (float)x;
         else if (name == "gainPitch") sp.gainPitch = (float)x;
@@ -83,8 +90,9 @@ int main(int argc, char** argv) {
             printf("usage: vp_wavbatch manifest.txt [--block B] [--blocks-per-call K] [--key 0..12] [--voc 0|1] [--pitch 0|1] "
                    "[--gain-voice dB] [--gain-synth dB] [--gain-voc dB] [--gain-pitch dB] [--pcm16] [--keep-latency] [--device d]\n"
                    "manifest lines: voice.wav sidechain.wav out.wav [key=N] [gainVoc=dB] [gainPitch=dB] [gainVoice=dB] [gainSynth=dB] "
-                   "[lpcVoice=N] [lpcSynth=N]\n"
-                   "  (the tokens set that job's key, gains and vocoder orders; they override --key / --gain-* for the job)\n");
+                   "[lpcVoice=N] [lpcSynth=N] [lpcPitch=N]\n"
+                   "  (the tokens set that job's key, gains, vocoder orders and pitch-corrector order; they override --key / --gain-* "
+                   "for the job)\n");
             return 0;
         } else if (argv[i][0] != '-' && manifest.empty()) manifest = argv[i];
         else { fprintf(stderr, "unknown argument %s\n", argv[i]); return 2; }
@@ -92,7 +100,7 @@ int main(int argc, char** argv) {
     if (manifest.empty() || B <= 0 || K <= 0) { fprintf(stderr, "vp_wavbatch: no manifest (see --help)\n"); return 2; }
     try {
         std::vector<Job> jobs;
-        bool perJob = false, perJobOrd = false;  // some line sets its own key or gains / its own orders
+        bool perJob = false, perJobOrd = false, perJobPitch = false;  // some line sets its own key or gains / orders / lpcPitch
         {
             std::ifstream mf(manifest);
             if (!mf) throw std::runtime_error("cannot open " + manifest);
@@ -105,10 +113,10 @@ int main(int argc, char** argv) {
                 if (!(ls >> j.synth >> j.out)) throw std::runtime_error("manifest line needs three paths: " + line);
                 j.sp.gainPitch = prm.gainPitch; j.sp.gainVoice = prm.gainVoice; j.sp.gainSynth = prm.gainSynth;
                 j.sp.gainVoc = prm.gainVoc; j.sp.keyPitch = prm.keyPitch;
-                j.so.lpcVoice = prm.lpcVoice; j.so.lpcSynth = prm.lpcSynth;
-                if (!parse_stream_tokens(ls, j.sp, j.so, perJob, perJobOrd))
+                j.so.lpcVoice = prm.lpcVoice; j.so.lpcSynth = prm.lpcSynth; j.lpcPitch = prm.lpcPitch;
+                if (!parse_stream_tokens(ls, j.sp, j.so, j.lpcPitch, perJob, perJobOrd, perJobPitch))
                     throw std::runtime_error("manifest tokens after the paths are key=N gainVoc= gainPitch= gainVoice= gainSynth= "
-                                             "lpcVoice=N lpcSynth=N: " + line);
+                                             "lpcVoice=N lpcSynth=N lpcPitch=N: " + line);
                 jobs.push_back(std::move(j));
             }
         }
@@ -126,9 +134,16 @@ int main(int argc, char** argv) {
         const int S = (int)jobs.size();
         vpb200::VocoderBatchProcessor proc(device);
         proc.params = prm;
-        int maxV = 0, maxS = 0;  // the workspace rows are sized for the largest order of the manifest
-        for (const Job& j : jobs) { maxV = std::max(maxV, j.so.lpcVoice); maxS = std::max(maxS, j.so.lpcSynth); }
-        proc.prepareToPlay((double)fs, B, S, K, maxV, maxS);
+        int maxV = 0, maxS = 0, maxP = 0;  // the workspace rows are sized for the largest orders of the manifest
+        for (const Job& j : jobs) {
+            maxV = std::max(maxV, j.so.lpcVoice); maxS = std::max(maxS, j.so.lpcSynth); maxP = std::max(maxP, j.lpcPitch);
+        }
+        proc.prepareToPlay((double)fs, B, S, K, maxV, maxS, maxP);
+        if (perJobPitch) {  // read when a stream starts: set before the first block, each job starts with its own
+            std::vector<int> lp;
+            for (const Job& j : jobs) lp.push_back(j.lpcPitch);
+            proc.myBuffer.setStreamPitchOrders(0, S, lp.data());
+        }
         if (perJob)
             for (const Job& j : jobs) proc.streamParams.push_back(j.sp);
         if (perJobOrd)
