@@ -304,6 +304,61 @@ int vp_engine_reset(vp_engine* e);
  * their widest (one capture). Cost: one kernel launch in the next call, none when no reset is pending. */
 int vp_engine_reset_streams(vp_engine* e, const int* streams, int count);
 
+/* ---- per-stream state snapshots: move a running stream to another slot or engine, checkpoint a render ----------------
+ * A snapshot holds what a stream carries from one process call to the next (input histories, gate sums, carried and
+ * orphan vocoder rows, energy histories, the last two pitch records, the mark state, the carried chunk gains), its
+ * vp_stream_params and vp_stream_orders in force and its lpcPitch in force and next. Scheduled events are not state and are
+ * not saved.
+ *
+ * Format (opaque to callers, versioned, self-checking): one header of VP_SNAPSHOT_HEADER_BYTES, then `count` records of
+ * VP_SNAPSHOT_RECORD_BYTES + 16 x unitsPerStream bytes each. The header holds a magic ("VPSS"), the format version
+ * (VP_SNAPSHOT_VERSION), a checksum, the layout key -- sample rate, samplesPerBlock, history length H, gate-carry rows,
+ * the reserved row widths (capV / capS / capP), the window and the 16-byte units of each carried segment -- the record
+ * count and the source's frame grids. A record is a fixed part (checksum, the stream's params, orders, lpcPitch in force /
+ * next, the own order of each carried and orphan vocoder row = its last non-zero coefficient) followed by the raw state.
+ * Checksums are FNV-1a 64 over little-endian 64-bit words with the checksum field zero (header: over the header; record:
+ * over the fixed part, then the raw state).
+ *
+ * Compatibility. A record loads only into an engine with the same layout key (VP_E_STATE otherwise) and the same GRID
+ * PHASE: the frame grids with every position taken relative to blocksDone x samplesPerBlock (next vocoder frame, live
+ * orphan frames, next pitch chunk and its nChunk, carried pitch frames and their processed chunks, carried vocoder
+ * frames on the grid). Engines that ran the same block sequence with the same vocBool / pitchBool switches have the same
+ * phase -- the shards of one streaming host, also when their blocksDone differ by a whole grid period -- and any move
+ * within one engine does. VP_E_STATE on a phase mismatch. Exception: an engine that has processed no block since
+ * vp_engine_prepare / vp_engine_reset ADOPTS the snapshot's grids, block count included (checkpoint / resume, and
+ * resizing a batch: save the live streams, prepare an engine with another nStreams or workspace, load); its slots that are
+ * not loaded then hold the state of silence since prepare (what vp_engine_reset_streams gives). The mode
+ * (vp_engine_set_mode) is not part of the key.
+ *
+ * Cost: one gather / scatter kernel over (listed stream x 16-byte unit) plus the copy over the host link (about 43 KB
+ * per stream at 48 kHz); pinned and device staging buffers are allocated at the first save / load that needs them,
+ * outside the workspace budget (VP_E_NOMEM before anything is issued when they cannot be had). */
+#define VP_SNAPSHOT_VERSION 1
+#define VP_SNAPSHOT_HEADER_BYTES 352
+#define VP_SNAPSHOT_RECORD_BYTES 144  /* fixed part of a record; the raw state follows */
+/* *bytes = the size of a snapshot of `count` streams for the engine as prepared. VP_E_ARG for e or bytes NULL or
+ * count < 0, VP_E_STATE before vp_engine_prepare. */
+int vp_engine_snapshot_size(const vp_engine* e, int count, size_t* bytes);
+/* The state streams[0 .. count) start their next process call with -> buf (any host memory, at least
+ * vp_engine_snapshot_size bytes). Waits for every call already issued (the mark chain on the side stream included), then
+ * gathers and copies. A stream with a reset pending (vp_engine_reset_streams) is saved as the silent state that reset
+ * gives. Changes nothing in the engine. VP_E_STATE before vp_engine_prepare or after a process call that failed half way;
+ * VP_E_ARG for count < 0, a NULL list or buffer, an index outside [0, nStreams) or a buffer that is too small. */
+int vp_engine_save_streams(vp_engine* e, const int* streams, int count, void* buf, size_t bytes);
+/* Record i of buf becomes the state of slot streams[i]; count must be the snapshot's record count. Everything is
+ * validated on the host before anything is issued: magic, version and checksums (VP_E_ARG), the layout key and grid phase
+ * (VP_E_STATE), the records' params / orders / lpcPitch (VP_E_RANGE outside the plug-in's ranges, VP_E_STATE above the
+ * reservation), and every integer of the raw state a kernel uses as a bound or an index -- mark counts, periods
+ * (VP_E_RANGE); a buffer shorter than the snapshot, a NULL list, an index outside [0, nStreams) or a slot listed twice is
+ * VP_E_ARG. On any error nothing changes. The load is then issued on the engine's stream behind every call already
+ * issued (one upload through a pinned staging buffer, one scatter kernel) and returns once buf has been read, without
+ * waiting for the GPU otherwise. Each loaded slot takes the record's params, orders and lpcPitch (in force and next: a load
+ * is a start of that slot), and drops its pending reset and its pending scheduled events; a reset or an event requested
+ * after the load applies on top of it. The engine's row widths grow to cover the loaded rows' own orders, so a stream
+ * with low orders keeps a uniform batch on its tuned kernels. Streaming needs no new graph capture for a load unless it
+ * changes what selects the captured kernels (whether orders differ and the widest, row widths, some stream's dry path). */
+int vp_engine_load_streams(vp_engine* e, const int* streams, int count, const void* buf, size_t bytes);
+
 /* Host-only helper (no CUDA): the frame grids a sequence of process calls produces -- call c processes nBlocks[c] blocks
  * with params[c] in force (only vocBool, pitchBool, lpcVoice, lpcSynth matter). For hosts that want to know how many frame
  * records a call will report, and for the CPU tests of the grid bookkeeping. The orders are the engine-wide ones: the plan

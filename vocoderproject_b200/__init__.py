@@ -18,6 +18,7 @@ VP_MAX_MARKS = 24
 VP_MODE_PARITY, VP_MODE_DEFINED = 0, 1
 VP_WINDOW_SINE, VP_WINDOW_HANN = 0, 1
 VP_NSTAGES = 16
+VP_SNAPSHOT_VERSION, VP_SNAPSHOT_HEADER_BYTES, VP_SNAPSHOT_RECORD_BYTES = 1, 352, 144
 PF_GATED, PF_VOICED, PF_HAS_MARKS = 1, 2, 4
 PF_NEAR_GATE, PF_NEAR_YIN, PF_UB, PF_YIN_RECHECKED = 16, 32, 64, 128
 
@@ -34,6 +35,7 @@ ABI_SYMBOLS = [
     "vp_engine_set_stream_params", "vp_engine_get_stream_params", "vp_engine_reset_streams", "vp_engine_schedule_stream_params",
     "vp_engine_set_stream_orders", "vp_engine_get_stream_orders", "vp_engine_schedule_stream_orders",
     "vp_engine_reserve_pitch_order", "vp_engine_set_stream_pitch_orders", "vp_engine_get_stream_pitch_orders",
+    "vp_engine_snapshot_size", "vp_engine_save_streams", "vp_engine_load_streams",
 ]
 
 
@@ -173,6 +175,9 @@ def load_library(path=None):
         "vp_engine_reserve_pitch_order": (i, [vp, i]),
         "vp_engine_set_stream_pitch_orders": (i, [vp, i, i, C.POINTER(i)]),
         "vp_engine_get_stream_pitch_orders": (i, [vp, i, i, C.POINTER(i), C.POINTER(i)]),
+        "vp_engine_snapshot_size": (i, [vp, i, C.POINTER(sz)]),
+        "vp_engine_save_streams": (i, [vp, C.POINTER(i), i, C.c_void_p, sz]),
+        "vp_engine_load_streams": (i, [vp, C.POINTER(i), i, C.c_char_p, sz]),
         "vp_engine_stream_buffers": (i, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]),
         "vp_engine_stream_block": (i, [vp]),
         "vp_engine_stream_stats": (i, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
@@ -332,6 +337,32 @@ class Engine:
         streams = [int(s) for s in streams]
         arr = (C.c_int * max(len(streams), 1))(*streams)
         self._check(self.lib.vp_engine_reset_streams(self.h, arr, len(streams)))
+
+    # ---- per-stream state snapshots: move a running stream to another slot or engine, checkpoint a render ----
+    def snapshot_size(self, count):
+        """Bytes of a snapshot of `count` streams (header + count records) for this engine as prepared."""
+        n = C.c_size_t(0)
+        self._check(self.lib.vp_engine_snapshot_size(self.h, int(count), C.byref(n)))
+        return n.value
+
+    def save_streams(self, streams):
+        """The state the listed streams start their next process call with, as an opaque, self-checking blob (bytes).
+        Waits for every call already issued; changes nothing in the engine."""
+        streams = [int(s) for s in streams]
+        arr = (C.c_int * max(len(streams), 1))(*streams)
+        n = self.snapshot_size(len(streams))
+        buf = C.create_string_buffer(n)
+        self._check(self.lib.vp_engine_save_streams(self.h, arr, len(streams), buf, n))
+        return buf.raw
+
+    def load_streams(self, streams, blob):
+        """Record i of blob (save_streams of this or a compatible engine) becomes the state of slot streams[i]: same layout
+        key, same grid phase, or this engine has processed no block since prepare / reset (it then adopts the blob's grids).
+        Validated before anything is issued; on an error nothing changes."""
+        streams = [int(s) for s in streams]
+        arr = (C.c_int * max(len(streams), 1))(*streams)
+        blob = bytes(blob)
+        self._check(self.lib.vp_engine_load_streams(self.h, arr, len(streams), blob, len(blob)))
 
     # ---- low-latency streaming: one host block per call through pinned buffers and a CUDA graph per block phase ----
     def stream_buffers(self):

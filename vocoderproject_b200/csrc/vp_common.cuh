@@ -277,6 +277,8 @@ struct VPResetSegs {
 };
 // one launch: the silent state of streams list[0 .. count) (list == NULL: streams 0 .. count - 1) in every segment
 void vp_launch_reset_streams(cudaStream_t st, const VPResetSegs& segs, const int* list, int count);
+// one launch: streams list[0 .. count) of every segment -> stage [count][unitsPerStream] x 16 bytes (save), or back (load)
+void vp_launch_snapshot_streams(cudaStream_t st, const VPResetSegs& segs, const int* list, int count, void* stage, bool save);
 // the [nBlocks][S] table of a call with scheduled changes: entry (b, s) = the last event of stream s at or before call-local
 // block b (events of s: evBlk / evVal[off[s] .. off[s + 1]), ascending blocks), else cur[s]
 void vp_launch_expand_stream_params(cudaStream_t st, const VPStreamParam* cur, const int* off, const int* evBlk,

@@ -152,6 +152,13 @@ struct vp_engine {
     std::vector<int> rsList;
     int *rsPinned = nullptr, *dRsList = nullptr;
     cudaEvent_t evRsUp = nullptr;
+    // ---- stream snapshots (vp_engine_save_streams / vp_engine_load_streams): packed records [count][unitsPerStream] followed
+    // by the stream list, staged through pinned host memory (snapPinned) and device memory (dSnap) of snapCap bytes each,
+    // allocated at the first save / load that needs them, outside the workspace budget. evSnapUp marks when the last upload
+    // has read snapPinned; evSnapSide orders a save behind the side stream's mark chain.
+    uint8_t *snapPinned = nullptr, *dSnap = nullptr;
+    size_t snapCap = 0;
+    cudaEvent_t evSnapUp = nullptr, evSnapSide = nullptr;
     double *dRV = nullptr, *dRS = nullptr, *dAV = nullptr, *dAS = nullptr, *dEeV = nullptr, *dEeS = nullptr, *dG = nullptr, *dGs = nullptr;
     int *dPeriod = nullptr, *dList = nullptr, *dListCount = nullptr;
     uint32_t* dYFlags = nullptr;
@@ -375,6 +382,9 @@ static void free_workspace(vp_engine* e) {
     if (e->spPinned) { cudaFreeHost(e->spPinned); e->spPinned = nullptr; }
     if (e->pordPinned) { cudaFreeHost(e->pordPinned); e->pordPinned = nullptr; }
     if (e->rsPinned) { cudaFreeHost(e->rsPinned); e->rsPinned = nullptr; }
+    if (e->snapPinned) { cudaFreeHost(e->snapPinned); e->snapPinned = nullptr; }
+    if (e->dSnap) { cudaFree(e->dSnap); e->dSnap = nullptr; }
+    e->snapCap = 0;
     void** ptrs[] = {(void**)&e->dSP, (void**)&e->dOrdP, (void**)&e->dRsList, (void**)&e->dGate, (void**)&e->dRV, (void**)&e->dRS, (void**)&e->dAV, (void**)&e->dAS, (void**)&e->dEeV,
                      (void**)&e->dEeS, (void**)&e->dG, (void**)&e->dGs, (void**)&e->dPeriod, (void**)&e->dList, (void**)&e->dListCount,
                      (void**)&e->dYFlags, (void**)&e->dFrames, (void**)&e->dAP, (void**)&e->dOutE, (void**)&e->dOutV,
@@ -416,7 +426,9 @@ extern "C" int vp_engine_create(vp_engine** out, int device) {
         cudaEventCreate(&e->evT0) != cudaSuccess || cudaEventCreate(&e->evT1) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->evSpUp, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&e->evRsUp, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&e->evSchUp, cudaEventDisableTiming) != cudaSuccess) {
+        cudaEventCreateWithFlags(&e->evSchUp, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&e->evSnapUp, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&e->evSnapSide, cudaEventDisableTiming) != cudaSuccess) {
         cudaGetLastError();
         delete e;
         return VP_E_CUDA;
@@ -455,6 +467,7 @@ extern "C" void vp_engine_destroy(vp_engine* e) {
     for (int i = 0; i < 8; ++i) cudaEventDestroy(e->evTimer[i]);
     for (auto ev : e->evSide) cudaEventDestroy(ev);
     cudaEventDestroy(e->evFork); cudaEventDestroy(e->evJoin); cudaEventDestroy(e->evSpUp); cudaEventDestroy(e->evRsUp); cudaEventDestroy(e->evSchUp);
+    cudaEventDestroy(e->evSnapUp); cudaEventDestroy(e->evSnapSide);
     for (int i = 0; i < 2; ++i) { cudaEventDestroy(e->evYin[i]); cudaEventDestroy(e->evMarks[i]); cudaEventDestroy(e->evSideDone[i]); cudaEventDestroy(e->evMix[i]); }
     cudaStreamDestroy(e->st); cudaStreamDestroy(e->stIn); cudaStreamDestroy(e->stOut); cudaStreamDestroy(e->st2);
     delete e;
@@ -889,6 +902,395 @@ static int apply_stream_resets(vp_engine* e) {
     e->launches++;
     for (int s : e->rsList) e->rsMark[s] = 0;
     e->rsList.clear();
+    return VP_OK;
+}
+
+// ---------------------------------------------------------------------------
+// Stream snapshots (vp_engine_save_streams / vp_engine_load_streams). A blob is one SnapHeader and `count` records; a
+// record is a SnapRecord followed by the stream's raw units of every carried_state() segment, in segment order. The header
+// holds the layout key (what must match for the raw units to mean the same thing) and the source's frame grids.
+// ---------------------------------------------------------------------------
+#define VP_SNAP_MAGIC 0x53535056u  // "VPSS"
+#define VP_SNAP_VERSION 1u
+struct SnapHeader {
+    uint32_t magic, version;
+    uint64_t checksum;  // FNV-1a over the header's 64-bit words with this field zero
+    // layout key
+    double sampleRate;
+    int32_t B, H, gateCarry, capV, capS, capP, window, nSeg, unitsPerStream, count, reserved0, reserved1;
+    int32_t segUnits[VP_RESET_MAXSEG];
+    // the source's GridState
+    int64_t blocksDone, nextFrameV, nextChunkP;
+    int64_t orphAbs[VP_ORPH], carryAbsP[VP_PC];
+    int32_t alignedV, nChunk;
+    int32_t alignedOrdV[VP_VC], alignedOrdS[VP_VC], orphOrdV[VP_ORPH], orphOrdS[VP_ORPH], carryLimP[VP_PC];
+};
+struct SnapRecord {
+    uint64_t checksum;  // FNV-1a over the record's 64-bit words (this struct, then the raw units) with this field zero
+    vp_stream_params p;
+    vp_stream_orders o;
+    int32_t lpcPitchIn, lpcPitchNext;
+    int32_t rowOrdV[VP_VC], rowOrdS[VP_VC], orphRowOrdV[VP_ORPH], orphRowOrdS[VP_ORPH];  // last non-zero coefficient index
+    int32_t reserved;
+};
+static_assert(sizeof(SnapHeader) == VP_SNAPSHOT_HEADER_BYTES && sizeof(SnapRecord) == VP_SNAPSHOT_RECORD_BYTES,
+              "snapshot layout documented in vp_engine.h");
+static_assert(sizeof(SnapHeader) % 16 == 0 && sizeof(SnapRecord) % 16 == 0, "raw units stay 16-byte aligned");
+
+static uint64_t snap_hash(uint64_t h, const void* p, size_t bytes) {  // bytes % 8 == 0
+    const uint8_t* b = (const uint8_t*)p;
+    for (size_t i = 0; i < bytes; i += 8) {
+        uint64_t w;
+        memcpy(&w, b + i, 8);
+        h = (h ^ w) * 1099511628211ull;
+    }
+    return h;
+}
+static const uint64_t kSnapHashSeed = 14695981039346656037ull;
+static uint64_t snap_header_hash(SnapHeader h) { h.checksum = 0; return snap_hash(kSnapHashSeed, &h, sizeof h); }
+static uint64_t snap_record_hash(SnapRecord r, const uint8_t* raw, size_t rawBytes) {
+    r.checksum = 0;
+    return snap_hash(snap_hash(kSnapHashSeed, &r, sizeof r), raw, rawBytes);
+}
+
+static size_t snap_record_bytes(const VPResetSegs& segs) { return sizeof(SnapRecord) + (size_t)segs.unitsPerStream * 16; }
+
+// byte offset of the segment at `base` inside a record's raw units
+static size_t seg_offset(const VPResetSegs& segs, const void* base) {
+    size_t off = 0;
+    for (int j = 0; j < segs.nSeg && segs.seg[j].base != base; ++j) off += (size_t)segs.seg[j].units * 16;
+    return off;
+}
+
+static void snap_layout(const vp_engine* e, const VPResetSegs& segs, SnapHeader* h) {
+    memset(h, 0, sizeof *h);
+    h->magic = VP_SNAP_MAGIC; h->version = VP_SNAP_VERSION;
+    h->sampleRate = e->fs; h->B = e->B; h->H = e->H; h->gateCarry = e->gateCarry;
+    h->capV = e->capV; h->capS = e->capS; h->capP = e->capP; h->window = e->window;
+    h->nSeg = segs.nSeg; h->unitsPerStream = segs.unitsPerStream;
+    for (int j = 0; j < segs.nSeg; ++j) h->segUnits[j] = segs.seg[j].units;
+}
+static bool same_layout(const SnapHeader& a, const SnapHeader& b) {
+    if (a.sampleRate != b.sampleRate || a.B != b.B || a.H != b.H || a.gateCarry != b.gateCarry || a.capV != b.capV ||
+        a.capS != b.capS || a.capP != b.capP || a.window != b.window || a.nSeg != b.nSeg || a.unitsPerStream != b.unitsPerStream)
+        return false;
+    return memcmp(a.segUnits, b.segUnits, sizeof a.segUnits) == 0;
+}
+
+static void snap_put_grid(const GridState& gs, SnapHeader* h) {
+    h->blocksDone = gs.blocksDone; h->nextFrameV = gs.nextFrameV; h->nextChunkP = gs.nextChunkP;
+    h->alignedV = gs.alignedV; h->nChunk = gs.nChunk;
+    for (int j = 0; j < VP_VC; ++j) { h->alignedOrdV[j] = gs.alignedOrdV[j]; h->alignedOrdS[j] = gs.alignedOrdS[j]; }
+    for (int j = 0; j < VP_ORPH; ++j) { h->orphAbs[j] = gs.orphAbs[j]; h->orphOrdV[j] = gs.orphOrdV[j]; h->orphOrdS[j] = gs.orphOrdS[j]; }
+    for (int j = 0; j < VP_PC; ++j) { h->carryAbsP[j] = gs.carryAbsP[j]; h->carryLimP[j] = gs.carryLimP[j]; }
+}
+static void snap_get_grid(const SnapHeader& h, GridState* gs) {
+    gs->blocksDone = h.blocksDone; gs->nextFrameV = h.nextFrameV; gs->nextChunkP = h.nextChunkP;
+    gs->alignedV = h.alignedV; gs->nChunk = h.nChunk;
+    for (int j = 0; j < VP_VC; ++j) { gs->alignedOrdV[j] = h.alignedOrdV[j]; gs->alignedOrdS[j] = h.alignedOrdS[j]; }
+    for (int j = 0; j < VP_ORPH; ++j) { gs->orphAbs[j] = h.orphAbs[j]; gs->orphOrdV[j] = h.orphOrdV[j]; gs->orphOrdS[j] = h.orphOrdS[j]; }
+    for (int j = 0; j < VP_PC; ++j) { gs->carryAbsP[j] = h.carryAbsP[j]; gs->carryLimP[j] = h.carryLimP[j]; }
+}
+
+// an orphan slot whose frame still emits at the next call (an expired one is a free slot: grid_begin frees it first)
+static bool orph_live(const GridState& gs, int j) {
+    return gs.orphAbs[j] >= 0 && gs.orphAbs[j] + gs.z.wlenV > gs.blocksDone * (long long)gs.B;
+}
+
+// The grid phase: every absolute position relative to the next call's start, with the counters that go with it (the row
+// widths are not part of it). Two engines with the same phase run the same frames at the same call-local positions.
+struct GridPhase {
+    long long nextV, nextP, orph[VP_ORPH], carry[VP_PC];
+    int nChunk, alignedV, lim[VP_PC];
+};
+static GridPhase grid_phase(const GridState& gs) {
+    GridPhase p;
+    memset(&p, 0, sizeof p);
+    const long long u0 = gs.blocksDone * (long long)gs.B;
+    p.nextV = gs.nextFrameV - u0; p.nextP = gs.nextChunkP - u0; p.nChunk = gs.nChunk; p.alignedV = gs.alignedV;
+    for (int j = 0; j < VP_ORPH; ++j) p.orph[j] = orph_live(gs, j) ? gs.orphAbs[j] - u0 : -1;
+    for (int j = 0; j < VP_PC; ++j) {
+        p.carry[j] = gs.carryAbsP[j] >= 0 ? gs.carryAbsP[j] - u0 : 1;
+        p.lim[j] = gs.carryAbsP[j] >= 0 ? gs.carryLimP[j] : 0;
+    }
+    return p;
+}
+
+// A grid state a target adopts whole must be one that process calls can produce: the kernels size and index by it.
+static bool grid_state_ok(const GridState& gs, int capV, int capS) {
+    const vp_sizes& z = gs.z;
+    if (gs.blocksDone < 0 || gs.blocksDone > (1LL << 40)) return false;
+    const long long u0 = gs.blocksDone * (long long)gs.B;
+    if (gs.nextFrameV - u0 < 0 || gs.nextFrameV - u0 >= z.hopV || gs.nextChunkP - u0 < 0 || gs.nextChunkP - u0 >= z.chunk) return false;
+    if (gs.alignedV < 0 || gs.alignedV > VP_VC || gs.nChunk < 0 || gs.nChunk > 3) return false;
+    for (int j = 0; j < VP_VC; ++j)
+        if (gs.alignedOrdV[j] < 0 || gs.alignedOrdV[j] > capV || gs.alignedOrdS[j] < 0 || gs.alignedOrdS[j] > capS) return false;
+    for (int j = 0; j < VP_ORPH; ++j) {
+        if (gs.orphOrdV[j] < 0 || gs.orphOrdV[j] > capV || gs.orphOrdS[j] < 0 || gs.orphOrdS[j] > capS) return false;
+        if (gs.orphAbs[j] < -1 || (gs.orphAbs[j] >= 0 && gs.orphAbs[j] >= u0)) return false;
+    }
+    for (int j = 0; j < VP_PC; ++j) {
+        if (gs.carryAbsP[j] < -1 || (gs.carryAbsP[j] >= 0 && (gs.carryAbsP[j] >= u0 || u0 - gs.carryAbsP[j] > (1LL << 30)))) return false;
+        if (gs.carryLimP[j] < 0 || gs.carryLimP[j] > 4) return false;
+    }
+    return true;
+}
+
+// last coefficient index whose bits are not zero (rows are zero padded: truncating there is exact, -0.0 included)
+static int row_order(const uint8_t* row, int len) {
+    for (int k = len - 1; k > 0; --k) {
+        uint64_t w;
+        memcpy(&w, row + 8 * (size_t)k, 8);
+        if (w) return k;
+    }
+    return 0;
+}
+static void snap_row_orders(vp_engine* e, const VPResetSegs& segs, const uint8_t* raw, SnapRecord* r) {
+    const size_t oCV = seg_offset(segs, e->cAV), oCS = seg_offset(segs, e->cAS), oOV = seg_offset(segs, e->oAV),
+                 oOS = seg_offset(segs, e->oAS);
+    const int wV = e->capV + 1, wS = e->capS + 1;
+    for (int i = 0; i < VP_VC; ++i) {
+        r->rowOrdV[i] = row_order(raw + oCV + (size_t)i * wV * 8, wV);
+        r->rowOrdS[i] = row_order(raw + oCS + (size_t)i * wS * 8, wS);
+    }
+    for (int j = 0; j < VP_ORPH; ++j) {
+        r->orphRowOrdV[j] = row_order(raw + oOV + (size_t)j * wV * 8, wV);
+        r->orphRowOrdS[j] = row_order(raw + oOS + (size_t)j * wS * 8, wS);
+    }
+}
+
+// the raw units of a stream that has heard silence since prepare (what k_reset_streams writes)
+static void snap_silent(const VPResetSegs& segs, uint8_t* raw) {
+    for (int j = 0; j < segs.nSeg; ++j) {
+        const VPResetSeg& sg = segs.seg[j];
+        double* d = reinterpret_cast<double*>(raw);
+        const size_t n = (size_t)sg.units * 2;
+        for (size_t k = 0; k < n; ++k) d[k] = (sg.kind == VP_FILL_GATED) ? -1.0 : 0.0;
+        if (sg.kind == VP_FILL_ONE_AT) d[sg.oneAt] = 1.0;
+        raw += (size_t)sg.units * 16;
+    }
+}
+
+// Every integer of the raw state that a kernel takes as a bound or an index: mark counts within the storage, periods within
+// the lag range (they index the note and Hann tables).
+static bool snap_raw_ok(vp_engine* e, const VPResetSegs& segs, const uint8_t* raw) {
+    const int tauMax = e->sz.tauMax;
+    auto period_ok = [&](int p) { return p >= 0 && p <= tauMax; };
+    VPMarkState m;
+    memcpy(&m, raw + seg_offset(segs, e->cMarks), sizeof m);
+    if (m.nAn < 0 || m.nAn > VP_SLOTS || m.nSt < 0 || m.nSt > VP_SLOTS) return false;
+    if (!period_ok(m.period) || !period_ok(m.prevPeriod) || !period_ok(m.prevVoicedPeriod) || !period_ok(m.periodNew)) return false;
+    const size_t oF = seg_offset(segs, e->cFrames);
+    for (int j = 0; j < VP_PC; ++j) {
+        vp_pitch_frame f;
+        memcpy(&f, raw + oF + j * sizeof f, sizeof f);
+        if (f.nAn < 0 || f.nAn > VP_MAX_MARKS || f.nSt < 0 || f.nSt > VP_MAX_MARKS || f.nAnOv < 0 || f.nAnOv > VP_MAX_MARKS) return false;
+        if (!period_ok(f.period) || !period_ok(f.periodPsola) || !period_ok(f.periodNew)) return false;
+    }
+    return true;
+}
+
+// pinned + device staging for `count` records (raw units, then the stream list); VP_E_NOMEM before anything is issued
+static int snap_staging(vp_engine* e, int count, size_t rawBytes) {
+    const size_t need = (size_t)count * rawBytes + ((size_t)count * sizeof(int) + 15) / 16 * 16;
+    if (need <= e->snapCap) return VP_OK;
+    VP_CUDA_OK(cudaEventSynchronize(e->evSnapUp));  // the last upload has read the old pinned buffer
+    if (e->snapPinned) cudaFreeHost(e->snapPinned);
+    if (e->dSnap) cudaFree(e->dSnap);  // (cudaFree waits for the device: only when a larger list comes)
+    e->snapPinned = nullptr; e->dSnap = nullptr; e->snapCap = 0;
+    if (cudaHostAlloc((void**)&e->snapPinned, need, cudaHostAllocDefault) != cudaSuccess ||
+        cudaMalloc((void**)&e->dSnap, need) != cudaSuccess) {
+        cudaGetLastError();
+        if (e->snapPinned) cudaFreeHost(e->snapPinned);
+        e->snapPinned = nullptr; e->dSnap = nullptr;
+        return vp_err(e, VP_E_NOMEM, "no pinned host or device memory for the snapshot staging buffers");
+    }
+    e->snapCap = need;
+    return VP_OK;
+}
+
+// the checks save and load share: state, list (in range; a load also refuses duplicates), buffer
+static int snap_check_list(vp_engine* e, const int* streams, int count, const void* buf, bool unique) {
+    if (!e->prepared) return vp_err(e, VP_E_STATE, "vp_engine_prepare has not been called");
+    if (e->failed) return vp_err(e, VP_E_STATE, "an earlier process call failed half way: the carried stream state is undefined, call vp_engine_reset");
+    if (count < 0 || (count > 0 && !streams) || !buf) return vp_err(e, VP_E_ARG, "streams and buf must be non-null and count >= 0");
+    std::vector<uint8_t> seen(unique ? (size_t)e->S : 0, 0);
+    for (int i = 0; i < count; ++i) {
+        if (streams[i] < 0 || streams[i] >= e->S) return vp_err(e, VP_E_ARG, "stream index outside [0, nStreams)");
+        if (unique && seen[streams[i]]++) return vp_err(e, VP_E_ARG, "a stream is listed twice");
+    }
+    return VP_OK;
+}
+
+extern "C" int vp_engine_snapshot_size(const vp_engine* e, int count, size_t* bytes) {
+    if (!e || !bytes || count < 0) return VP_E_ARG;
+    if (!e->prepared) return VP_E_STATE;
+    *bytes = sizeof(SnapHeader) + (size_t)count * snap_record_bytes(carried_state(const_cast<vp_engine*>(e)));
+    return VP_OK;
+}
+
+extern "C" int vp_engine_save_streams(vp_engine* e, const int* streams, int count, void* buf, size_t bytes) {
+    if (!e) return VP_E_ARG;
+    int rc = snap_check_list(e, streams, count, buf, false);
+    if (rc) return rc;
+    const VPResetSegs segs = carried_state(e);
+    const size_t rawB = (size_t)segs.unitsPerStream * 16, recB = snap_record_bytes(segs);
+    if (bytes < sizeof(SnapHeader) + (size_t)count * recB) return vp_err(e, VP_E_ARG, "buffer smaller than vp_engine_snapshot_size");
+    VP_CUDA_OK(cudaSetDevice(e->device));
+    if ((rc = snap_staging(e, count, rawB))) return rc;
+    if (count > 0) {
+        // behind every call already issued, the side stream's mark chain included: one gather, one copy back
+        int* list = reinterpret_cast<int*>(e->snapPinned + (size_t)count * rawB);
+        VP_CUDA_OK(cudaEventSynchronize(e->evSnapUp));
+        memcpy(list, streams, (size_t)count * sizeof(int));
+        VP_CUDA_OK(cudaEventRecord(e->evSnapSide, e->st2));
+        VP_CUDA_OK(cudaStreamWaitEvent(e->st, e->evSnapSide, 0));
+        VP_CUDA_OK(cudaMemcpyAsync(e->dSnap + (size_t)count * rawB, list, (size_t)count * sizeof(int), cudaMemcpyHostToDevice, e->st));
+        vp_launch_snapshot_streams(e->st, segs, reinterpret_cast<const int*>(e->dSnap + (size_t)count * rawB), count, e->dSnap, true);
+        VP_CUDA_OK(vp_take_launch_error());
+        VP_CUDA_OK(cudaMemcpyAsync(e->snapPinned, e->dSnap, (size_t)count * rawB, cudaMemcpyDeviceToHost, e->st));
+        VP_CUDA_OK(cudaEventRecord(e->evSnapUp, e->st));
+        VP_CUDA_OK(cudaStreamSynchronize(e->st));
+    }
+    SnapHeader h;
+    snap_layout(e, segs, &h);
+    snap_put_grid(e->gs, &h);
+    h.count = count;
+    h.checksum = snap_header_hash(h);
+    uint8_t* out = (uint8_t*)buf;
+    memcpy(out, &h, sizeof h);
+    for (int i = 0; i < count; ++i) {
+        const int s = streams[i];
+        uint8_t* rec = out + sizeof h + (size_t)i * recB;
+        uint8_t* raw = rec + sizeof(SnapRecord);
+        if (e->rsMark[s]) snap_silent(segs, raw);  // a reset of it is pending: the state that reset gives
+        else memcpy(raw, e->snapPinned + (size_t)i * rawB, rawB);
+        SnapRecord r;
+        memset(&r, 0, sizeof r);
+        r.p = e->sprm[s]; r.o = e->sord[s]; r.lpcPitchIn = e->pordIn[s]; r.lpcPitchNext = e->pordNext[s];
+        snap_row_orders(e, segs, raw, &r);
+        r.checksum = snap_record_hash(r, raw, rawB);
+        memcpy(rec, &r, sizeof r);
+    }
+    return VP_OK;
+}
+
+extern "C" int vp_engine_load_streams(vp_engine* e, const int* streams, int count, const void* buf, size_t bytes) {
+    if (!e) return VP_E_ARG;
+    int rc = snap_check_list(e, streams, count, buf, true);
+    if (rc) return rc;
+    const VPResetSegs segs = carried_state(e);
+    const size_t rawB = (size_t)segs.unitsPerStream * 16, recB = snap_record_bytes(segs);
+    // ---- everything is validated on the host before anything is issued
+    SnapHeader h, mine;
+    if (bytes < sizeof h) return vp_err(e, VP_E_ARG, "buffer smaller than a snapshot header");
+    memcpy(&h, buf, sizeof h);
+    if (h.magic != VP_SNAP_MAGIC || h.version != VP_SNAP_VERSION) return vp_err(e, VP_E_ARG, "not a stream snapshot of this format version");
+    if (h.checksum != snap_header_hash(h)) return vp_err(e, VP_E_ARG, "snapshot header checksum mismatch");
+    snap_layout(e, segs, &mine);
+    if (!same_layout(h, mine))
+        return vp_err(e, VP_E_STATE, "snapshot of an engine with another layout (sample rate, block size, reserved orders or window)");
+    if (h.count != count) return vp_err(e, VP_E_ARG, "count differs from the number of records in the snapshot");
+    if (bytes < sizeof h + (size_t)count * recB) return vp_err(e, VP_E_ARG, "buffer shorter than the snapshot it holds");
+    if (count == 0) return VP_OK;
+    GridState src = e->gs;
+    snap_get_grid(h, &src);
+    const bool adopt = e->gs.blocksDone == 0;  // a target that has processed no block takes the source's grids
+    if (adopt) {
+        if (!grid_state_ok(src, e->capV, e->capS)) return vp_err(e, VP_E_ARG, "snapshot grid state out of range");
+    } else {
+        const GridPhase a = grid_phase(src), b = grid_phase(e->gs);
+        if (memcmp(&a, &b, sizeof a) != 0)
+            return vp_err(e, VP_E_STATE, "snapshot grid phase differs from this engine's (another block sequence or bypass history)");
+    }
+    const uint8_t* in = (const uint8_t*)buf + sizeof h;
+    std::vector<SnapRecord> recs((size_t)count);
+    for (int i = 0; i < count; ++i) {
+        const uint8_t* rec = in + (size_t)i * recB;
+        const uint8_t* raw = rec + sizeof(SnapRecord);
+        SnapRecord& r = recs[i];
+        memcpy(&r, rec, sizeof r);
+        if (r.checksum != snap_record_hash(r, raw, rawB)) return vp_err(e, VP_E_ARG, "snapshot record checksum mismatch");
+        if (!stream_params_ok(r.p)) return vp_err(e, VP_E_RANGE, "snapshot record: parameter outside the plug-in's range");
+        if ((rc = check_orders(e, &r.o, 1, 1))) return rc;
+        if (r.lpcPitchIn < 2 || r.lpcPitchIn > 100 || r.lpcPitchNext < 2 || r.lpcPitchNext > 100)
+            return vp_err(e, VP_E_RANGE, "snapshot record: lpcPitch outside the plug-in's range");
+        if (r.lpcPitchIn > e->capP || r.lpcPitchNext > e->capP) return vp_err(e, VP_E_STATE, "snapshot record: lpcPitch beyond the reservation");
+        if (!snap_raw_ok(e, segs, raw)) return vp_err(e, VP_E_RANGE, "snapshot record: mark count or period outside its range");
+        SnapRecord chk = r;
+        snap_row_orders(e, segs, raw, &chk);
+        if (memcmp(&chk, &r, sizeof r) != 0) return vp_err(e, VP_E_ARG, "snapshot record: row orders do not match its rows");
+    }
+    VP_CUDA_OK(cudaSetDevice(e->device));
+    if ((rc = snap_staging(e, count, rawB))) return rc;
+    // ---- issued behind every call already issued: one upload (the pinned buffer is rewritten only after the last upload has
+    // read it), one scatter
+    VP_CUDA_OK(cudaEventSynchronize(e->evSnapUp));
+    int* list = reinterpret_cast<int*>(e->snapPinned + (size_t)count * rawB);
+    for (int i = 0; i < count; ++i) memcpy(e->snapPinned + (size_t)i * rawB, in + (size_t)i * recB + sizeof(SnapRecord), rawB);
+    memcpy(list, streams, (size_t)count * sizeof(int));
+    const size_t upB = (size_t)count * rawB + (size_t)count * sizeof(int);
+    VP_CUDA_OK(cudaMemcpyAsync(e->dSnap, e->snapPinned, upB, cudaMemcpyHostToDevice, e->st));
+    VP_CUDA_OK(cudaEventRecord(e->evSnapUp, e->st));
+    vp_launch_snapshot_streams(e->st, segs, reinterpret_cast<const int*>(e->dSnap + (size_t)count * rawB), count, e->dSnap, false);
+    VP_CUDA_OK(vp_take_launch_error());
+    e->launches++;
+    // ---- host bookkeeping
+    std::vector<uint8_t> loaded((size_t)e->S, 0);
+    for (int i = 0; i < count; ++i) loaded[streams[i]] = 1;
+    if (adopt) {
+        snap_get_grid(h, &e->gs);
+        // events before the adopted block would have applied already: the values in force from them on
+        bool changed = false;
+        for (auto it = e->sched.begin(); it != e->sched.end() && it->first.first < e->gs.blocksDone;) {
+            const int s = it->first.second;
+            const vp_engine::Pending& q = it->second;
+            changed = put_one_stream(e, s, q.hasP ? q.p : e->sprm[s], q.hasO ? q.o : e->sord[s]) || changed;
+            it = e->sched.erase(it);
+        }
+        if (changed) stream_table_changed(e);
+    }
+    // the row widths cover each loaded row's own order (not the source's batch-wide widest)
+    for (const SnapRecord& r : recs) {
+        for (int i = VP_VC - e->gs.alignedV; i < VP_VC; ++i) {
+            e->gs.alignedOrdV[i] = std::max(e->gs.alignedOrdV[i], r.rowOrdV[i]);
+            e->gs.alignedOrdS[i] = std::max(e->gs.alignedOrdS[i], r.rowOrdS[i]);
+        }
+        for (int j = 0; j < VP_ORPH; ++j) {
+            if (!orph_live(e->gs, j)) continue;
+            e->gs.orphOrdV[j] = std::max(e->gs.orphOrdV[j], r.orphRowOrdV[j]);
+            e->gs.orphOrdS[j] = std::max(e->gs.orphOrdS[j], r.orphRowOrdS[j]);
+        }
+    }
+    {   // the carried chunk gains stay uniform only if every loaded one is the batch's
+        const size_t oPG = seg_offset(segs, e->cPG[e->histCur]);
+        float g0;
+        memcpy(&g0, in + sizeof(SnapRecord) + oPG, sizeof g0);
+        bool same = e->pgCarryAny || e->pgCarry == g0;
+        for (int i = 0; i < count && same; ++i) {
+            float pg[VP_PC * 4];
+            memcpy(pg, in + (size_t)i * recB + sizeof(SnapRecord) + oPG, sizeof pg);
+            for (float g : pg) same = same && g == g0;
+        }
+        e->pgCarry = same ? g0 : -1.0f;
+        e->pgCarryAny = false;
+    }
+    bool changed = false, ordChanged = false;
+    for (int i = 0; i < count; ++i) {
+        const int s = streams[i];
+        changed = put_one_stream(e, s, recs[i].p, recs[i].o) || changed;
+        if (e->pordIn[s] != recs[i].lpcPitchIn) { e->pordIn[s] = recs[i].lpcPitchIn; ordChanged = true; }
+        e->pordNext[s] = recs[i].lpcPitchNext;
+        e->rsMark[s] = 0;
+    }
+    if (changed) stream_table_changed(e);
+    if (ordChanged) pitch_orders_changed(e);
+    // a loaded slot drops its pending reset and its pending scheduled events
+    e->rsList.erase(std::remove_if(e->rsList.begin(), e->rsList.end(), [&](int s) { return loaded[s] != 0; }), e->rsList.end());
+    for (auto it = e->sched.begin(); it != e->sched.end();) {
+        if (loaded[it->first.second]) it = e->sched.erase(it);
+        else ++it;
+    }
     return VP_OK;
 }
 

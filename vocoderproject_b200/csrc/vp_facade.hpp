@@ -159,6 +159,24 @@ public:
     // prepareToPlay for some instances of the running batch (a slot handed to a new user): from the next block on, each
     // listed stream continues as one that has heard only silence since prepare; the others are not touched
     void restartStreams(const int* streams, int count) { engine.check(vp_engine_reset_streams(engine.h, streams, count)); }
+    // per-stream state snapshots: the state streams[0 .. count) start their next block with, as an opaque self-checking blob
+    // (waits for the GPU; changes nothing), and back into slots of this or a compatible instance set (same sample rate, block
+    // size, reservations and window; same grid phase, or nothing processed since prepare / restart)
+    std::vector<uint8_t> saveStreams(const int* streams, int count) {
+        size_t bytes = 0;
+        engine.check(vp_engine_snapshot_size(engine.h, count, &bytes));
+        std::vector<uint8_t> blob(bytes);
+        engine.check(vp_engine_save_streams(engine.h, streams, count, blob.data(), blob.size()));
+        return blob;
+    }
+    // each loaded slot takes the saved key, gains and orders: the per-stream values pushed with every block are refreshed
+    void loadStreams(const int* streams, int count, const std::vector<uint8_t>& blob) {
+        engine.check(vp_engine_load_streams(engine.h, streams, count, blob.data(), blob.size()));
+        streamParams.resize((size_t)S);
+        engine.check(vp_engine_get_stream_params(engine.h, 0, S, streamParams.data()));
+        streamOrders.resize((size_t)S);
+        engine.check(vp_engine_get_stream_orders(engine.h, 0, S, streamOrders.data()));
+    }
     // automation at block accuracy: each event gives one stream its key and gains from an absolute block on (blocks counted
     // since prepare / restart); the engine applies them where the reference reads each value, also inside one multi-block call.
     // Pending events survive setParams / setStreamParams (which change the value from the next block on); restart drops them,

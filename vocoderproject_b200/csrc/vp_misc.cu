@@ -223,6 +223,37 @@ void vp_launch_reset_streams(cudaStream_t st, const VPResetSegs& segs, const int
     VP_LAUNCH(k_reset_streams<<<grid, 256, 0, st>>>(segs, list, count));
 }
 
+// Stream snapshots (vp_engine_save_streams / vp_engine_load_streams): the same segments, gathered into / scattered from a
+// packed staging buffer [count][unitsPerStream] of 16-byte units (a stream's units in segment order). Same grid as
+// k_reset_streams; one 16-byte load and one 16-byte store per unit.
+__device__ __forceinline__ double2* vp_seg_unit(const VPResetSegs& segs, int unit, size_t s) {
+    int j = 0, u = unit;
+    while (u >= segs.seg[j].units) { u -= segs.seg[j].units; ++j; }
+    return reinterpret_cast<double2*>(segs.seg[j].base) + s * (size_t)segs.seg[j].units + u;
+}
+__global__ void __launch_bounds__(256) k_save_streams(VPResetSegs segs, const int* __restrict__ list, int count,
+                                                      double2* __restrict__ stage) {
+    const int unit = blockIdx.x * blockDim.x + threadIdx.x;
+    if (unit >= segs.unitsPerStream) return;
+    for (int i = blockIdx.y; i < count; i += gridDim.y) {
+        const double2* src = vp_seg_unit(segs, unit, (size_t)__ldg(list + i));
+        stage[(size_t)i * segs.unitsPerStream + unit] = *src;
+    }
+}
+__global__ void __launch_bounds__(256) k_load_streams(VPResetSegs segs, const int* __restrict__ list, int count,
+                                                      const double2* __restrict__ stage) {
+    const int unit = blockIdx.x * blockDim.x + threadIdx.x;
+    if (unit >= segs.unitsPerStream) return;
+    for (int i = blockIdx.y; i < count; i += gridDim.y)
+        *vp_seg_unit(segs, unit, (size_t)__ldg(list + i)) = __ldg(stage + (size_t)i * segs.unitsPerStream + unit);
+}
+void vp_launch_snapshot_streams(cudaStream_t st, const VPResetSegs& segs, const int* list, int count, void* stage, bool save) {
+    if (count <= 0 || segs.unitsPerStream <= 0) return;
+    const dim3 grid((unsigned)((segs.unitsPerStream + 255) / 256), (unsigned)std::min(count, 65535));
+    if (save) VP_LAUNCH(k_save_streams<<<grid, 256, 0, st>>>(segs, list, count, (double2*)stage));
+    else VP_LAUNCH(k_load_streams<<<grid, 256, 0, st>>>(segs, list, count, (const double2*)stage));
+}
+
 // PitchProcess::silence() (PitchProcess.cpp:146-158) for every stream: both mark vectors cleared (their storage keeps its
 // values), pitch = prevPitch = 0, period = prevPeriod = 0. prevVoicedPeriod, periodNew and beta are not touched.
 __global__ void __launch_bounds__(128) k_marks_silence(VPMarkState* __restrict__ carry, int S) {
