@@ -413,14 +413,27 @@ int vp_engine_process_host_pcm16(vp_engine* e, int nBlocks, const int16_t* voice
 
 int vp_engine_sync(vp_engine* e);
 
-/* Low-latency streaming, one host block per call (BASELINE config 5). The engine owns pinned host buffers
- * voice / synthL / outL, each float[nStreams][samplesPerBlock]: fill the inputs, call vp_engine_stream_block, read
- * outL when it returns (L == R; gainSynth must be off on every stream, else VP_E_ARG; synthR is not carried). Equivalent to
- * vp_engine_process_host(e, 1, ...). The block's H2D copies, kernels and D2H copy are replayed from a CUDA graph
- * captured the first time each block phase (position of the block on the frame grids) occurs. Per-stream key and gain
- * changes between blocks need no new capture (the table is uploaded before the graph is launched); whether some stream has
- * the dry voice on is part of the graph's identity (it selects the mix kernel). */
+/* Low-latency streaming, one host block per call (BASELINE config 5). The engine owns pinned host buffers, each
+ * float[nStreams][samplesPerBlock], zero-initialised: fill the inputs, call vp_engine_stream_block, read the outputs when
+ * it returns. The block's H2D copies, kernels and D2H copies are replayed from a CUDA graph captured the first time each
+ * block phase (position of the block on the frame grids) occurs. Per-stream key and gain changes between blocks need no
+ * new capture (the table is uploaded before the graph is launched); whether some stream has a dry path on (voice or
+ * side-chain) is part of the graph's identity (it selects the mix kernel).
+ *   Mono, vp_engine_stream_buffers: voice / synthL / outL. Each block equals vp_engine_process_host(e, 1, voice, synthL,
+ * NULL, outL, NULL, B): the right side-chain channel is the left one, L == R. The dry side-chain must be off on every
+ * stream (gainSynth <= -59 dB, also through a scheduled event), else the block is refused with VP_E_ARG.
+ *   Stereo, vp_engine_stream_buffers_stereo: voice / synthL / outL are the mono buffers (either getter may come first and
+ * both return the same three pointers), synthR / outR are the right side-chain and the right output. From its first call
+ * on, every block equals vp_engine_process_host(e, 1, voice, synthL, synthR, outL, outR, B) bit for bit: the right
+ * side-chain's ring is carried from synthR on every block, outR is written for every stream (R == L where the dry
+ * side-chain is off), and the dry side-chain may be on for any stream, set or scheduled. Blocks streamed in mono before the
+ * switch keep their meaning (right channel = left channel). Stereo lasts until the next vp_engine_prepare, which frees
+ * every streaming buffer; it moves 2 x nStreams x samplesPerBlock x 4 more bytes over the host link per block.
+ * Any out pointer may be NULL. VP_E_ARG for e == NULL, VP_E_STATE before vp_engine_prepare, VP_E_NOMEM / VP_E_CUDA when
+ * the buffers cannot be had: the right-channel buffers are installed all together or not at all, so after such an error
+ * the engine streams in mono (with the mono buffers, if those could be allocated). */
 int vp_engine_stream_buffers(vp_engine* e, float** voice, float** synthL, float** outL);
+int vp_engine_stream_buffers_stereo(vp_engine* e, float** voice, float** synthL, float** synthR, float** outL, float** outR);
 int vp_engine_stream_block(vp_engine* e);
 int vp_engine_stream_stats(const vp_engine* e, uint64_t* graphLaunches, uint64_t* graphCaptures);
 

@@ -35,7 +35,7 @@ ABI_SYMBOLS = [
     "vp_engine_set_stream_params", "vp_engine_get_stream_params", "vp_engine_reset_streams", "vp_engine_schedule_stream_params",
     "vp_engine_set_stream_orders", "vp_engine_get_stream_orders", "vp_engine_schedule_stream_orders",
     "vp_engine_reserve_pitch_order", "vp_engine_set_stream_pitch_orders", "vp_engine_get_stream_pitch_orders",
-    "vp_engine_snapshot_size", "vp_engine_save_streams", "vp_engine_load_streams",
+    "vp_engine_snapshot_size", "vp_engine_save_streams", "vp_engine_load_streams", "vp_engine_stream_buffers_stereo",
 ]
 
 
@@ -179,6 +179,7 @@ def load_library(path=None):
         "vp_engine_save_streams": (i, [vp, C.POINTER(i), i, C.c_void_p, sz]),
         "vp_engine_load_streams": (i, [vp, C.POINTER(i), i, C.c_char_p, sz]),
         "vp_engine_stream_buffers": (i, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]),
+        "vp_engine_stream_buffers_stereo": (i, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]),
         "vp_engine_stream_block": (i, [vp]),
         "vp_engine_stream_stats": (i, [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
         "vp_measure_peaks2": (i, [vp, C.POINTER(dbl), C.POINTER(dbl)]),
@@ -365,15 +366,22 @@ class Engine:
         self._check(self.lib.vp_engine_load_streams(self.h, arr, len(streams), blob, len(blob)))
 
     # ---- low-latency streaming: one host block per call through pinned buffers and a CUDA graph per block phase ----
-    def stream_buffers(self):
-        """(voice, synthL, outL): numpy views [S][B] of the engine's pinned host buffers."""
-        pv, ps, po = C.c_void_p(), C.c_void_p(), C.c_void_p()
-        self._check(self.lib.vp_engine_stream_buffers(self.h, C.byref(pv), C.byref(ps), C.byref(po)))
+    def stream_buffers(self, stereo=False):
+        """(voice, synthL, outL): numpy views [S][B] of the engine's pinned host buffers. stereo=True: (voice, synthL, synthR,
+        outL, outR), and from then on until the next prepare every stream_block carries the right side-chain and returns
+        the right output (the dry side-chain may then be on for any stream)."""
         shape = (self.n_streams, self.block)
 
         def view(p):
             buf = (C.c_float * (shape[0] * shape[1])).from_address(p.value)
             return np.frombuffer(buf, dtype=np.float32).reshape(shape)
+        if stereo:
+            pv, ps, pr, po, por = (C.c_void_p() for _ in range(5))
+            self._check(self.lib.vp_engine_stream_buffers_stereo(self.h, C.byref(pv), C.byref(ps), C.byref(pr), C.byref(po),
+                                                                 C.byref(por)))
+            return view(pv), view(ps), view(pr), view(po), view(por)
+        pv, ps, po = C.c_void_p(), C.c_void_p(), C.c_void_p()
+        self._check(self.lib.vp_engine_stream_buffers(self.h, C.byref(pv), C.byref(ps), C.byref(po)))
         return view(pv), view(ps), view(po)
 
     def stream_block(self):

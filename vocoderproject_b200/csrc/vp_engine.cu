@@ -184,6 +184,10 @@ struct vp_engine {
     // ---- low-latency streaming (one host block per call): pinned host I/O, fixed device I/O, one CUDA graph per block phase
     float *sHostV = nullptr, *sHostS = nullptr, *sHostO = nullptr;  // pinned [S][B]
     float *sDevV = nullptr, *sDevS = nullptr, *sDevO = nullptr;     // device [S][B]
+    // stereo streaming (vp_engine_stream_buffers_stereo): right side-chain in / right output, allocated together; sHostR set =
+    // every later block carries synthR and writes outR, until vp_engine_prepare frees them
+    float *sHostR = nullptr, *sHostOR = nullptr;  // pinned [S][B]
+    float *sDevR = nullptr, *sDevOR = nullptr;    // device [S][B]
     std::map<std::vector<long long>, cudaGraphExec_t> graphs;
     uint64_t graphLaunches = 0, graphCaptures = 0;
     // host-path staging (device), 3 slices
@@ -406,6 +410,10 @@ static void free_workspace(vp_engine* e) {
     if (e->sDevV) { cudaFree(e->sDevV); e->sDevV = nullptr; }
     if (e->sDevS) { cudaFree(e->sDevS); e->sDevS = nullptr; }
     if (e->sDevO) { cudaFree(e->sDevO); e->sDevO = nullptr; }
+    if (e->sHostR) { cudaFreeHost(e->sHostR); e->sHostR = nullptr; }
+    if (e->sHostOR) { cudaFreeHost(e->sHostOR); e->sHostOR = nullptr; }
+    if (e->sDevR) { cudaFree(e->sDevR); e->sDevR = nullptr; }
+    if (e->sDevOR) { cudaFree(e->sDevOR); e->sDevOR = nullptr; }
 }
 
 extern "C" int vp_engine_create(vp_engine** out, int device) {
@@ -2314,13 +2322,46 @@ extern "C" int vp_engine_stream_buffers(vp_engine* e, float** voice, float** syn
     return VP_OK;
 }
 
+// The four right-channel buffers are allocated together and only then installed: a failed allocation leaves the engine in
+// mono streaming.
+extern "C" int vp_engine_stream_buffers_stereo(vp_engine* e, float** voice, float** synthL, float** synthR, float** outL,
+                                               float** outR) {
+    int rc = vp_engine_stream_buffers(e, voice, synthL, outL);
+    if (rc) return rc;
+    if (!e->sHostR) {
+        const size_t bytes = (size_t)e->S * e->B * sizeof(float);
+        float *hR = nullptr, *hO = nullptr, *dR = nullptr, *dO = nullptr;
+        cudaError_t ce = cudaHostAlloc((void**)&hR, bytes, cudaHostAllocDefault);
+        if (ce == cudaSuccess) ce = cudaHostAlloc((void**)&hO, bytes, cudaHostAllocDefault);
+        if (ce == cudaSuccess) ce = cudaMalloc((void**)&dR, bytes);
+        if (ce == cudaSuccess) ce = cudaMalloc((void**)&dO, bytes);
+        if (ce != cudaSuccess) {
+            if (hR) cudaFreeHost(hR);
+            if (hO) cudaFreeHost(hO);
+            if (dR) cudaFree(dR);
+            if (dO) cudaFree(dO);
+            cudaGetLastError();
+            return vp_fail(e, ce, "stereo streaming buffers", __FILE__, __LINE__);
+        }
+        memset(hR, 0, bytes); memset(hO, 0, bytes);
+        e->sHostR = hR; e->sHostOR = hO; e->sDevR = dR; e->sDevOR = dO;
+    }
+    if (synthR) *synthR = e->sHostR;
+    if (outR) *outR = e->sHostOR;
+    return VP_OK;
+}
+
 extern "C" int vp_engine_stream_block(vp_engine* e) {
     if (!e) return VP_E_ARG;
     if (!e->prepared || !e->sHostV) return vp_err(e, VP_E_STATE, "call vp_engine_prepare and vp_engine_stream_buffers first");
     VP_CUDA_OK(cudaSetDevice(e->device));
     // the block's scheduled changes go into the [S] table here (a one-block call has no event after its first block)
     { int rc = plan_schedule(e, 1); if (rc) return rc; }
-    if (e->anySynth) return vp_err(e, VP_E_ARG, "streaming mode carries side-chain channel 0 only: gainSynth must be off on every stream");
+    // stereo: the right side-chain goes up and the right output comes back with every block, so the dry side-chain may be on
+    const bool stereo = e->sHostR != nullptr;
+    if (e->anySynth && !stereo)
+        return vp_err(e, VP_E_ARG, "mono streaming carries side-chain channel 0 only: gainSynth must be off on every stream "
+                                   "(vp_engine_stream_buffers_stereo streams both channels)");
     // per-stream key and gains are table data: a change is uploaded here, outside the graph, and needs no new capture
     // so are per-stream resets: one kernel before the graph, the block phase (the graph's key) does not change
     { int rc = upload_stream_params(e); if (!rc) rc = apply_stream_resets(e); if (rc) return rc; }
@@ -2337,6 +2378,9 @@ extern "C" int vp_engine_stream_block(vp_engine* e) {
                                   g.vocOn, g.pitchOn, g.vocMix, g.pitchMix, e->callAnyDry, g.ordV, g.ordS, g.ordTab, g.ordP, g.ordTabP};
     for (int j = 0; j < VP_ORPH; ++j) { key.push_back(g.orphPos[j]); key.push_back(g.orphOrdV[j]); key.push_back(g.orphOrdS[j]); }
     for (int j = 0; j < VP_PC; ++j) { key.push_back(g.carryPosP[j]); key.push_back(g.carryLimP[j]); }
+    // stereo graphs copy the right channels and hand them to the mix and the history update; whether some stream has the
+    // dry side-chain on is already in the key (callAnyDry selects the mix kernel), its gain is table data
+    key.push_back(stereo ? 1 : 0);
     auto it = e->graphs.find(key);
     if (it == e->graphs.end()) {
         const bool st = e->stageTiming;
@@ -2348,14 +2392,18 @@ extern "C" int vp_engine_stream_block(vp_engine* e) {
         int rc = VP_OK;
         cudaError_t ce = cudaMemcpyAsync(e->sDevV, e->sHostV, bytes, cudaMemcpyHostToDevice, e->st);
         if (ce == cudaSuccess) ce = cudaMemcpyAsync(e->sDevS, e->sHostS, bytes, cudaMemcpyHostToDevice, e->st);
+        if (ce == cudaSuccess && stereo) ce = cudaMemcpyAsync(e->sDevR, e->sHostR, bytes, cudaMemcpyHostToDevice, e->st);
         if (ce == cudaSuccess) {
+            // stereo: the mix writes R for every stream (R == L where the dry side-chain is off), as process_host's output
             for (int s0 = 0; s0 < e->S && rc == VP_OK; s0 += e->Sc) {
                 const int Sp = std::min(e->Sc, e->S - s0);
                 const size_t off = (size_t)s0 * e->B;
                 e->passCount = 0;
-                rc = run_pass(e, g, Sp, s0, e->sDevV + off, e->sDevS + off, nullptr, e->sDevO + off, nullptr);
+                rc = run_pass(e, g, Sp, s0, e->sDevV + off, e->sDevS + off, stereo ? e->sDevR + off : nullptr, e->sDevO + off,
+                              stereo ? e->sDevOR + off : nullptr);
             }
             if (rc == VP_OK) ce = cudaMemcpyAsync(e->sHostO, e->sDevO, bytes, cudaMemcpyDeviceToHost, e->st);
+            if (rc == VP_OK && ce == cudaSuccess && stereo) ce = cudaMemcpyAsync(e->sHostOR, e->sDevOR, bytes, cudaMemcpyDeviceToHost, e->st);
         }
         cudaError_t ce2 = cudaStreamEndCapture(e->st, &graph);
         e->stageTiming = st;
